@@ -8,6 +8,7 @@ One "step" = one SIMPLE iteration (the body of the loop at src/solver.rs:60-222 
   python bench.py --scaling strong [--size 256] --gpus N                    # ONE size^3 mesh cut into N slabs
   python bench.py --mesh couette|channel|tet                                # BASELINE.json configs 1, 2 and 5 (in kind)
   python bench.py --impl reference [--steps K] [--warmup W]                 # the reference's CPU path (oracle restatement)
+  python bench.py ... --dump-outputs DIR                                    # also write u, v, w, p of the last timed step as DIR/*.npy
 
 Prints ONE JSON line (rank 0). See DESIGN.md §7 for what every key means and how the roofline figures are derived.
 """
@@ -31,6 +32,8 @@ SPMV_SAMPLE = 17      # CUDA events around every 17th SpMV launch inside the tim
 RESET_EVERY = 6       # SIMPLE iterations between resets of the fields (see run_ours.step)
 METRIC = "SIMPLE iters/s"
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+DUMP_BYTES = 64_000_000   # --dump-outputs: the most all arrays may take together
+DUMP_SAMPLE = 1 << 20     # cells kept when the full fields would take more
 
 
 def workload_name(shape):
@@ -111,28 +114,27 @@ def oracle_run(m, steps=1, warmup=0):
 
 
 def run_reference(args, rank, world):
-    """The reference's own CPU implementation of the path, timed on the host cores. The Rust crate cannot be built in this
-    image (no cargo/rustc, no network: DESIGN.md §2), so this times oracle/ — its C++ restatement, single-threaded like ORC —
-    on THE SAME MESH as our arm's N = 1 workload (size^3 cells, default 128^3): one full SIMPLE iteration from rest takes about
-    two minutes there, so the step count is capped at 1 (no warm-up) whatever --steps / --warmup say; `sample` states it.
+    """The reference's path on the host cores, as oracle/ restates it in C++ (single-threaded like ORC; DESIGN.md §2 says why the
+    Rust crate itself is not timed), on THE SAME MESH as our arm's N = 1 workload (size^3 cells, default 128^3): --warmup untimed
+    SIMPLE iterations from rest, then --steps timed ones. One iteration takes about two minutes of one core at 128^3.
     At N > 1 our arm's global mesh has N x size^3 cells (weak scaling): the reference is still timed on size^3 and its rate is
     expressed in global-mesh iterations (cell count ratio), `same_config` false."""
     if rank != 0:
         return
     n = args.size if args.size else 128
-    steps = 1 if n >= 96 else max(1, min(args.steps, 3))
+    steps = args.steps
     t_wall = time.perf_counter()
-    cells, dt, phases = oracle_run(n, steps=steps, warmup=0)
+    cells, dt, phases = oracle_run(n, steps=steps, warmup=args.warmup)
     cell_rate = cells * steps / dt
     strong = args.scaling == "strong"
     gcells = cells if strong else world * cells
     iters_global = cell_rate / gcells
     value = iters_global if strong else world * iters_global      # same units as our arm's `value`
     shape = (n, n, n)
-    sample = (f"{steps} full SIMPLE iteration(s) from rest on the {n}^3 hex channel itself ({cells} cells, {dt:.1f} s), same settings as our arm; "
-              f"--steps {args.steps} --warmup {args.warmup} capped to {steps}/0 (one iteration is ~2 min of one core at 128^3)")
+    sample = (f"{steps} full SIMPLE iteration(s) after {args.warmup} untimed one(s) from rest on the {n}^3 hex channel itself ({cells} cells, "
+              f"{dt:.1f} s), same settings as our arm")
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "iter/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
-            "steps_timed": steps, "warmup_done": 0,
+            "steps_timed": steps, "warmup_done": args.warmup,
             "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": {"workload": workload_name(shape), "solver": "Multigrid(BiCGSTAB x50, 3 levels, Jacobi precond)", "momentum": "CD1",
                        "velocity_interpolation": "RhieChow", "pressure_interpolation": "SecondOrder", "pressure_relaxation": P_RELAX,
@@ -203,7 +205,7 @@ def run_e2e(args, world, dist, torch, orc_b200, mesh, settings, solver, ctx, bar
     solver.reset()
     solver.iterate(2)
     start_fields = solver.get_fields()   # every e2e step starts from the same host fields (2 iterations from rest)
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.e2e_steps
     sets = [[torch.from_numpy(f.copy()).pin_memory().numpy() for f in start_fields] for _ in range(e2e_steps)]
     # one untimed call first: the one-shot entry creates its own device state (5 matrices, 15 vectors), and the caching
     # allocator has to see those sizes once — like the W warm-up steps of the resident leg
@@ -241,6 +243,21 @@ def multi_gpu_parity(ctx, torch, dist, orc_b200, syn, local_rank, rank, world):
                        "digits, DESIGN.md §5, so larger comparisons say nothing about the partitioning.)")
     dist.barrier()
     return out
+
+
+def dump_outputs(path, fields):
+    """Writes u, v, w, p as <path>/{u,v,w,p}.npy (float64). When the four fields together exceed DUMP_BYTES, every field keeps the
+    same DUMP_SAMPLE cells, drawn with a fixed seed, so two builds of the project on the same mesh write the same cells;
+    <path>/cell_index.npy (float64) then lists them."""
+    os.makedirs(path, exist_ok=True)
+    out = dict(zip("uvwp", fields))
+    n = out["u"].size
+    if 4 * 8 * n > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+        out = {k: f[idx] for k, f in out.items()}
+        out["cell_index"] = idx
+    for k, f in out.items():
+        np.save(os.path.join(path, f"{k}.npy"), np.asarray(f, dtype=np.float64))
 
 
 def pooled(detail, peak, codes):
@@ -389,6 +406,7 @@ def run_ours(args, rank, world):
         ctx.prof_enable(False)
         phases = {k: (v - phases0[k]) / args.steps for k, v in solver.phase_ms().items()}   # timed steps only
         batched = solver.batched
+        fields = solver.get_fields() if args.dump_outputs else None    # before the untimed step below moves them on
         ctx.prof_config(classes=None, sample_every=1)
         ctx.prof_enable(True)
         step()                                  # untimed: device time per kernel class, events around every launch
@@ -396,7 +414,7 @@ def run_ours(args, rank, world):
         classes.pop("bicgstab", None)           # brackets the other classes
         ctx.prof_enable(False)
         clocks = sampler.finish() if sampler else None
-        return ms, launches, prof, sp_ref_bytes, sp_detail, phases, batched, classes, clocks, rep
+        return ms, launches, prof, sp_ref_bytes, sp_detail, phases, batched, classes, clocks, rep, fields
 
     # The reference's algorithm is marginally unstable on the synthetic boxes (DESIGN.md §5): how many iterations a start from
     # rest survives depends on rounding (summation orders, the partitioning). If a run meets "Multigrid diverged" the whole
@@ -404,7 +422,7 @@ def run_ours(args, rank, world):
     restarts = 0
     while True:
         try:
-            ms, launches, prof, sp_ref_bytes, sp_detail, phases, batched, classes, clocks, rep = measure()
+            ms, launches, prof, sp_ref_bytes, sp_detail, phases, batched, classes, clocks, rep, fields = measure()
             break
         except orc_b200.OrcError as e:
             if "diverged" not in str(e) or not reset_every or reset_every <= 2 or restarts >= 3:
@@ -421,6 +439,8 @@ def run_ours(args, rank, world):
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fields)
     global_iters = args.steps / (ms * 1e-3)             # SIMPLE iterations of the GLOBAL mesh per second
     # weak scaling: one global problem of world x size^3 cells; `value` counts size^3-cell-equivalent iterations (= cell-updates/s
     # / size^3) so that it is a whole-job aggregate; strong scaling and N = 1: iterations of the one mesh.
@@ -541,7 +561,7 @@ def run_ours(args, rank, world):
         "phases_ms_per_step": phases,
         "cpu_baseline": cpu,
         "e2e": {"value": e2e_value, "unit": "iter/s", "global_iters_per_s": e2e_global, "h2d_bytes_per_step": 32 * cells, "d2h_bytes_per_step": 32 * cells,
-                "call": "orc_solve_steady(iteration_count=1) per step, pinned host u/v/w/p", "steps": max(1, min(args.steps, 3))},
+                "call": "orc_solve_steady(iteration_count=1) per step, pinned host u/v/w/p", "steps": args.e2e_steps},
         "small_meshes": small_runs,
         "partition_parity": parity,
         "gpu_launches": int(launches),
@@ -571,9 +591,16 @@ def main():
     ap.add_argument("--reset-every", type=int, default=RESET_EVERY, help="SIMPLE iterations between resets of the fields (the reference's "
                     "algorithm diverges on the synthetic boxes after a few iterations; sooner on larger ones)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end leg (profiling runs under ncu)")
+    ap.add_argument("--e2e-steps", type=int, default=3, help="calls timed in the end-to-end leg (each copies the fields in and out)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="one GPU: write u, v, w, p after the last timed step to DIR/<name>.npy "
+                    "(float64; a fixed, seeded sample of cells when the four fields exceed 64 MB, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0 or args.e2e_steps < 1:
+        ap.error("--steps and --e2e-steps must be at least 1, --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs writes the fields of the GPU path (--impl ours) on one GPU only")
     if args.impl == "reference":
         run_reference(args, rank, world)
     else:
