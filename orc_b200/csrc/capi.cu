@@ -531,6 +531,7 @@ int32_t orc_spmv(orc_ctx* ctx, const orc_csr* a, const double* x, double* y) {
     ORC_TRY({
         require(ctx && a && x && y, "null argument");
         Ctx& c = ctx->c;
+        c.exact_order = false;   // the fast kernels, whatever reduction mode the last solve on this context used
         HostVecIn dx(c, x, a->m->ncols);
         DBuf<double> dy(&c, (size_t)std::max<int64_t>(a->m->nrows, 1));
         spmv(c, *a->m, dx.d, dy);
@@ -1227,6 +1228,7 @@ int32_t orc_prof_get(orc_ctx* ctx, double* ms, double* bytes, uint64_t* count, i
     });
 }
 static double bench_spmv(Ctx& c, const DCsr& A, int K, int reps) {
+    c.exact_order = false;   // times the fast kernels, whatever reduction mode the last solve on this context used
     const int S = K == 1 ? 1 : 4;
     DBuf<double> x(&c, (size_t)std::max<int64_t>(A.ncols, 1) * S), y(&c, (size_t)std::max<int64_t>(A.nrows, 1) * S);
     dev_fill(c, x, 1., A.ncols * S);
@@ -1243,6 +1245,7 @@ static double bench_spmv(Ctx& c, const DCsr& A, int K, int reps) {
     return ms / reps;
 }
 static double bench_bicgstab(Ctx& c, const DCsr& A, int K, int reps) {
+    c.exact_order = false;
     const int S = K == 1 ? 1 : 4;
     const size_t n = (size_t)std::max<int64_t>(A.nrows, 1) * S;
     DBuf<double> x(&c, n), b(&c, n);

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 import scipy.sparse as sp
 
+import fast_model as fm
 import orc_b200
 from orc_b200 import linear_algebra as la
 from orc_b200.settings import SolutionMethod, PreconditionMethod, RestrictionMethods
@@ -62,12 +63,13 @@ def assert_csr_equal(g, o, exact_values=True, tol=0.0):
 def assert_spmv(a, y, yo, x):
     """Rows shorter than 10 on average go through the thread-per-row kernel whose in-row sums run in ascending column order:
     bit-exact. Longer rows (AMG coarse levels) use G lanes per row and a fixed shuffle tree: equal to rounding, measured
-    against the row's own magnitude sum |a_ik x_k|."""
+    against the row's own magnitude sum |a_ik x_k| (model-free), and bit-exact against that tree in tests/fast_model.py."""
     if a.nnz < 10 * a.shape[0]:
         assert np.array_equal(y, yo)
     else:
         mag = abs(a) @ np.abs(x)
         assert np.all(np.abs(y - yo) <= 1e-14 * np.maximum(mag, 1e-300))
+        assert np.array_equal(y, fm.spmv(fm.Mat.from_scipy(a), x)[0])
 
 
 @pytest.mark.parametrize("n,density", [(1, 1.0), (37, 0.2), (1000, 0.004), (5000, 0.001), (1000, 0.01), (5000, 0.004), (300, 0.5), (2000, 0.03)])
@@ -92,7 +94,8 @@ def test_spmv_long_rows_and_empty_rows(oracle, ctx):
 
 
 def test_spmv_short_rows_spanning_staging_chunks(oracle, ctx):
-    """A few very long rows inside a short-row matrix: the staged kernel must carry a row's ordered sum across chunks."""
+    """A few very long rows (4000 and 2000 entries) inside a short-row matrix: the thread-per-row kernel sums each of them
+    alone, in ascending column order, however long it is."""
     rng = np.random.default_rng(9)
     a = random_spd_like(4000, 0.0005, seed=77).tolil()
     a[100, :] = rng.standard_normal(4000)
