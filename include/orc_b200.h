@@ -234,6 +234,9 @@ int32_t orc_steady_phase_ms(orc_steady* st, double* out5);
 int32_t orc_steady_batched(orc_steady* st, int32_t* out);
 /* per-level sizes of the last Multigrid solve: out[2*l] = rows, out[2*l+1] = nnz, l = 0..levels */
 int32_t orc_steady_level_sizes(orc_steady* st, int64_t* out, int32_t cap, int32_t* n_levels);
+/* orc_gradients of the handle's resident u, v, w, p, without their round trip through the host: the OWNED rows (n_own of a
+ * partition, after a halo exchange of the four fields), same layout, NULL outputs and errors as orc_gradients. */
+int32_t orc_steady_gradients(orc_steady* st, int32_t gradient, double* grad_p3n, double* grad_u9n);
 void orc_steady_destroy(orc_steady* st);
 
 /* ---- flow initialisation: the step before the loop (src/solver.rs:246-352) ------------------------- */
@@ -242,7 +245,9 @@ enum { ORC_CONSTRAINT_PRESSURE_ONLY = 0, ORC_CONSTRAINT_VELOCITY_ONLY = 1, ORC_C
 int32_t orc_check_boundary_conditions(const orc_mesh* m, int32_t* constraint_type);
 /* the Laplace system assembled by initialize_pressure_field (src/solver.rs:437-494); b_out: n_cells doubles */
 int32_t orc_build_pressure_laplace(orc_ctx* ctx, orc_mesh* m, orc_csr** a_out, double* b_out);
-/* initialize_flow (src/solver.rs:246-352): returns u, v, w, p (n_cells doubles each, host). `reduction_mode` as in orc_settings. */
+/* initialize_flow (src/solver.rs:246-352): returns u, v, w, p (n_cells doubles each, host). `reduction_mode` as in orc_settings.
+ * Both initialisations also take a partition mesh (all ranks call them together): they write its OWNED cells (n_own doubles), as
+ * orc_steady_get_fields does; ORC_REDUCE_REFERENCE_ORDER is single-GPU only (ORC_E_UNSUPPORTED), Auto means Fast there. */
 int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, uint64_t iteration_count, int32_t reduction_mode, double* u,
                             double* v, double* w, double* p);
 /* initialize_flow_new (src/solver.rs:354-410; the reference's current main() calls it, src/tests.rs:195-197): pressure field for

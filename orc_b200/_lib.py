@@ -51,7 +51,7 @@ EXPORTS = [
     "orc_iterative_solve3", "orc_build_restriction", "orc_galerkin", "orc_multigrid_trace", "orc_build_momentum_diffusion", "orc_init_momentum_matrix",
     "orc_build_momentum_advection", "orc_build_pressure_correction", "orc_pressure_gradient", "orc_apply_pressure_correction",
     "orc_solve_steady", "orc_check_boundary_conditions", "orc_build_pressure_laplace", "orc_initialize_flow", "orc_initialize_flow_new", "orc_build_velocity_potential", "orc_potential_gradient", "orc_gradients", "orc_steady_create", "orc_steady_set_fields", "orc_steady_get_fields", "orc_steady_iterate", "orc_steady_reset",
-    "orc_steady_phase_ms", "orc_steady_batched", "orc_steady_level_sizes", "orc_steady_destroy", "orc_bench_amg_setup", "orc_bench_spmv", "orc_bench_bicgstab", "orc_bench_spmv_batch", "orc_bench_bicgstab_batch", "orc_prof_enable", "orc_prof_config", "orc_prof_get", "orc_prof_get_ref_bytes", "orc_prof_get_spmv_detail", "orc_comm_unique_id", "orc_ctx_comm_init", "orc_ctx_peer_window", "orc_ctx_peer_open", "orc_ctx_peer_disable", "orc_ctx_peer_enabled", "orc_mesh_partition", "orc_mesh_partition_window",
+    "orc_steady_phase_ms", "orc_steady_batched", "orc_steady_level_sizes", "orc_steady_gradients", "orc_steady_destroy", "orc_bench_amg_setup", "orc_bench_spmv", "orc_bench_bicgstab", "orc_bench_spmv_batch", "orc_bench_bicgstab_batch", "orc_prof_enable", "orc_prof_config", "orc_prof_get", "orc_prof_get_ref_bytes", "orc_prof_get_spmv_detail", "orc_comm_unique_id", "orc_ctx_comm_init", "orc_ctx_peer_window", "orc_ctx_peer_open", "orc_ctx_peer_disable", "orc_ctx_peer_enabled", "orc_mesh_partition", "orc_mesh_partition_window",
     "orc_mesh_partition_info", "orc_mesh_partition_maps",
 ]
 

@@ -135,7 +135,9 @@ static orc_steady* steady_create(orc_ctx* octx, orc_mesh* m, const orc_settings*
         st->N_global = m->plan->n_global;
         st->env.comm = &octx->comm; st->env.halo = m->dev[&c].halo.get();
         if (st->env.on()) {
-            require(s->solver_type == ORC_SOLVER_BICGSTAB || s->solver_type == ORC_SOLVER_MULTIGRID, "multi-GPU solves support BiCGSTAB and Multigrid");
+            // Gauss-Seidel's sweep is one dependency chain over all rows: it has no partitioned form
+            require(s->solver_type == ORC_SOLVER_JACOBI || s->solver_type == ORC_SOLVER_BICGSTAB || s->solver_type == ORC_SOLVER_MULTIGRID,
+                    "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid");
             st->env.halo->agree_on_peer(c, octx->comm);
             Comm* cm = st->env.comm; Halo* hl = st->env.halo; Ctx* cp = &c;
             st->work.halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); };
@@ -914,7 +916,8 @@ int32_t orc_solve_steady(orc_ctx* ctx, orc_mesh* m, double* u, double* v, double
 // ---- flow initialisation: the step before the loop (src/solver.rs:246-352, 414-509, 703-770) ---------------------------------
 // check_boundary_conditions (:710-770), host logic. The two angle checks compare against TOL = 5 * 180 / PI = 286.5 (radians),
 // so they can never fire; the counters are u16 and count EVERY face of the mesh for a moving wall: a release build wraps.
-static int check_boundary_conditions(const HostMesh& h) {
+// `mesh_faces`: the face count of the whole mesh (h.n_faces unless h is a partition).
+static int check_boundary_conditions(const HostMesh& h, int64_t mesh_faces) {
     const double PI = (double)3.14159274101257324f;  // std::f32::consts::PI as Float
     const double TOL = 5. * 180. / PI;
     uint16_t pressure_bc = 0, velocity_bc = 0;
@@ -926,11 +929,11 @@ static int check_boundary_conditions(const HostMesh& h) {
     for (const HostZone& z : h.zones) {
         switch (z.type) {
             case ORC_BC_WALL:
-                if (sqrt(z.vec[0] * z.vec[0] + z.vec[1] * z.vec[1] + z.vec[2] * z.vec[2]) > 0.)
-                    for (int64_t f = 0; f < h.n_faces; ++f) {
-                        velocity_bc = (uint16_t)(velocity_bc + 1);
+                if (sqrt(z.vec[0] * z.vec[0] + z.vec[1] * z.vec[1] + z.vec[2] * z.vec[2]) > 0.) {
+                    velocity_bc = (uint16_t)(velocity_bc + (uint16_t)mesh_faces);   // += 1 per face, wrapping
+                    for (int64_t f = 0; f < h.n_faces; ++f)
                         if (PI / 2. - fabs(angle(f, z.vec)) > TOL) throw Error(ORC_E_INVALID, "Wall velocity must be tangent to faces in zone.");
-                    }
+                }
                 break;
             case ORC_BC_VELOCITY_INLET:
                 velocity_bc = (uint16_t)(velocity_bc + 1);
@@ -946,7 +949,7 @@ static int check_boundary_conditions(const HostMesh& h) {
     throw Error(ORC_E_INVALID, "You must set boundary conditions.");
 }
 int32_t orc_check_boundary_conditions(const orc_mesh* m, int32_t* constraint_type) {
-    ORC_TRY({ require(m && m->h && constraint_type, "null argument"); *constraint_type = check_boundary_conditions(*m->h); });
+    ORC_TRY({ require(m && m->h && constraint_type, "null argument"); *constraint_type = check_boundary_conditions(*m->h, m->h->n_faces); });
 }
 int32_t orc_build_pressure_laplace(orc_ctx* ctx, orc_mesh* m, orc_csr** a_out, double* b_out) {
     ORC_TRY({
@@ -962,6 +965,67 @@ int32_t orc_build_pressure_laplace(orc_ctx* ctx, orc_mesh* m, orc_csr** a_out, d
         *a_out = wrap(detach(c, std::move(a)));
     });
 }
+// ---- the initialisation on a partition mesh: every rank runs the same steps on its owned cells, collectives in lockstep ----
+static double allreduce_host(Ctx& c, Comm& cm, double v, int op) {
+    if (!cm.active()) return v;
+    DBuf<double> d(&c, 1);
+    ORC_CUDA(cudaMemcpyAsync(d.p, &v, sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    cm.allreduce(c, d.p, 1, op);
+    ORC_CUDA(cudaMemcpyAsync(&v, d.p, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
+    c.sync();
+    return v;
+}
+// check_solver_flags with the status word of all ranks: some flags are local (a singular least-squares fit on one rank), and every
+// rank must return the same status (and stay in the collectives together)
+static void check_agreed_flags(Ctx& c, const DistEnv& env) {
+    if (!env.on()) { check_solver_flags(c); return; }
+    DBuf<double> d(&c, 1);
+    k_flags_to_double<<<1, 1, 0, c.stream>>>(c.d_flags, d.p);
+    c.after_launch("k_flags_to_double");
+    env.comm->allreduce(c, d.p, 1, 0);
+    double h = 0.;
+    ORC_CUDA(cudaMemcpyAsync(&h, d.p, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
+    c.sync();
+    c.clear_flags();
+    throw_for_flags(flags_from_double(h));
+}
+struct InitEnv {
+    DistEnv env;
+    bool exact_order = false;
+    int constraint = ORC_CONSTRAINT_PRESSURE_ONLY;
+    int64_t lo = 0, n_own = 0;   // the cells the caller receives
+};
+// What both initialisations do first: the boundary-condition check over the WHOLE mesh (a partition counts the faces whose c0 it
+// owns, so that every face is counted once), the reduction mode, and the halo plan of a partition.
+static InitEnv init_env(orc_ctx* ctx, orc_mesh* m, int reduction_mode) {
+    Ctx& c = ctx->c;
+    InitEnv ie;
+    const HostMesh& h = *m->h;
+    if (!m->plan) {
+        ie.constraint = check_boundary_conditions(h, h.n_faces);
+        DMesh& d = device_mesh(c, m);
+        ie.exact_order = resolve_exact_order(reduction_mode, d.N);
+        ie.n_own = d.N;
+        return ie;
+    }
+    require(ctx->comm.nranks == m->plan->nranks && ctx->comm.rank == m->plan->rank, "partition mesh does not match the context's communicator");
+    if (reduction_mode == ORC_REDUCE_REFERENCE_ORDER) throw Error(ORC_E_UNSUPPORTED, "reference-order reductions are single-GPU only");
+    DMesh& d = device_mesh(c, m);
+    ie.env.comm = &ctx->comm; ie.env.halo = m->dev[&c].halo.get();
+    if (ie.env.on()) ie.env.halo->agree_on_peer(c, ctx->comm);
+    int64_t own_faces = 0;
+    for (int64_t f = 0; f < h.n_faces; ++f) own_faces += (h.face_c0[f] >= d.own_lo && h.face_c0[f] < d.own_hi);
+    ie.constraint = check_boundary_conditions(h, (int64_t)allreduce_host(c, ctx->comm, (double)own_faces, 0));
+    ie.lo = d.own_lo; ie.n_own = d.own_hi - d.own_lo;
+    return ie;
+}
+static void xch(Ctx& c, const InitEnv& ie, std::initializer_list<double*> f) {
+    if (!ie.env.on()) return;
+    double* a[Halo::kMaxFields]; int k = 0;
+    for (double* q : f) a[k++] = q;
+    ie.env.halo->exchange(c, *ie.env.comm, a, k);
+}
+
 // initialize_flow (:246-352): Laplace pressure field (Jacobi x10), one UD / LinearWeighted momentum assembly at rest, then six
 // rounds of BiCGSTAB on a_u * (1 - f) + a_di * f, f = 1, 0.8, ... for u, v and w. The three blended matrices are bit-identical
 // (UD), so the three solves of a round run in lockstep like the momentum solves of the loop.
@@ -969,10 +1033,10 @@ int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, ui
                             double* v, double* w, double* p) {
     ORC_TRY({
         require(ctx && m && u && v && w && p, "null argument");
-        require(!m->plan, "initialize_flow runs on the whole mesh (single GPU)");
         Ctx& c = ctx->c;
         c.clear_flags();
-        check_boundary_conditions(*m->h);                                                                  // :272
+        const InitEnv ie = init_env(ctx, m, reduction_mode);                                                 // :272
+        DistEnv env = ie.env;
         DMesh& d = device_mesh(c, m);
         const int64_t N = d.N;
         const size_t Nz = (size_t)std::max<int64_t>(N, 1);
@@ -985,22 +1049,25 @@ int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, ui
         init_momentum_matrix(c, d, *a_u); init_momentum_matrix(c, d, *a_v); init_momentum_matrix(c, d, *a_w);  // :280-282
         dev_fill(c, diag_u, 1., N); dev_fill(c, diag_v, 1., N); dev_fill(c, diag_w, 1., N);
         SolveParams sp;
-        sp.exact_order = resolve_exact_order(reduction_mode, N);
+        sp.exact_order = ie.exact_order;
         // initialize_pressure_field (:414-509)
         build_pressure_laplace(c, d, *lap, pb);
         sp.iterations = 10; sp.method = ORC_SOLVER_JACOBI; sp.relaxation = 0.1; sp.threshold = 1e-6; sp.preconditioner = ORC_PC_JACOBI;
-        iterative_solve(c, *lap, pb, dp, sp, nullptr);                                                     // :498-507
-        check_solver_flags(c);
+        iterative_solve_dist(c, env, *lap, pb, dp, sp, nullptr);                                            // :498-507
+        check_agreed_flags(c, env);
         // :288-306: UD, LinearWeighted velocity and pressure interpolation, Green-Gauss cell based; u = v = w = 0
         AsmSettings as;
         as.momentum = ORC_MOM_UD; as.limiter = ORC_PSI_UD; as.p_interp = ORC_P_LINEAR_WEIGHTED; as.v_interp = ORC_V_LINEAR_WEIGHTED;
         as.gradient = ORC_G_GREEN_GAUSS_CELL; as.assembly_mode = ORC_ASSEMBLY_EXACT;
         AsmWork work;
+        if (env.on()) { Comm* cm = env.comm; Halo* hl = env.halo; Ctx* cp = &c; work.halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); }; }
+        xch(c, ie, {dp.p});                                                                                // the neighbours' pressure
         build_momentum_advection(c, d, work, as, rho, *a_u, *a_v, *a_w, *a_di, diag_u, diag_v, diag_w, du, dv, dw, dp, b_u, b_v, b_w, pe3);
         dev_axpy_inplace(c, b_u, b_u_di, N); dev_axpy_inplace(c, b_v, b_v_di, N); dev_axpy_inplace(c, b_w, b_w_di, N);  // :307-309
         sp.iterations = iteration_count; sp.method = ORC_SOLVER_BICGSTAB; sp.relaxation = 0.5; sp.threshold = 1e-6;
-        const bool lockstep = solve_batchable(sp) && csr_values_identical(c, *a_u, *a_v) && csr_values_identical(c, *a_u, *a_w) &&
-                              !(getenv("ORC_B200_BATCH") && atoi(getenv("ORC_B200_BATCH")) == 0);
+        bool lockstep = solve_batchable(sp) && csr_values_identical(c, *a_u, *a_v) && csr_values_identical(c, *a_u, *a_w) &&
+                        !(getenv("ORC_B200_BATCH") && atoi(getenv("ORC_B200_BATCH")) == 0);
+        if (env.on()) lockstep = allreduce_host(c, *env.comm, lockstep ? 1. : 0., 3) == 1.;   // the solves hold collectives: one branch for all
         double f = 1.;
         while (f >= 0.) {                                                                                  // :316-350
             if (lockstep) {
@@ -1008,17 +1075,17 @@ int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, ui
                 DBuf<double> b4(&c, Nz * 4), x4(&c, Nz * 4);
                 pack3(c, N, b_u, b_v, b_w, b4);
                 pack3(c, N, du, dv, dw, x4);
-                iterative_solve(c, *blend, b4, x4, sp, nullptr, 3);
+                iterative_solve_dist(c, env, *blend, b4, x4, sp, nullptr, 3);
                 unpack3(c, N, x4, du, dv, dw);
             } else {
-                csr_blend(c, *a_u, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_u, du, sp, nullptr);
-                csr_blend(c, *a_v, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_v, dv, sp, nullptr);
-                csr_blend(c, *a_w, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_w, dw, sp, nullptr);
+                csr_blend(c, *a_u, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_u, du, sp, nullptr);
+                csr_blend(c, *a_v, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_v, dv, sp, nullptr);
+                csr_blend(c, *a_w, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_w, dw, sp, nullptr);
             }
             f -= 0.2;
         }
-        to_host(c, u, du, N); to_host(c, v, dv, N); to_host(c, w, dw, N); to_host(c, p, dp, N);
-        check_solver_flags(c);
+        to_host(c, u, du + ie.lo, ie.n_own); to_host(c, v, dv + ie.lo, ie.n_own); to_host(c, w, dw + ie.lo, ie.n_own); to_host(c, p, dp + ie.lo, ie.n_own);
+        check_agreed_flags(c, env);
     });
 }
 
@@ -1057,11 +1124,11 @@ int32_t orc_initialize_flow_new(orc_ctx* ctx, orc_mesh* m, double mu, double rho
                                 double* v, double* w, double* p) {
     ORC_TRY({
         require(ctx && m && u && v && w && p, "null argument");
-        require(!m->plan, "initialize_flow_new runs on the whole mesh (single GPU)");
         (void)mu; (void)rho; (void)iteration_count;   // unused by the reference as well (:354-358, `_iteration_count` :414)
         Ctx& c = ctx->c;
         c.clear_flags();
-        const int constraint = check_boundary_conditions(*m->h);                                           // :395
+        const InitEnv ie = init_env(ctx, m, reduction_mode);                                               // :395
+        DistEnv env = ie.env;
         DMesh& d = device_mesh(c, m);
         const int64_t N = d.N;
         const size_t Nz = (size_t)std::max<int64_t>(N, 1);
@@ -1069,54 +1136,78 @@ int32_t orc_initialize_flow_new(orc_ctx* ctx, orc_mesh* m, double mu, double rho
         for (DBuf<double>* q : {&du, &dv, &dw, &dp, &rhs, &psi}) q->zero();
         CsrPtr a = mesh_matrix(c, d);
         SolveParams sp;
-        sp.exact_order = resolve_exact_order(reduction_mode, N);
+        sp.exact_order = ie.exact_order;
         sp.preconditioner = ORC_PC_JACOBI; sp.iterations = 10; sp.relaxation = 0.1; sp.threshold = 1e-6;
-        if (constraint == ORC_CONSTRAINT_PRESSURE_ONLY || constraint == ORC_CONSTRAINT_HYBRID) {            // :399-402
+        if (ie.constraint == ORC_CONSTRAINT_PRESSURE_ONLY || ie.constraint == ORC_CONSTRAINT_HYBRID) {      // :399-402
             build_pressure_laplace(c, d, *a, rhs);
             sp.method = ORC_SOLVER_JACOBI;
-            iterative_solve(c, *a, rhs, dp, sp, nullptr);                                                  // :498-507
+            iterative_solve_dist(c, env, *a, rhs, dp, sp, nullptr);                                        // :498-507
         } else {                                                                                           // :403-405
             build_velocity_potential(c, d, *a, rhs);
             sp.method = ORC_SOLVER_BICGSTAB;
-            iterative_solve(c, *a, rhs, psi, sp, nullptr);                                                 // :592-601
+            iterative_solve_dist(c, env, *a, rhs, psi, sp, nullptr);                                       // :592-601
+            xch(c, ie, {psi.p});                                                                           // the neighbours' psi
             potential_gradient(c, d, psi, du, dv, dw);                                                     // :624-693
         }
-        to_host(c, u, du, N); to_host(c, v, dv, N); to_host(c, w, dw, N); to_host(c, p, dp, N);
-        check_solver_flags(c);
+        to_host(c, u, du + ie.lo, ie.n_own); to_host(c, v, dv + ie.lo, ie.n_own); to_host(c, w, dw + ie.lo, ie.n_own); to_host(c, p, dp + ie.lo, ie.n_own);
+        check_agreed_flags(c, env);
     });
 }
 // calculate_pressure_gradient / calculate_velocity_gradient of every cell (src/solver.rs:774-949): what write_gradients prints
 // (src/io.rs:623-662). grad_p3n: N x 3, grad_u9n: N x 9 row-major tensors; either may be null.
+static void require_gradient_scheme(int32_t gradient, bool pressure) {
+    if (gradient == ORC_G_GREEN_GAUSS_NODE && pressure) throw Error(ORC_E_UNSUPPORTED, "unsupported Green-Gauss scheme");   // solver.rs:901
+    if (gradient != ORC_G_GREEN_GAUSS_CELL && gradient != ORC_G_GREEN_GAUSS_NODE && gradient != ORC_G_LEAST_SQUARES)
+        throw Error(ORC_E_UNSUPPORTED, "unsupported gradient scheme");                                                      // :870, 948
+}
+// the gradients of device fields u, v, w, p; rows [lo, lo + cnt) of the mesh go to the host in orc_gradients' layout
+static void gradients_to_host(Ctx& c, const DMesh& d, const double* u, const double* v, const double* w, const double* p, int32_t gradient,
+                              int64_t lo, int64_t cnt, double* grad_p3n, double* grad_u9n) {
+    const size_t N = (size_t)std::max<int64_t>(d.N, 1);
+    const int g = (gradient == ORC_G_LEAST_SQUARES) ? ORC_G_LEAST_SQUARES : ORC_G_GREEN_GAUSS_CELL;
+    if (grad_p3n) {
+        DBuf<double> gx(&c, N), gy(&c, N), gz(&c, N);
+        pressure_gradient(c, d, p, gx, gy, gz, g);
+        std::vector<double> hx(N), hy(N), hz(N);
+        to_host(c, hx.data(), gx, d.N); to_host(c, hy.data(), gy, d.N); to_host(c, hz.data(), gz, d.N);
+        c.sync();
+        for (int64_t i = 0; i < cnt; ++i) { grad_p3n[3 * i] = hx[lo + i]; grad_p3n[3 * i + 1] = hy[lo + i]; grad_p3n[3 * i + 2] = hz[lo + i]; }
+    }
+    if (grad_u9n) {
+        DBuf<double> gu(&c, 9 * N);
+        velocity_gradient(c, d, u, v, w, gu, g);
+        std::vector<double> h(9 * N);
+        to_host(c, h.data(), gu, 9 * d.N);
+        c.sync();
+        for (int64_t i = 0; i < cnt; ++i) for (int k = 0; k < 9; ++k) grad_u9n[9 * i + k] = h[(size_t)k * d.N + lo + i];
+    }
+}
 int32_t orc_gradients(orc_ctx* ctx, orc_mesh* m, const double* u, const double* v, const double* w, const double* p, int32_t gradient,
                       double* grad_p3n, double* grad_u9n) {
     ORC_TRY({
         require(ctx && m && u && v && w && p, "null argument");
-        if (gradient == ORC_G_GREEN_GAUSS_NODE && grad_p3n) throw Error(ORC_E_UNSUPPORTED, "unsupported Green-Gauss scheme");   // solver.rs:901
-        if (gradient != ORC_G_GREEN_GAUSS_CELL && gradient != ORC_G_GREEN_GAUSS_NODE && gradient != ORC_G_LEAST_SQUARES)
-            throw Error(ORC_E_UNSUPPORTED, "unsupported gradient scheme");                                                      // :870, 948
+        require_gradient_scheme(gradient, grad_p3n != nullptr);
         Ctx& c = ctx->c;
         DMesh& d = device_mesh(c, m);
-        const size_t N = (size_t)std::max<int64_t>(d.N, 1);
         HostVecIn du(c, u, d.N), dv(c, v, d.N), dw(c, w, d.N), dp(c, p, d.N);
         c.clear_flags();
-        const int g = (gradient == ORC_G_LEAST_SQUARES) ? ORC_G_LEAST_SQUARES : ORC_G_GREEN_GAUSS_CELL;
-        if (grad_p3n) {
-            DBuf<double> gx(&c, N), gy(&c, N), gz(&c, N);
-            pressure_gradient(c, d, dp.d, gx, gy, gz, g);
-            std::vector<double> hx(N), hy(N), hz(N);
-            to_host(c, hx.data(), gx, d.N); to_host(c, hy.data(), gy, d.N); to_host(c, hz.data(), gz, d.N);
-            c.sync();
-            for (int64_t i = 0; i < d.N; ++i) { grad_p3n[3 * i] = hx[i]; grad_p3n[3 * i + 1] = hy[i]; grad_p3n[3 * i + 2] = hz[i]; }
-        }
-        if (grad_u9n) {
-            DBuf<double> gu(&c, 9 * N);
-            velocity_gradient(c, d, du.d, dv.d, dw.d, gu, g);
-            std::vector<double> h(9 * N);
-            to_host(c, h.data(), gu, 9 * d.N);
-            c.sync();
-            for (int64_t i = 0; i < d.N; ++i) for (int k = 0; k < 9; ++k) grad_u9n[9 * i + k] = h[(size_t)k * d.N + i];
-        }
+        gradients_to_host(c, d, du.d, dv.d, dw.d, dp.d, gradient, 0, d.N, grad_p3n, grad_u9n);
         check_solver_flags(c);
+    });
+}
+int32_t orc_steady_gradients(orc_steady* st, int32_t gradient, double* grad_p3n, double* grad_u9n) {
+    ORC_TRY({
+        require(st != nullptr, "null argument");
+        require_gradient_scheme(gradient, grad_p3n != nullptr);
+        Ctx& c = *st->c;
+        DMesh& d = device_mesh(c, st->mesh);
+        c.clear_flags();
+        if (st->env.on()) {   // the neighbours' u, v, w, p (the handle's halo cells hold whatever the last exchange left)
+            double* f[4] = {st->u.p, st->v.p, st->w.p, st->p.p};
+            st->env.halo->exchange(c, *st->env.comm, f, 4);
+        }
+        gradients_to_host(c, d, st->u, st->v, st->w, st->p, gradient, d.own_lo, d.own_hi - d.own_lo, grad_p3n, grad_u9n);
+        check_agreed_flags(c, st->env);
     });
 }
 

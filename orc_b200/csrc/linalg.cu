@@ -277,6 +277,7 @@ struct SpmvArgs {
     int iter;
     int defer;  // EP_JACOBI_RES: leave the convergence decision to k_dot_ref (reference-order norm)
     int dist;   // multi-GPU: publish the LOCAL totals (stage_slot); the scalars are derived after the allreduce
+    int row0;   // Jacobi epilogues: kernel row i is row i + row0 of the vectors (a partition solves its owned rows only)
     int nv;     // virtual blocks of this launch (Ctx::kVirtualBlocks): the unit of the fused reductions
 };
 
@@ -316,15 +317,17 @@ __device__ __forceinline__ void spmv_row_epilogue(const SpmvArgs& a, int i, cons
 #pragma unroll
         for (int k = 0; k < K; ++k) { const double r = bi[k] - acc[k]; acc0[k] += r * r; }
     } else if (EPI == EP_JACOBI) {  // K == 1 only (launch_spmv)
-        double xi = a.x[i];
+        const int g = i + a.row0;
+        double xi = a.x[g];
         if (xi != xi) nanflag = 1;
-        a.y[i] = a.w * (a.b[i] - acc[0]) + xi * a.one_minus_w;
+        a.y[g] = a.w * (a.b[g] - acc[0]) + xi * a.one_minus_w;
     } else if (EPI == EP_JACOBI_RES) {  // K == 1 only
-        double xi = a.x[i];
-        double r = a.b[i] - acc[0];
+        const int g = i + a.row0;
+        double xi = a.x[g];
+        double r = a.b[g] - acc[0];
         acc0[0] += r * r;
         if (xi != xi) nanflag = 1; else acc1[0] = fmax(acc1[0], fabs(xi));
-        a.y2[i] = xi;
+        a.y2[g] = xi;
     }
 }
 // number of fused sums of an epilogue: quantity q of system k lives in partial lane q * K + k (K = 3: at most 6 of 8 lanes)
@@ -361,6 +364,22 @@ __device__ __forceinline__ void spmv_block_partials(const SpmvArgs& a, int vb, i
         vb_park<K>(sh, lv, acc0);
     }
 }
+// The Jacobi decision that follows the residual (linear_algebra.rs:202-216) from the totals of the scaled system: sum of r^2, max |xn|
+// over the rows that are not NaN, and the number of NaN rows. One thread; the single-GPU residual kernel and k_jacobi_decide share it.
+__device__ __forceinline__ void jacobi_decide(double* scal, int* flags, int iter, double threshold, double sum_r2, double max_abs, double nan_rows) {
+    double r = sqrt(sum_r2);
+    scal[S_NORM] = r;
+    // `initial_residual` starts at 0 in every call (:170) and is taken at iter_num == 1 (:208, Q9)
+    const double initial = (iter == 0) ? 0. : scal[S_JAC_INIT];
+    if (iter == 1) {
+        scal[S_JAC_INIT] = r;
+    } else if (r / initial < threshold) {
+        atomicOr(flags, DF_CONVERGED);
+        return;  // `break` precedes the magnitude check (:209-216)
+    }
+    if (nan_rows == 0. && max_abs > 1e10) atomicOr(flags, DF_JACOBI_HUGE);  // a NaN maximum compares false in the reference
+}
+
 // the last block to finish combines the partials of all virtual blocks in a fixed order and derives the scalars that
 // follow in the reference
 template <int EPI, int K>
@@ -389,6 +408,10 @@ __device__ __forceinline__ void spmv_finalize(const SpmvArgs& a, int n_local, do
 #pragma unroll
     for (int k = 0; k < K; ++k) {
         double* scal = a.scal + k * SCAL_STRIDE;
+        if (a.dist && EPI == EP_JACOBI_RES) {  // the three local totals that k_jacobi_decide reduces: sum at S_TMP0.., max at S_MAXABS
+            scal[S_TMP0] = T0[0]; scal[S_TMP1] = T2; scal[S_MAXABS] = T1[0];
+            return;
+        }
         if (a.dist) { a.scal[stage_slot<K>(0, k)] = T0[k]; a.scal[stage_slot<K>(1, k)] = T1[k]; continue; }
         if (EPI == EP_SUM_ALPHA) {
             scal[S_ALPHA] = scal[S_RHO] / T0[k];
@@ -402,17 +425,7 @@ __device__ __forceinline__ void spmv_finalize(const SpmvArgs& a, int n_local, do
             if (nrm != nrm) atomicOr(a.flags, DF_MG_NAN);
         } else if (EPI == EP_JACOBI_RES) {
             if (a.defer) { scal[S_MAXABS] = T1[0]; scal[S_TMP1] = T2; return; }
-            double r = sqrt(T0[0]);
-            scal[S_NORM] = r;
-            // `initial_residual` starts at 0 in every call (:170) and is taken at iter_num == 1 (:208, Q9)
-            const double initial = (a.iter == 0) ? 0. : scal[S_JAC_INIT];
-            if (a.iter == 1) {
-                scal[S_JAC_INIT] = r;
-            } else if (r / initial < a.threshold) {
-                atomicOr(a.flags, DF_CONVERGED);
-                return;  // `break` precedes the magnitude check (:209-216)
-            }
-            if (T2 == 0. && T1[0] > 1e10) atomicOr(a.flags, DF_JACOBI_HUGE);  // a NaN maximum compares false in the reference
+            jacobi_decide(scal, a.flags, a.iter, a.threshold, T0[0], T1[0], T2);
         }
     }
     }
@@ -912,12 +925,12 @@ CsrPtr jacobi_scale(Ctx& c, DCsr& A, const double* b, double* b_out, int K) {
 // =================================================================================================
 // Jacobi (linear_algebra.rs:172-218)
 // =================================================================================================
-__global__ void k_jacobi_prepare(int n, const int* __restrict__ rowptr, const int* __restrict__ col, const int* __restrict__ diag,
+__global__ void k_jacobi_prepare(int lo, int hi, const int* __restrict__ rowptr, const int* __restrict__ col, const int* __restrict__ diag,
                                  const double* __restrict__ val, const double* __restrict__ b, double* __restrict__ val0,
                                  double* __restrict__ b0, int* flags) {
-    // a_prime = v / a(i,i) off the diagonal, 0 on it; b_prime = b / a(i,i). a.get(i,i) panics if not stored.
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+    // a_prime = v / a(i,i) off the diagonal, 0 on it; b_prime = b / a(i,i). a.get(i,i) panics if not stored. Rows [lo, hi).
+    int i = lo + blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= hi) return;
     int d = diag[i];
     if (d < 0) { atomicOr(flags, DF_MISSING_ENTRY); return; }
     double aii = val[d];
@@ -931,7 +944,7 @@ static void jacobi(Ctx& c, DCsr& A, const double* b, double* x, const SolveParam
     csr_ensure_diag(c, A);
     CsrPtr A0 = csr_like(c, A);
     DBuf<double> b0(&c, n), xn(&c, n);
-    k_jacobi_prepare<<<(int)((n + 255) / 256), 256, 0, c.stream>>>((int)n, A.rowptr, A.col, A.diag, A.val, b, A0->val, b0, c.d_flags);
+    k_jacobi_prepare<<<(int)((n + 255) / 256), 256, 0, c.stream>>>(0, (int)n, A.rowptr, A.col, A.diag, A.val, b, A0->val, b0, c.d_flags);
     c.after_launch("k_jacobi_prepare");
     for (uint64_t it = 0; it < sp.iterations; ++it) {
         SpmvArgs a{};
@@ -2375,6 +2388,71 @@ static void bicgstab_dist(Ctx& c, DistEnv& env, const DCsr& A, const double* b, 
     }
 }
 
+// Jacobi over a row-partitioned matrix (linear_algebra.rs:172-218). The update is row-local and a partition keeps the column order
+// of every row, so the iterates are the single-GPU fast mode's bit for bit; only the residual norm that decides the break is summed
+// per rank and then across ranks. Every rank takes that decision (the latch, the magnitude check) from the same reduced bits.
+__global__ void k_jacobi_decide(double* scal, int* flags, PeerAr pa_sum, PeerAr pa_max, int iter, double threshold) {
+    if (pa_sum.nranks > 1) {   // peer path: the two allreduces in this launch (sum of r^2 and NaN rows, then max |xn|)
+        peer_allreduce_warp(pa_sum, scal + S_TMP0, 2, 0, flags);
+        peer_allreduce_warp(pa_max, scal + S_MAXABS, 1, 2, flags);
+    }
+    if (threadIdx.x != 0) return;
+    if (*(volatile int*)flags & DF_CONVERGED) return;   // latched: the residual kernel published nothing
+    jacobi_decide(scal, flags, iter, threshold, scal[S_TMP0], scal[S_MAXABS], scal[S_TMP1]);
+}
+static void jacobi_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double* x, const SolveParams& sp) {
+    const int64_t n = A.nrows;   // local cells incl. halo; halo rows are empty and store no diagonal
+    Halo& H = *env.halo;
+    Comm& cm = *env.comm;
+    const int64_t lo = H.own_lo, nown = H.own_hi - H.own_lo;
+    csr_ensure_diag(c, A);
+    CsrPtr A0 = csr_like(c, A);
+    DBuf<double> b0(&c, (size_t)std::max<int64_t>(n, 1)), xn(&c, (size_t)std::max<int64_t>(n, 1));
+    xn.zero();
+    if (nown > 0) {
+        k_jacobi_prepare<<<(int)((nown + 255) / 256), 256, 0, c.stream>>>((int)lo, (int)(lo + nown), A.rowptr, A.col, A.diag, A.val, b, A0->val, b0,
+                                                                          c.d_flags);
+        c.after_launch("k_jacobi_prepare");
+    }
+    // the owned rows as a matrix of their own: row i of the view is row lo + i (SpmvArgs::row0), columns stay local ids
+    auto owned_rows = [&](const DCsr& M) {
+        DCsr v;   // no context: the view frees nothing
+        v.nrows = nown; v.ncols = M.ncols; v.nnz = M.nnz; v.rowptr = M.rowptr + lo; v.col = M.col; v.val = M.val;
+        return v;
+    };
+    const DCsr A0v = owned_rows(*A0), Av = owned_rows(A);
+    for (uint64_t it = 0; it < sp.iterations; ++it) {
+        H.exchange(c, cm, x);
+        if (nown > 0) {
+            SpmvArgs a{};
+            a.x = x; a.y = xn; a.b = b0; a.w = sp.relaxation; a.one_minus_w = 1. - sp.relaxation; a.row0 = (int)lo;
+            launch_spmv<EP_JACOBI>(c, A0v, a);
+        }
+        H.exchange(c, cm, xn);
+        if (nown > 0) {
+            SpmvArgs r{};
+            r.x = xn; r.y2 = x; r.b = b; r.dist = 1; r.row0 = (int)lo;
+            launch_spmv<EP_JACOBI_RES>(c, Av, r);
+        } else {
+            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_TMP0, 0, 2 * sizeof(double), c.stream));   // a rank without cells adds nothing
+            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_MAXABS, 0, sizeof(double), c.stream));
+        }
+        PeerAr ps, pm;   // nranks == 1: NCCL has reduced the totals already
+        if (cm.peer.on) {
+            ps = cm.next_allreduce();
+            pm = cm.next_allreduce();
+        } else {
+            cm.allreduce(c, c.d_scal + S_TMP0, 2, 0);
+            cm.allreduce(c, c.d_scal + S_MAXABS, 1, 2);
+        }
+        ProfScope pscope(c, PC_OTHER, 0.);
+        k_jacobi_decide<<<1, 32, 0, c.stream>>>(c.d_scal, c.d_flags, ps, pm, (int)it, sp.threshold);
+        c.after_launch("k_jacobi_decide");
+    }
+    k_clear_latch<<<1, 1, 0, c.stream>>>(c.d_flags);
+    c.after_launch("k_clear_latch");
+}
+
 // rows/columns [lo, hi) of A as a standalone CSR with indices shifted to 0 (the rank's diagonal block)
 __global__ void k_block_counts(int lo, int hi, const int* __restrict__ rowptr, const int* __restrict__ col, int* cnt) {
     int i = lo + blockIdx.x * blockDim.x + threadIdx.x;
@@ -2440,6 +2518,7 @@ void iterative_solve_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double
         bp = b_tmp;
     }
     switch (sp.method) {
+        case ORC_SOLVER_JACOBI: jacobi_dist(c, env, *Ap, bp, x, sp); break;
         case ORC_SOLVER_BICGSTAB:
             if (K == 1) bicgstab_dist<1>(c, env, *Ap, bp, x, sp.iterations);
             else bicgstab_dist<3>(c, env, *Ap, bp, x, sp.iterations);
@@ -2462,7 +2541,7 @@ void iterative_solve_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double
             dev_axpy_inplace(c, x + H.own_lo * S, corr, nown * S);
             break;
         }
-        default: throw Error(ORC_E_UNSUPPORTED, "multi-GPU solves support BiCGSTAB and Multigrid");
+        default: throw Error(ORC_E_UNSUPPORTED, "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid");
     }
 }
 

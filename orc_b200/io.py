@@ -50,18 +50,33 @@ def _vector_display(x, y, z):   # impl Display for Vector (src/lib.rs:551-556)
     return f"({_rust_exp(x, 2)}, {_rust_exp(y, 2)}, {_rust_exp(z, 2)})"
 
 
+def _owned_centroids(mesh):
+    """Cell centroids of the cells a caller holds fields for: the owned cells of a partition mesh (its local cells are
+    [lower halo | owned | upper halo]), all cells otherwise."""
+    cc = mesh.export()["cell_centroid"]
+    try:
+        info = mesh.partition_info()
+    except _lib.OrcError:
+        return cc
+    return cc[info["n_lo"]:info["n_lo"] + info["n_own"]]
+
+
 def write_data(mesh, u, v, w, p, output_file_name, decimal_precision=None):
     """write_data (src/io.rs:572-591) / write_data_with_precision (:593-619) when `decimal_precision` is given: one line per cell,
-    `centroid \\t (u, v, w) \\t p`."""
+    `centroid \\t (u, v, w) \\t p`. On a partition mesh the fields are the owned cells' and so are the lines: the rank files,
+    concatenated in rank order, are the whole mesh's file."""
     import numpy as np
-    cc = mesh.export()["cell_centroid"].tolist()
+    cc = _owned_centroids(mesh).tolist()
+    n = len(cc)
     cols = [np.asarray(a, dtype=np.float64).tolist() for a in (u, v, w, p)]
+    if any(len(c) != n for c in cols):
+        raise ValueError(f"u, v, w, p must hold {n} values, one per (owned) cell")
     e, prec = _rust_exp, decimal_precision
     if decimal_precision is None:
         print(f"Writing data to {output_file_name}...")
     with open(output_file_name, "w") as f:
-        for lo in range(0, mesh.n_cells, 65536):          # plain Python floats and one write per block: the loop is the cost at 10^6+ cells
-            hi = min(lo + 65536, mesh.n_cells)
+        for lo in range(0, n, 65536):          # plain Python floats and one write per block: the loop is the cost at 10^6+ cells
+            hi = min(lo + 65536, n)
             f.write("".join(f"({e(c[0], 2)}, {e(c[1], 2)}, {e(c[2], 2)})\t({e(a, prec)}, {e(b, prec)}, {e(g, prec)})\t{e(d, prec)}\n"
                             for c, a, b, g, d in zip(cc[lo:hi], cols[0][lo:hi], cols[1][lo:hi], cols[2][lo:hi], cols[3][lo:hi])))
     if decimal_precision is None:
@@ -81,8 +96,12 @@ def write_gradients(mesh, u, v, w, p, output_file_name, decimal_precision, gradi
     gradients come from the device (orc_gradients), Green-Gauss cell based or least squares."""
     from .discretization import calculate_gradients
     gp, gu = calculate_gradients(mesh, u, v, w, p, gradient_scheme, ctx)
-    n = mesh.n_cells
-    cc, gul, gpl = mesh.export()["cell_centroid"].tolist(), gu.reshape(n, 9).tolist(), gp.tolist()
+    _write_gradient_lines(output_file_name, mesh.export()["cell_centroid"], gp, gu, decimal_precision)
+
+
+def _write_gradient_lines(output_file_name, centroids, gp, gu, decimal_precision):
+    n = len(centroids)
+    cc, gul, gpl = centroids.tolist(), gu.reshape(n, 9).tolist(), gp.tolist()
     print(f"Writing data to {output_file_name}...")
     with open(output_file_name, "w") as f:
         for lo in range(0, n, 65536):

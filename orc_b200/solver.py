@@ -8,6 +8,14 @@ from .context import default_context
 from .mesh import _f64, _p
 
 
+def _exposed_cells(mesh):
+    """The cells a call exchanges with the caller: the owned cells of a partition mesh, all cells otherwise."""
+    try:
+        return mesh.partition_info()["n_own"]
+    except _lib.OrcError:
+        return mesh.n_cells
+
+
 def solve_steady(mesh, u, v, w, p, numerical_settings, rho, mu, iteration_count, reporting_interval, ctx=None, on_report=None):
     """Same argument order as the reference. u, v, w, p are numpy float64 vectors updated IN PLACE (the reference's
     &mut DVector). Reports (the line printed at src/solver.rs:213-215) go to `on_report(dict)`; default prints them."""
@@ -15,10 +23,7 @@ def solve_steady(mesh, u, v, w, p, numerical_settings, rho, mu, iteration_count,
     mesh._bind(ctx)
     s = numerical_settings.to_c()
     arrs = [u, v, w, p]
-    try:
-        n_expected = mesh.partition_info()["n_own"]   # a partition mesh exchanges its OWNED cells with the caller
-    except _lib.OrcError:
-        n_expected = mesh.n_cells
+    n_expected = _exposed_cells(mesh)
     for a in arrs:
         if not (isinstance(a, np.ndarray) and a.dtype == np.float64 and a.flags.c_contiguous and a.size == n_expected):
             raise ValueError("u, v, w, p must be contiguous float64 arrays of length n_cells")
@@ -55,10 +60,11 @@ def check_boundary_conditions(mesh):
 
 def initialize_flow(mesh, mu, rho, iteration_count, ctx=None, reduction_mode=0):
     """src/solver.rs:246-352, same argument order; returns (u, v, w, p). `reduction_mode`: settings.ReductionMode (the reference
-    has no such knob: ReferenceOrder makes the result bit-identical to its CPU path, Fast is the throughput mode)."""
+    has no such knob: ReferenceOrder makes the result bit-identical to its CPU path, Fast is the throughput mode). On a partition
+    mesh every rank calls it with its own context and gets the fields of its owned cells."""
     ctx = ctx or default_context()
     mesh._bind(ctx)
-    n = mesh.n_cells
+    n = _exposed_cells(mesh)
     u, v, w, p = (np.zeros(n) for _ in range(4))
     print("Initializing pressure field...")
     print("Initializing velocity field...")
@@ -72,10 +78,11 @@ def initialize_flow_new(mesh, mu, rho, iteration_count, ctx=None, reduction_mode
     """src/solver.rs:354-410, same argument order; returns (u, v, w, p). What the reference's current main() calls before
     solve_steady (src/tests.rs:195-197): the Laplace pressure field for PressureOnly / Hybrid boundary-condition systems (the
     overlapping match arm: a Hybrid system gets no velocity field), initialize_velocity_field (:511-696) for VelocityOnly ones.
-    `reduction_mode`: settings.ReductionMode (default Auto)."""
+    `reduction_mode`: settings.ReductionMode (default Auto). On a partition mesh every rank calls it with its own context and gets
+    the fields of its owned cells."""
     ctx = ctx or default_context()
     mesh._bind(ctx)
-    n = mesh.n_cells
+    n = _exposed_cells(mesh)
     u, v, w, p = (np.zeros(n) for _ in range(4))
     print("Initializing flow...")
     _lib.check(_lib.lib().orc_initialize_flow_new(ctx.handle, mesh.handle, C.c_double(mu), C.c_double(rho), C.c_uint64(iteration_count),
@@ -94,11 +101,7 @@ class SteadySolver:
         self._h = C.c_void_p()
         _lib.check(_lib.lib().orc_steady_create(self.ctx.handle, mesh.handle, C.byref(self._s), C.c_double(rho), C.c_double(mu),
                                                 C.byref(self._h)))
-        self.n = mesh.n_cells
-        try:
-            self.n = mesh.partition_info()["n_own"]   # a partition exposes its owned cells
-        except _lib.OrcError:
-            pass
+        self.n = _exposed_cells(mesh)
 
     def set_fields(self, u, v, w, p):
         u, v, w, p = _f64(u), _f64(v), _f64(w), _f64(p)
@@ -113,6 +116,20 @@ class SteadySolver:
         rep = _lib.Report()
         _lib.check(_lib.lib().orc_steady_iterate(self._h, C.c_uint64(iterations), C.byref(rep)))
         return {k: getattr(rep, k) for k, _ in _lib.Report._fields_}
+
+    def gradients(self, gradient_scheme=0):
+        """discretization.calculate_gradients of the resident fields -> ((n, 3), (n, 3, 3)), n = the exposed (owned) cells. On a
+        partition mesh every rank calls it together (the fields' halo cells are exchanged first)."""
+        gp, gu = np.zeros((self.n, 3)), np.zeros((self.n, 3, 3))
+        _lib.check(_lib.lib().orc_steady_gradients(self._h, C.c_int32(int(gradient_scheme)), _p(gp), _p(gu)))
+        return gp, gu
+
+    def write_gradients(self, output_file_name, decimal_precision, gradient_scheme):
+        """io.write_gradients of the resident fields. A partition writes the lines of its owned cells: the rank files, concatenated
+        in rank order, are the whole mesh's file."""
+        from .io import _owned_centroids, _write_gradient_lines
+        gp, gu = self.gradients(gradient_scheme)
+        _write_gradient_lines(output_file_name, _owned_centroids(self.mesh), gp, gu, decimal_precision)
 
     def reset(self):
         """Back to the state solve_steady starts from: zero fields, momentum matrices re-initialised (diag 1)."""

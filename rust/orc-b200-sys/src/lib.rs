@@ -46,6 +46,8 @@ extern "C" {
     // initialize_flow (src/solver.rs:246-352); reduction_mode: 0 = ORC_REDUCE_FAST, 1 = ORC_REDUCE_REFERENCE_ORDER
     pub fn orc_initialize_flow(ctx: *mut orc_ctx, m: *mut orc_mesh, mu: f64, rho: f64, iteration_count: u64, reduction_mode: i32,
         u: *mut f64, v: *mut f64, w: *mut f64, p: *mut f64) -> i32;
+    // calculate_*_gradient (src/solver.rs:774-949) of the steady handle's resident fields: n x 3 and n x 9 row-major, either may be null
+    pub fn orc_steady_gradients(st: *mut orc_steady, gradient: i32, grad_p3n: *mut f64, grad_u9n: *mut f64) -> i32;
     // check_boundary_conditions (src/solver.rs:710-770): 0 PressureOnly, 1 VelocityOnly, 2 Hybrid
     pub fn orc_check_boundary_conditions(m: *const orc_mesh, constraint_type: *mut i32) -> i32;
 }
