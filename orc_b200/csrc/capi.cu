@@ -123,6 +123,61 @@ struct orc_steady {
     }
 };
 
+// The DistEnv of a partition mesh whose device mirror exists on ctx: the plan must match the communicator. With several ranks, all
+// of them agree on the peer path (collective) and `work`'s assembly exchanges its halo cells.
+static DistEnv partition_env(orc_ctx* ctx, orc_mesh* m, AsmWork* work) {
+    Ctx& c = ctx->c;
+    require(ctx->comm.nranks == m->plan->nranks && ctx->comm.rank == m->plan->rank, "partition mesh does not match the context's communicator");
+    DistEnv env;
+    env.comm = &ctx->comm; env.halo = m->dev[&c].halo.get();
+    if (env.on()) {
+        env.halo->agree_on_peer(c, ctx->comm);
+        Comm* cm = env.comm; Halo* hl = env.halo; Ctx* cp = &c;
+        if (work) work->halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); };
+    }
+    return env;
+}
+// fills the halo cells of up to Halo::kMaxFields vectors from their owners on a partition; nothing on one GPU
+static void exchange(Ctx& c, const DistEnv& env, std::initializer_list<double*> fields) {
+    if (!env.on()) return;
+    double* f[Halo::kMaxFields]; int k = 0;
+    for (double* q : fields) f[k++] = q;
+    env.halo->exchange(c, *env.comm, f, k);
+}
+static double allreduce_host(Ctx& c, Comm& cm, double v, int op) {
+    if (!cm.active()) return v;
+    DBuf<double> d(&c, 1);
+    ORC_CUDA(cudaMemcpyAsync(d.p, &v, sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    cm.allreduce(c, d.p, 1, op);
+    ORC_CUDA(cudaMemcpyAsync(&v, d.p, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
+    c.sync();
+    return v;
+}
+
+// The three momentum systems (matrices a, b, c3) are independent (solver.rs:99-136 reads only what the assembly wrote) and, unless the
+// scheme is TVD, their matrices are bit-identical (a_nb.x == a_nb.y == a_nb.z, discretization.rs:217-232): solve them in lockstep with
+// ONE pass over the matrix and ONE AMG hierarchy. Verified on the device on every call; on a partition every rank must take the same
+// branch (the solves contain collectives), so the ranks agree on it (min). ORC_B200_BATCH=0 switches it off (A/B runs, tests).
+static bool lockstep_enabled() {
+    const char* e = getenv("ORC_B200_BATCH");
+    return !(e && atoi(e) == 0);
+}
+static bool lockstep(Ctx& c, const DistEnv& env, bool enabled, const SolveParams& sp, const DCsr& a, const DCsr& b, const DCsr& c3) {
+    if (!solve_batchable(sp)) return false;
+    double same = (enabled && csr_values_identical(c, a, b) && csr_values_identical(c, a, c3)) ? 1. : 0.;
+    if (env.on()) same = allreduce_host(c, *env.comm, same, 3);
+    return same == 1.;
+}
+// the K = 3 solve of a x_k = b_k, k = u, v, w, on interleaved cells (linalg.cu: Cell<3>)
+static void solve_lockstep(Ctx& c, const DistEnv& env, DCsr& a, const double* bu, const double* bv, const double* bw, double* u, double* v,
+                           double* w, int64_t N, const SolveParams& sp) {
+    DBuf<double> b4(&c, (size_t)std::max<int64_t>(N, 1) * 4), x4(&c, (size_t)std::max<int64_t>(N, 1) * 4);
+    pack3(c, N, bu, bv, bw, b4);
+    pack3(c, N, u, v, w, x4);
+    iterative_solve(c, a, b4, x4, sp, nullptr, 3, &env);
+    unpack3(c, N, x4, u, v, w);
+}
+
 static orc_steady* steady_create(orc_ctx* octx, orc_mesh* m, const orc_settings* s, double rho, double mu) {
     Ctx& c = octx->c;
     require(s != nullptr, "null settings");
@@ -131,17 +186,12 @@ static orc_steady* steady_create(orc_ctx* octx, orc_mesh* m, const orc_settings*
     std::unique_ptr<orc_steady> st(new orc_steady());
     st->c = &c; st->octx = octx; st->mesh = m; st->dm = &d; st->s = *s; st->rho = rho; st->mu = mu; st->N = d.N; st->N_global = d.N;
     if (m->plan) {
-        require(octx->comm.nranks == m->plan->nranks && octx->comm.rank == m->plan->rank, "partition mesh does not match the context's communicator");
         st->N_global = m->plan->n_global;
-        st->env.comm = &octx->comm; st->env.halo = m->dev[&c].halo.get();
-        if (st->env.on()) {
-            // Gauss-Seidel's sweep is one dependency chain over all rows: it has no partitioned form
+        st->env = partition_env(octx, m, &st->work);
+        // Gauss-Seidel's sweep is one dependency chain over all rows: it has no partitioned form
+        if (st->env.on())
             require(s->solver_type == ORC_SOLVER_JACOBI || s->solver_type == ORC_SOLVER_BICGSTAB || s->solver_type == ORC_SOLVER_MULTIGRID,
                     "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid");
-            st->env.halo->agree_on_peer(c, octx->comm);
-            Comm* cm = st->env.comm; Halo* hl = st->env.halo; Ctx* cp = &c;
-            st->work.halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); };
-        }
     }
     const size_t N = (size_t)std::max<int64_t>(d.N, 1);
     for (DBuf<double>* b : {&st->b_u_di, &st->b_v_di, &st->b_w_di, &st->b_u, &st->b_v, &st->b_w, &st->pc_b, &st->p_prime, &st->du, &st->dv,
@@ -150,7 +200,7 @@ static orc_steady* steady_create(orc_ctx* octx, orc_mesh* m, const orc_settings*
         b->zero();  // halo entries of a partition are never written by the assembly kernels
     }
     st->scal.alloc(&c, 16);
-    if (const char* e = getenv("ORC_B200_BATCH")) st->batch_momentum = (atoi(e) != 0);
+    st->batch_momentum = lockstep_enabled();
     st->a_di = mesh_matrix(c, d); st->a_u = mesh_matrix(c, d); st->a_v = mesh_matrix(c, d); st->a_w = mesh_matrix(c, d); st->pc_a = mesh_matrix(c, d);
     build_momentum_diffusion(c, d, mu, *st->a_di, st->b_u_di, st->b_v_di, st->b_w_di);                  // solver.rs:41-42
     init_momentum_matrix(c, d, *st->a_u); init_momentum_matrix(c, d, *st->a_v); init_momentum_matrix(c, d, *st->a_w);  // :43-45
@@ -191,55 +241,31 @@ static void steady_iterate(orc_steady& st, uint64_t iterations, uint64_t report_
         const uint64_t iter_number = ++st.iteration;
         ORC_CUDA(cudaEventRecord(st.ev[0], c.stream));
         const bool dist = st.env.on();
-        auto xch = [&](std::initializer_list<double*> f) {
-            if (!dist) return;
-            double* a[4]; int k = 0;
-            for (double* q : f) a[k++] = q;
-            st.env.halo->exchange(c, *st.env.comm, a, k);
-        };
-        xch({st.u.p, st.v.p, st.w.p, st.p.p});                                                             // C1: neighbours' fields
+        exchange(c, st.env, {st.u.p, st.v.p, st.w.p, st.p.p});                                              // C1: neighbours' fields
         int pid = c.prof_begin(PC_ASSEMBLY, 0.);
         build_momentum_advection(c, d, st.work, as, st.rho, *st.a_u, *st.a_v, *st.a_w, *st.a_di, st.du, st.dv, st.dw, st.u, st.v, st.w, st.p,
                                  st.b_u, st.b_v, st.b_w, st.scal.p + 8);                                   // solver.rs:61-79
         dev_axpy_inplace(c, st.b_u, st.b_u_di, N); dev_axpy_inplace(c, st.b_v, st.b_v_di, N); dev_axpy_inplace(c, st.b_w, st.b_w_di, N);  // :80-82
         c.prof_end(pid);
-        xch({st.du.p, st.dv.p, st.dw.p});  // new diagonals for the pressure system; they are the "old" state of the next assembly (C4)
+        exchange(c, st.env, {st.du.p, st.dv.p, st.dw.p});  // new diagonals for the pressure system; the "old" state of the next assembly (C4)
         ORC_CUDA(cudaEventRecord(st.ev[1], c.stream));
-        // The three momentum systems are independent (solver.rs:99-136 reads only what the assembly wrote) and, unless the
-        // scheme is TVD, their matrices are bit-identical (a_nb.x == a_nb.y == a_nb.z, discretization.rs:217-232): solve them
-        // in lockstep with ONE pass over the matrix and ONE AMG hierarchy. Verified on the device every iteration.
-        bool batch3 = st.batch_momentum && solve_batchable(sp);
-        if (batch3) {
-            double same = (csr_values_identical(c, *st.a_u, *st.a_v) && csr_values_identical(c, *st.a_u, *st.a_w)) ? 1. : 0.;
-            if (dist) {  // every rank must take the same branch: the solves contain collectives
-                ORC_CUDA(cudaMemcpyAsync(st.scal.p + 11, &same, sizeof(double), cudaMemcpyHostToDevice, c.stream));
-                st.env.comm->allreduce(c, st.scal.p + 11, 1, 3);
-                ORC_CUDA(cudaMemcpyAsync(&same, st.scal.p + 11, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-                c.sync();
-            }
-            batch3 = (same == 1.);
-        }
-        st.last_batched = batch3;
-        if (batch3) {
-            DBuf<double> b4(&c, (size_t)std::max<int64_t>(N, 1) * 4), x4(&c, (size_t)std::max<int64_t>(N, 1) * 4);
-            pack3(c, N, st.b_u, st.b_v, st.b_w, b4);
-            pack3(c, N, st.u, st.v, st.w, x4);
-            iterative_solve_dist(c, st.env, *st.a_u, b4, x4, sp, nullptr, 3);
-            unpack3(c, N, x4, st.u, st.v, st.w);
+        st.last_batched = lockstep(c, st.env, st.batch_momentum, sp, *st.a_u, *st.a_v, *st.a_w);
+        if (st.last_batched) {
+            solve_lockstep(c, st.env, *st.a_u, st.b_u, st.b_v, st.b_w, st.u, st.v, st.w, N, sp);
         } else {
-            iterative_solve_dist(c, st.env, *st.a_u, st.b_u, st.u, sp, nullptr);                            // :99-110
-            iterative_solve_dist(c, st.env, *st.a_v, st.b_v, st.v, sp, nullptr);                            // :112-123
-            iterative_solve_dist(c, st.env, *st.a_w, st.b_w, st.w, sp, nullptr);                            // :125-136
+            iterative_solve(c, *st.a_u, st.b_u, st.u, sp, nullptr, 1, &st.env);                            // :99-110
+            iterative_solve(c, *st.a_v, st.b_v, st.v, sp, nullptr, 1, &st.env);                            // :112-123
+            iterative_solve(c, *st.a_w, st.b_w, st.w, sp, nullptr, 1, &st.env);                            // :125-136
         }
-        xch({st.u.p, st.v.p, st.w.p});
+        exchange(c, st.env, {st.u.p, st.v.p, st.w.p});
         ORC_CUDA(cudaEventRecord(st.ev[2], c.stream));
         pid = c.prof_begin(PC_ASSEMBLY, 0.);
         build_pressure_correction(c, d, st.work, as, st.rho, st.du, st.dv, st.dw, st.u, st.v, st.w, st.p, *st.pc_a, st.pc_b);  // :137-148
         c.prof_end(pid);
         ORC_CUDA(cudaEventRecord(st.ev[3], c.stream));
         dev_scale(c, st.p_prime, 0., N);                                                                   // p_prime *= 0.  (:167)
-        iterative_solve_dist(c, st.env, *st.pc_a, st.pc_b, st.p_prime, sp, &st.trace);                      // :168-179
-        xch({st.p_prime.p});
+        iterative_solve(c, *st.pc_a, st.pc_b, st.p_prime, sp, &st.trace, 1, &st.env);                     // :168-179
+        exchange(c, st.env, {st.p_prime.p});
         ORC_CUDA(cudaEventRecord(st.ev[4], c.stream));
         apply_pressure_correction(c, d, st.du, st.dv, st.dw, st.p_prime, st.u, st.v, st.w, st.p, st.s.pressure_relaxation,
                                   st.s.momentum_relaxation, st.scal.p);                                    // :193-204
@@ -966,15 +992,6 @@ int32_t orc_build_pressure_laplace(orc_ctx* ctx, orc_mesh* m, orc_csr** a_out, d
     });
 }
 // ---- the initialisation on a partition mesh: every rank runs the same steps on its owned cells, collectives in lockstep ----
-static double allreduce_host(Ctx& c, Comm& cm, double v, int op) {
-    if (!cm.active()) return v;
-    DBuf<double> d(&c, 1);
-    ORC_CUDA(cudaMemcpyAsync(d.p, &v, sizeof(double), cudaMemcpyHostToDevice, c.stream));
-    cm.allreduce(c, d.p, 1, op);
-    ORC_CUDA(cudaMemcpyAsync(&v, d.p, sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-    c.sync();
-    return v;
-}
 // check_solver_flags with the status word of all ranks: some flags are local (a singular least-squares fit on one rank), and every
 // rank must return the same status (and stay in the collectives together)
 static void check_agreed_flags(Ctx& c, const DistEnv& env) {
@@ -996,8 +1013,8 @@ struct InitEnv {
     int64_t lo = 0, n_own = 0;   // the cells the caller receives
 };
 // What both initialisations do first: the boundary-condition check over the WHOLE mesh (a partition counts the faces whose c0 it
-// owns, so that every face is counted once), the reduction mode, and the halo plan of a partition.
-static InitEnv init_env(orc_ctx* ctx, orc_mesh* m, int reduction_mode) {
+// owns, so that every face is counted once), the reduction mode, and the halo plan of a partition (its hook goes into `work`).
+static InitEnv init_env(orc_ctx* ctx, orc_mesh* m, int reduction_mode, AsmWork* work) {
     Ctx& c = ctx->c;
     InitEnv ie;
     const HostMesh& h = *m->h;
@@ -1008,22 +1025,14 @@ static InitEnv init_env(orc_ctx* ctx, orc_mesh* m, int reduction_mode) {
         ie.n_own = d.N;
         return ie;
     }
-    require(ctx->comm.nranks == m->plan->nranks && ctx->comm.rank == m->plan->rank, "partition mesh does not match the context's communicator");
     if (reduction_mode == ORC_REDUCE_REFERENCE_ORDER) throw Error(ORC_E_UNSUPPORTED, "reference-order reductions are single-GPU only");
     DMesh& d = device_mesh(c, m);
-    ie.env.comm = &ctx->comm; ie.env.halo = m->dev[&c].halo.get();
-    if (ie.env.on()) ie.env.halo->agree_on_peer(c, ctx->comm);
+    ie.env = partition_env(ctx, m, work);
     int64_t own_faces = 0;
     for (int64_t f = 0; f < h.n_faces; ++f) own_faces += (h.face_c0[f] >= d.own_lo && h.face_c0[f] < d.own_hi);
     ie.constraint = check_boundary_conditions(h, (int64_t)allreduce_host(c, ctx->comm, (double)own_faces, 0));
     ie.lo = d.own_lo; ie.n_own = d.own_hi - d.own_lo;
     return ie;
-}
-static void xch(Ctx& c, const InitEnv& ie, std::initializer_list<double*> f) {
-    if (!ie.env.on()) return;
-    double* a[Halo::kMaxFields]; int k = 0;
-    for (double* q : f) a[k++] = q;
-    ie.env.halo->exchange(c, *ie.env.comm, a, k);
 }
 
 // initialize_flow (:246-352): Laplace pressure field (Jacobi x10), one UD / LinearWeighted momentum assembly at rest, then six
@@ -1035,8 +1044,9 @@ int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, ui
         require(ctx && m && u && v && w && p, "null argument");
         Ctx& c = ctx->c;
         c.clear_flags();
-        const InitEnv ie = init_env(ctx, m, reduction_mode);                                                 // :272
-        DistEnv env = ie.env;
+        AsmWork work;
+        const InitEnv ie = init_env(ctx, m, reduction_mode, &work);                                          // :272
+        const DistEnv& env = ie.env;
         DMesh& d = device_mesh(c, m);
         const int64_t N = d.N;
         const size_t Nz = (size_t)std::max<int64_t>(N, 1);
@@ -1053,34 +1063,26 @@ int32_t orc_initialize_flow(orc_ctx* ctx, orc_mesh* m, double mu, double rho, ui
         // initialize_pressure_field (:414-509)
         build_pressure_laplace(c, d, *lap, pb);
         sp.iterations = 10; sp.method = ORC_SOLVER_JACOBI; sp.relaxation = 0.1; sp.threshold = 1e-6; sp.preconditioner = ORC_PC_JACOBI;
-        iterative_solve_dist(c, env, *lap, pb, dp, sp, nullptr);                                            // :498-507
+        iterative_solve(c, *lap, pb, dp, sp, nullptr, 1, &env);                                             // :498-507
         check_agreed_flags(c, env);
         // :288-306: UD, LinearWeighted velocity and pressure interpolation, Green-Gauss cell based; u = v = w = 0
         AsmSettings as;
         as.momentum = ORC_MOM_UD; as.limiter = ORC_PSI_UD; as.p_interp = ORC_P_LINEAR_WEIGHTED; as.v_interp = ORC_V_LINEAR_WEIGHTED;
         as.gradient = ORC_G_GREEN_GAUSS_CELL; as.assembly_mode = ORC_ASSEMBLY_EXACT;
-        AsmWork work;
-        if (env.on()) { Comm* cm = env.comm; Halo* hl = env.halo; Ctx* cp = &c; work.halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); }; }
-        xch(c, ie, {dp.p});                                                                                // the neighbours' pressure
+        exchange(c, env, {dp.p});                                                                          // the neighbours' pressure
         build_momentum_advection(c, d, work, as, rho, *a_u, *a_v, *a_w, *a_di, diag_u, diag_v, diag_w, du, dv, dw, dp, b_u, b_v, b_w, pe3);
         dev_axpy_inplace(c, b_u, b_u_di, N); dev_axpy_inplace(c, b_v, b_v_di, N); dev_axpy_inplace(c, b_w, b_w_di, N);  // :307-309
         sp.iterations = iteration_count; sp.method = ORC_SOLVER_BICGSTAB; sp.relaxation = 0.5; sp.threshold = 1e-6;
-        bool lockstep = solve_batchable(sp) && csr_values_identical(c, *a_u, *a_v) && csr_values_identical(c, *a_u, *a_w) &&
-                        !(getenv("ORC_B200_BATCH") && atoi(getenv("ORC_B200_BATCH")) == 0);
-        if (env.on()) lockstep = allreduce_host(c, *env.comm, lockstep ? 1. : 0., 3) == 1.;   // the solves hold collectives: one branch for all
+        const bool batch3 = lockstep(c, env, lockstep_enabled(), sp, *a_u, *a_v, *a_w);
         double f = 1.;
         while (f >= 0.) {                                                                                  // :316-350
-            if (lockstep) {
+            if (batch3) {
                 csr_blend(c, *a_u, 1. - f, *a_di, f, *blend);
-                DBuf<double> b4(&c, Nz * 4), x4(&c, Nz * 4);
-                pack3(c, N, b_u, b_v, b_w, b4);
-                pack3(c, N, du, dv, dw, x4);
-                iterative_solve_dist(c, env, *blend, b4, x4, sp, nullptr, 3);
-                unpack3(c, N, x4, du, dv, dw);
+                solve_lockstep(c, env, *blend, b_u, b_v, b_w, du, dv, dw, N, sp);
             } else {
-                csr_blend(c, *a_u, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_u, du, sp, nullptr);
-                csr_blend(c, *a_v, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_v, dv, sp, nullptr);
-                csr_blend(c, *a_w, 1. - f, *a_di, f, *blend); iterative_solve_dist(c, env, *blend, b_w, dw, sp, nullptr);
+                csr_blend(c, *a_u, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_u, du, sp, nullptr, 1, &env);
+                csr_blend(c, *a_v, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_v, dv, sp, nullptr, 1, &env);
+                csr_blend(c, *a_w, 1. - f, *a_di, f, *blend); iterative_solve(c, *blend, b_w, dw, sp, nullptr, 1, &env);
             }
             f -= 0.2;
         }
@@ -1127,8 +1129,8 @@ int32_t orc_initialize_flow_new(orc_ctx* ctx, orc_mesh* m, double mu, double rho
         (void)mu; (void)rho; (void)iteration_count;   // unused by the reference as well (:354-358, `_iteration_count` :414)
         Ctx& c = ctx->c;
         c.clear_flags();
-        const InitEnv ie = init_env(ctx, m, reduction_mode);                                               // :395
-        DistEnv env = ie.env;
+        const InitEnv ie = init_env(ctx, m, reduction_mode, nullptr);                                      // :395
+        const DistEnv& env = ie.env;
         DMesh& d = device_mesh(c, m);
         const int64_t N = d.N;
         const size_t Nz = (size_t)std::max<int64_t>(N, 1);
@@ -1141,12 +1143,12 @@ int32_t orc_initialize_flow_new(orc_ctx* ctx, orc_mesh* m, double mu, double rho
         if (ie.constraint == ORC_CONSTRAINT_PRESSURE_ONLY || ie.constraint == ORC_CONSTRAINT_HYBRID) {      // :399-402
             build_pressure_laplace(c, d, *a, rhs);
             sp.method = ORC_SOLVER_JACOBI;
-            iterative_solve_dist(c, env, *a, rhs, dp, sp, nullptr);                                        // :498-507
+            iterative_solve(c, *a, rhs, dp, sp, nullptr, 1, &env);                                         // :498-507
         } else {                                                                                           // :403-405
             build_velocity_potential(c, d, *a, rhs);
             sp.method = ORC_SOLVER_BICGSTAB;
-            iterative_solve_dist(c, env, *a, rhs, psi, sp, nullptr);                                       // :592-601
-            xch(c, ie, {psi.p});                                                                           // the neighbours' psi
+            iterative_solve(c, *a, rhs, psi, sp, nullptr, 1, &env);                                        // :592-601
+            exchange(c, env, {psi.p});                                                                     // the neighbours' psi
             potential_gradient(c, d, psi, du, dv, dw);                                                     // :624-693
         }
         to_host(c, u, du + ie.lo, ie.n_own); to_host(c, v, dv + ie.lo, ie.n_own); to_host(c, w, dw + ie.lo, ie.n_own); to_host(c, p, dp + ie.lo, ie.n_own);
@@ -1202,10 +1204,7 @@ int32_t orc_steady_gradients(orc_steady* st, int32_t gradient, double* grad_p3n,
         Ctx& c = *st->c;
         DMesh& d = device_mesh(c, st->mesh);
         c.clear_flags();
-        if (st->env.on()) {   // the neighbours' u, v, w, p (the handle's halo cells hold whatever the last exchange left)
-            double* f[4] = {st->u.p, st->v.p, st->w.p, st->p.p};
-            st->env.halo->exchange(c, *st->env.comm, f, 4);
-        }
+        exchange(c, st->env, {st->u.p, st->v.p, st->w.p, st->p.p});   // the halo cells hold whatever the last exchange left
         gradients_to_host(c, d, st->u, st->v, st->w, st->p, gradient, d.own_lo, d.own_hi - d.own_lo, grad_p3n, grad_u9n);
         check_agreed_flags(c, st->env);
     });

@@ -255,44 +255,32 @@ void Halo::build(Ctx& c, const PartPlan& p) {
     c.sync();
 }
 
-void Halo::exchange(Ctx& c, Comm& comm, double* const* fields, int nfields) {
+void Halo::exchange(Ctx& c, Comm& comm, double* const* fields, int nfields, int stride) {
+    ORC_REQUIRE(stride == 1 || stride == 4, ORC_E_INTERNAL, "halo exchange: cells hold 1 or 4 doubles");
     if (!comm.active() || nbr.empty()) return;
-    ORC_REQUIRE(nfields >= 1 && nfields <= kMaxFields, ORC_E_INVALID, "halo exchange: too many fields");
+    ORC_REQUIRE(nfields >= 1 && nfields * stride <= kMaxFields, ORC_E_INVALID, "halo exchange: too many fields");
     ProfScope ps(c, PC_OTHER, 0.);
-    if (exchange_peer(c, comm, fields, nfields, 1)) return;
+    if (exchange_peer(c, comm, fields, nfields, stride)) return;
     const int ns = send_ptr.back();
     for (int f = 0; f < nfields; ++f) {
-        k_halo_pack<<<grid_for(std::max(ns, 1), 256, c.sm_count * 4), 256, 0, c.stream>>>(ns, send_idx, fields[f], sendbuf.p + (size_t)f * ns);
-        c.after_launch("k_halo_pack");
+        double* out = sendbuf.p + (size_t)f * ns * stride;
+        if (stride == 1) {
+            k_halo_pack<<<grid_for(std::max(ns, 1), 256, c.sm_count * 4), 256, 0, c.stream>>>(ns, send_idx, fields[f], out);
+            c.after_launch("k_halo_pack");
+        } else {
+            k_halo_pack4<<<grid_for(std::max(ns, 1), 256, c.sm_count * 4), 256, 0, c.stream>>>(ns, send_idx, fields[f], out);
+            c.after_launch("k_halo_pack4");
+        }
     }
     Nccl& n = nccl();
     nccl_check(n.group_start(), "ncclGroupStart");
     for (int f = 0; f < nfields; ++f)
         for (size_t q = 0; q < nbr.size(); ++q) {
-            const int cnt = send_ptr[q + 1] - send_ptr[q];
-            if (cnt > 0) nccl_check(n.send(sendbuf.p + (size_t)f * ns + send_ptr[q], (size_t)cnt, kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclSend");
-            if (recv_count[q] > 0) nccl_check(n.recv(fields[f] + recv_begin[q], (size_t)recv_count[q], kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclRecv");
+            const size_t cnt = (size_t)(send_ptr[q + 1] - send_ptr[q]) * stride, rcnt = (size_t)recv_count[q] * stride;
+            double* out = sendbuf.p + ((size_t)f * ns + send_ptr[q]) * stride;
+            if (cnt > 0) nccl_check(n.send(out, cnt, kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclSend");
+            if (rcnt > 0) nccl_check(n.recv(fields[f] + (size_t)recv_begin[q] * stride, rcnt, kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclRecv");
         }
-    nccl_check(n.group_end(), "ncclGroupEnd");
-    ++c.launches;
-}
-
-void Halo::exchange_cells(Ctx& c, Comm& comm, double* x, int stride) {
-    if (stride == 1) { exchange(c, comm, x); return; }
-    ORC_REQUIRE(stride == 4 && kMaxFields >= 4, ORC_E_INTERNAL, "halo exchange: cells hold 1 or 4 doubles");
-    if (!comm.active() || nbr.empty()) return;
-    ProfScope ps(c, PC_OTHER, 0.);
-    { double* f1[1] = {x}; if (exchange_peer(c, comm, f1, 1, 4)) return; }
-    const int ns = send_ptr.back();
-    k_halo_pack4<<<grid_for(std::max(ns, 1), 256, c.sm_count * 4), 256, 0, c.stream>>>(ns, send_idx, x, sendbuf.p);
-    c.after_launch("k_halo_pack4");
-    Nccl& n = nccl();
-    nccl_check(n.group_start(), "ncclGroupStart");
-    for (size_t q = 0; q < nbr.size(); ++q) {
-        const int cnt = send_ptr[q + 1] - send_ptr[q];
-        if (cnt > 0) nccl_check(n.send(sendbuf.p + 4 * (size_t)send_ptr[q], 4 * (size_t)cnt, kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclSend");
-        if (recv_count[q] > 0) nccl_check(n.recv(x + 4 * (size_t)recv_begin[q], 4 * (size_t)recv_count[q], kNcclFloat64, nbr[q], comm.comm, c.stream), "ncclRecv");
-    }
     nccl_check(n.group_end(), "ncclGroupEnd");
     ++c.launches;
 }

@@ -108,11 +108,10 @@ struct Halo {
     bool exchange_peer(Ctx& c, Comm& comm, double* const* fields, int nfields, int stride);
     static constexpr int kMaxFields = 4;
     void build(Ctx& c, const PartPlan& p);
-    // exchanges up to kMaxFields vectors of length n_loc in one NCCL group: owned values -> the neighbours' halo slots
-    void exchange(Ctx& c, Comm& comm, double* const* fields, int nfields);
-    void exchange(Ctx& c, Comm& comm, double* f0) { double* f[1] = {f0}; exchange(c, comm, f, 1); }
-    // one vector of `stride`-double cells (stride 1 = plain vector, 4 = a batch of three systems, linalg.cu Cell<3>)
-    void exchange_cells(Ctx& c, Comm& comm, double* x, int stride);
+    // exchanges vectors of n_loc cells of `stride` doubles (1 = plain vector, 4 = a batch of three systems, linalg.cu Cell<3>) in
+    // one NCCL group: owned values -> the neighbours' halo slots. Up to kMaxFields doubles per cell over all fields.
+    void exchange(Ctx& c, Comm& comm, double* const* fields, int nfields, int stride = 1);
+    void exchange(Ctx& c, Comm& comm, double* x, int stride = 1) { exchange(c, comm, &x, 1, stride); }
 };
 
 struct DistEnv {  // what a distributed solve needs besides the matrices
@@ -120,10 +119,5 @@ struct DistEnv {  // what a distributed solve needs besides the matrices
     Halo* halo = nullptr;
     bool on() const { return comm && halo && comm->active(); }
 };
-
-// iterative_solve over a row-partitioned matrix (rows = local cells, halo rows empty; columns local ids incl. halo).
-// BiCGSTAB runs globally (halo exchange before every SpMV, allreduce for every scalar); Multigrid = global BiCGSTAB
-// pre-smoothing + the reference's multigrid_solve applied to THIS rank's diagonal block (partition-local aggregates).
-void iterative_solve_dist(Ctx& c, DistEnv& env, DCsr& a, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K = 1);
 
 }  // namespace orc

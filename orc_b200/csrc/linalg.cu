@@ -783,11 +783,65 @@ static void bicgstab_reference_order(Ctx& c, const DCsr& A, const double* b, dou
     }
 }
 
+// =================================================================================================
+// Multi-GPU solves (SURVEY.md §8e): rows partitioned by contiguous cell ranges, halo exchange before every SpMV (C1), one
+// small allreduce per scalar (C2). Local totals are published by the fused kernels; k_dist_scalar derives alpha/omega/
+// beta/rho from the reduced values with the reference's formulas, so the loop still never synchronises with the host.
+// =================================================================================================
+enum DistOp : int { DO_RHO_INIT = 0, DO_ALPHA, DO_OMEGA, DO_BETA, DO_NORMCHK };
+// With peer windows (dist.cuh) the allreduce of the staged totals happens in this same launch: one warp exchanges the `count * K`
+// doubles with every peer's mailbox, sums them in rank order, then threads 0 .. K-1 derive the scalars.
 template <int K>
-static void bicgstab_k(Ctx& c, const DCsr& A, const double* b, double* x, uint64_t iterations) {
+__global__ void k_dist_scalar(double* scal_all, int* flags, int op, PeerAr pa, int count) {
+    if (pa.nranks > 1) peer_allreduce_warp(pa, scal_all + (K == 1 ? (int)S_TMP0 : S_STAGE), count * K, 0, flags);
+    const int k = threadIdx.x;
+    if (k >= K) return;
+    double* scal = scal_all + k * SCAL_STRIDE;
+    const double t0 = scal_all[stage_slot<K>(0, k)], t1 = scal_all[stage_slot<K>(1, k)];
+    switch (op) {
+        case DO_RHO_INIT: scal[S_RHO] = t0; break;
+        case DO_ALPHA: scal[S_ALPHA] = scal[S_RHO] / t0; break;
+        case DO_OMEGA: scal[S_OMEGA] = t0 / t1; break;
+        case DO_BETA: {
+            const double rho_prev = scal[S_RHO];
+            scal[S_RHO_PREV] = rho_prev;
+            scal[S_RHO] = t0;
+            scal[S_BETA] = t0 / rho_prev * scal[S_ALPHA] / scal[S_OMEGA];
+            break;
+        }
+        default: {
+            const double nrm = sqrt(t0);
+            scal[S_NORM] = nrm;
+            if (nrm != nrm) atomicOr(flags, DF_MG_NAN);
+        }
+    }
+}
+// `count` quantities per system were published by a fused kernel (stage_slot): ONE allreduce for all systems
+template <int K>
+static void dist_scalar(Ctx& c, const DistEnv& env, int count, int op) {
+    PeerAr pa;   // nranks == 1: the totals are already reduced (NCCL below)
+    if (env.comm->peer.on) {
+        pa = env.comm->next_allreduce();
+    } else {
+        env.comm->allreduce(c, c.d_scal + (K == 1 ? (int)S_TMP0 : S_STAGE), count * K, 0);
+    }
+    ProfScope ps(c, PC_OTHER, 0.);
+    k_dist_scalar<K><<<1, 32, 0, c.stream>>>(c.d_scal, c.d_flags, op, pa, count);
+    c.after_launch("k_dist_scalar");
+}
+
+// On a partition (env->on()): A's rows are the local cells incl. halo (halo rows are empty). The halo of every SpMV input is
+// exchanged first, the fused kernels publish local totals (SpmvArgs::dist) and dist_scalar reduces them across the ranks.
+template <int K>
+static void bicgstab_k(Ctx& c, const DCsr& A, const double* b, double* x, uint64_t iterations, const DistEnv* env) {
+    const bool dist = env && env->on();
     const int64_t n = A.nrows;
     constexpr int S = Cell<K>::S;
     DBuf<double> r(&c, n * S), p(&c, n * S), nu(&c, n * S), s(&c, n * S), tv(&c, n * S);
+    if (dist) for (DBuf<double>* v : {&r, &p, &nu, &s, &tv}) v->zero();
+    const int64_t own_lo = dist ? env->halo->own_lo : 0, own_hi = dist ? env->halo->own_hi : n;   // rho sums the owned rows
+    auto exchange = [&](double* v) { if (dist) env->halo->exchange(c, *env->comm, v, S); };
+    auto reduce = [&](int count, int op) { if (dist) dist_scalar<K>(c, *env, count, op); };
     const int vg = grid_for(n, 256, Ctx::kVirtualBlocks), xr_cap = resident_blocks<k_bicg_xr<K>>(c, 256);
     // algorithmic bytes of the call: per iteration 2 SpMVs (matrix once, x and y per system) + the three vector kernels
     // (s: 3 passes, x/r: 6, p: 4 — `h` is fused away; the reference's model has 14 passes), plus the initial residual
@@ -795,24 +849,28 @@ static void bicgstab_k(Ctx& c, const DCsr& A, const double* b, double* x, uint64
     ProfScope whole(c, PC_BICG, (double)iterations * (2. * spmv_b + 104. * K * (double)n) + spmv_b + 16. * K * (double)n,
                     (double)iterations * K * (24. * (double)A.nnz + 152. * (double)n), (int64_t)A.nnz * 8 + K + 4);
     if (c.prof.enabled) c.prof.rows_of[A.nnz] = A.nrows;
-    {
-        SpmvArgs a{};
-        a.x = x; a.y = r; a.y2 = p; a.b = b;
-        launch_spmv<EP_RESID_INIT>(c, A, a, K);
-    }
+    exchange(x);
+    { SpmvArgs a{}; a.x = x; a.y = r; a.y2 = p; a.b = b; a.dist = dist; launch_spmv<EP_RESID_INIT>(c, A, a, K); }
+    reduce(1, DO_RHO_INIT);
     for (uint64_t it = 0; it < iterations; ++it) {
-        { SpmvArgs a{}; a.x = p; a.y = nu; launch_spmv<EP_SUM_ALPHA>(c, A, a, K); }
+        exchange(p);
+        { SpmvArgs a{}; a.x = p; a.y = nu; a.dist = dist; launch_spmv<EP_SUM_ALPHA>(c, A, a, K); }
+        reduce(1, DO_ALPHA);
         {
             ProfScope ps(c, PC_VECTOR, 24. * K * (double)n);
             k_bicg_s<K><<<vg, 256, 0, c.stream>>>(n, r, nu, s, c.d_scal);
             c.after_launch("k_bicg_s");
         }
-        { SpmvArgs a{}; a.x = s; a.y = tv; launch_spmv<EP_DOTS_OMEGA>(c, A, a, K); }
+        exchange(s);
+        { SpmvArgs a{}; a.x = s; a.y = tv; a.dist = dist; launch_spmv<EP_DOTS_OMEGA>(c, A, a, K); }
+        reduce(2, DO_OMEGA);
         {
             ProfScope ps(c, PC_VECTOR, 48. * K * (double)n);
-            k_bicg_xr<K><<<virtual_grid(vg, xr_cap), 256, 0, c.stream>>>(n, x, p, s, tv, r, c.d_scal, c.d_partials, c.d_counter, vg);
+            k_bicg_xr<K><<<virtual_grid(vg, xr_cap), 256, 0, c.stream>>>(n, x, p, s, tv, r, c.d_scal, c.d_partials, c.d_counter, vg, own_lo,
+                                                                          own_hi, dist);
             c.after_launch("k_bicg_xr");
         }
+        reduce(1, DO_BETA);
         {
             ProfScope ps(c, PC_VECTOR, 32. * K * (double)n);
             k_bicg_p<K><<<vg, 256, 0, c.stream>>>(n, r, p, nu, c.d_scal);
@@ -820,18 +878,20 @@ static void bicgstab_k(Ctx& c, const DCsr& A, const double* b, double* x, uint64
         }
     }
 }
-void bicgstab(Ctx& c, const DCsr& A, const double* b, double* x, uint64_t iterations, int K) {
+void bicgstab(Ctx& c, const DCsr& A, const double* b, double* x, uint64_t iterations, int K, const DistEnv* env) {
+    const bool dist = env && env->on();
     const int64_t n = A.nrows;
     ORC_REQUIRE(A.nrows == A.ncols, ORC_E_INVALID, "bicgstab: matrix must be square");
-    if (n == 0) return;
+    if (n == 0 && !dist) return;   // a rank without cells still takes part in the collectives
     if (c.exact_order) {
+        ORC_REQUIRE(!dist, ORC_E_UNSUPPORTED, "reference-order reductions are single-GPU only");
         ORC_REQUIRE(K == 1, ORC_E_UNSUPPORTED, "reference-order reductions solve one system at a time");
         if (small_solve_ok(c, A)) bicgstab_small(c, A, b, x, iterations);   // one launch, same arithmetic (small.cu)
         else bicgstab_reference_order(c, A, b, x, iterations);
         return;
     }
-    if (K == 1) bicgstab_k<1>(c, A, b, x, iterations);
-    else bicgstab_k<3>(c, A, b, x, iterations);
+    if (K == 1) bicgstab_k<1>(c, A, b, x, iterations, env);
+    else bicgstab_k<3>(c, A, b, x, iterations, env);
 }
 
 // =================================================================================================
@@ -938,26 +998,75 @@ __global__ void k_jacobi_prepare(int lo, int hi, const int* __restrict__ rowptr,
     b0[i] = b[i] / aii;
 }
 __global__ void k_clear_latch(int* f) { atomicAnd(f, ~DF_CONVERGED); }
-static void jacobi(Ctx& c, DCsr& A, const double* b, double* x, const SolveParams& sp) {
-    const int64_t n = A.nrows;
-    if (n == 0) return;
+// On a partition the update is row-local and a partition keeps the column order of every row, so the iterates are the single-GPU
+// fast mode's bit for bit; only the residual norm that decides the break is summed per rank and then across ranks. Every rank takes
+// that decision (the latch, the magnitude check) from the same reduced bits.
+__global__ void k_jacobi_decide(double* scal, int* flags, PeerAr pa_sum, PeerAr pa_max, int iter, double threshold) {
+    if (pa_sum.nranks > 1) {   // peer path: the two allreduces in this launch (sum of r^2 and NaN rows, then max |xn|)
+        peer_allreduce_warp(pa_sum, scal + S_TMP0, 2, 0, flags);
+        peer_allreduce_warp(pa_max, scal + S_MAXABS, 1, 2, flags);
+    }
+    if (threadIdx.x != 0) return;
+    if (*(volatile int*)flags & DF_CONVERGED) return;   // latched: the residual kernel published nothing
+    jacobi_decide(scal, flags, iter, threshold, scal[S_TMP0], scal[S_MAXABS], scal[S_TMP1]);
+}
+static void jacobi(Ctx& c, DCsr& A, const double* b, double* x, const SolveParams& sp, const DistEnv* env) {
+    const bool dist = env && env->on();
+    const int64_t n = A.nrows;   // on a partition: local cells incl. halo; halo rows are empty and store no diagonal
+    if (n == 0 && !dist) return;
+    const int64_t lo = dist ? env->halo->own_lo : 0, nown = dist ? env->halo->own_hi - lo : n;   // the rows this rank solves
     csr_ensure_diag(c, A);
     CsrPtr A0 = csr_like(c, A);
-    DBuf<double> b0(&c, n), xn(&c, n);
-    k_jacobi_prepare<<<(int)((n + 255) / 256), 256, 0, c.stream>>>(0, (int)n, A.rowptr, A.col, A.diag, A.val, b, A0->val, b0, c.d_flags);
-    c.after_launch("k_jacobi_prepare");
+    DBuf<double> b0(&c, (size_t)std::max<int64_t>(n, 1)), xn(&c, (size_t)std::max<int64_t>(n, 1));
+    if (dist) xn.zero();
+    if (nown > 0) {
+        k_jacobi_prepare<<<(int)((nown + 255) / 256), 256, 0, c.stream>>>((int)lo, (int)(lo + nown), A.rowptr, A.col, A.diag, A.val, b, A0->val, b0,
+                                                                          c.d_flags);
+        c.after_launch("k_jacobi_prepare");
+    }
+    // the owned rows as a matrix of their own: row i of the view is row lo + i (SpmvArgs::row0), columns stay local ids
+    auto owned_rows = [&](const DCsr& M) {
+        DCsr v;   // no context: the view frees nothing
+        v.nrows = nown; v.ncols = M.ncols; v.nnz = M.nnz; v.rowptr = M.rowptr + lo; v.col = M.col; v.val = M.val;
+        return v;
+    };
+    const DCsr A0v = owned_rows(*A0), Av = owned_rows(A);
     for (uint64_t it = 0; it < sp.iterations; ++it) {
-        SpmvArgs a{};
-        a.x = x; a.y = xn; a.b = b0; a.w = sp.relaxation; a.one_minus_w = 1. - sp.relaxation;
-        launch_spmv<EP_JACOBI>(c, *A0, a);
-        SpmvArgs r{};
-        r.x = xn; r.y2 = x; r.b = b; r.iter = (int)it; r.threshold = sp.threshold; r.defer = c.exact_order ? 1 : 0;
-        launch_spmv<EP_JACOBI_RES>(c, A, r);
-        if (c.exact_order) {  // r = (b' - A' x).norm() in nalgebra's accumulation order decides the break (:202-212)
+        if (dist) env->halo->exchange(c, *env->comm, x);
+        if (nown > 0) {
+            SpmvArgs a{};
+            a.x = x; a.y = xn; a.b = b0; a.w = sp.relaxation; a.one_minus_w = 1. - sp.relaxation; a.row0 = (int)lo;
+            launch_spmv<EP_JACOBI>(c, A0v, a);
+        }
+        if (dist) env->halo->exchange(c, *env->comm, xn);
+        if (nown > 0) {
+            SpmvArgs r{};
+            r.x = xn; r.y2 = x; r.b = b; r.iter = (int)it; r.threshold = sp.threshold; r.defer = c.exact_order ? 1 : 0; r.dist = dist;
+            r.row0 = (int)lo;
+            launch_spmv<EP_JACOBI_RES>(c, Av, r);
+        } else {
+            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_TMP0, 0, 2 * sizeof(double), c.stream));   // a rank without cells adds nothing
+            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_MAXABS, 0, sizeof(double), c.stream));
+        }
+        if (c.exact_order) {  // r = (b' - A' x).norm() in nalgebra's accumulation order decides the break (:202-212); one GPU only
             SpmvArgs q{};
             q.x = x; q.y = xn; q.b = b;
             launch_spmv<EP_RESID>(c, A, q);
             dot_ref(c, n, xn, xn, DOT_JACOBI_DECIDE, (int)it, sp.threshold);
+        }
+        if (dist) {   // the residual kernel published the local totals: reduce them and decide on every rank
+            Comm& cm = *env->comm;
+            PeerAr ps, pm;   // nranks == 1: NCCL has reduced the totals already
+            if (cm.peer.on) {
+                ps = cm.next_allreduce();
+                pm = cm.next_allreduce();
+            } else {
+                cm.allreduce(c, c.d_scal + S_TMP0, 2, 0);
+                cm.allreduce(c, c.d_scal + S_MAXABS, 1, 2);
+            }
+            ProfScope pscope(c, PC_OTHER, 0.);
+            k_jacobi_decide<<<1, 32, 0, c.stream>>>(c.d_scal, c.d_flags, ps, pm, (int)it, sp.threshold);
+            c.after_launch("k_jacobi_decide");
         }
     }
     // clear the convergence latch (stream ordered) so that later solves start fresh
@@ -2265,194 +2374,6 @@ bool solve_batchable(const SolveParams& sp) {
     return sp.method == ORC_SOLVER_MULTIGRID && sp.mg_smoother == ORC_SOLVER_BICGSTAB;
 }
 
-void iterative_solve(Ctx& c, DCsr& A, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K) {
-    ORC_REQUIRE(A.nrows == A.ncols, ORC_E_INVALID, "iterative_solve: matrix must be square");
-    ORC_REQUIRE(K == 1 || (K == 3 && solve_batchable(sp)), ORC_E_UNSUPPORTED, "this solver cannot run three systems in lockstep");
-    const int64_t n = A.nrows;
-    const int S = vstride(K);
-    c.exact_order = sp.exact_order;
-    CsrPtr a_tmp;
-    DBuf<double> b_tmp;
-    DCsr* Ap = &A;
-    const double* bp = b;
-    if (sp.preconditioner == ORC_PC_JACOBI) {  // :157-168
-        b_tmp.alloc(&c, std::max<int64_t>(n, 1) * S);
-        ProfScope ps(c, PC_SCALE, 0.);
-        a_tmp = jacobi_scale(c, A, b, b_tmp, K);
-        Ap = a_tmp.get();
-        bp = b_tmp;
-    }
-    switch (sp.method) {
-        case ORC_SOLVER_JACOBI: jacobi(c, *Ap, bp, x, sp); break;
-        case ORC_SOLVER_GAUSS_SEIDEL: gauss_seidel(c, *Ap, bp, x, sp); break;
-        case ORC_SOLVER_BICGSTAB: bicgstab(c, *Ap, bp, x, sp.iterations, K); break;
-        case ORC_SOLVER_MULTIGRID: {  // :270-296
-            if (trace) { trace->rows.clear(); trace->nnz.clear(); trace->rows.push_back(n); trace->nnz.push_back(Ap->nnz); }
-            SolveParams pre = sp;
-            pre.method = sp.mg_smoother;
-            iterative_solve(c, *Ap, bp, x, pre, nullptr, K);   // preconditions AGAIN (Q7)
-            DBuf<double> r(&c, std::max<int64_t>(n, 1) * S), corr(&c, std::max<int64_t>(n, 1) * S);
-            residual(c, *Ap, bp, x, r, K);
-            multigrid_solve(c, *Ap, r, corr, 1, sp, trace, K);
-            dev_axpy_inplace(c, x, corr, n * S);
-            break;
-        }
-        default: throw Error(ORC_E_UNSUPPORTED, "unsupported solution method");
-    }
-}
-
-// =================================================================================================
-// Multi-GPU solves (SURVEY.md §8e): rows partitioned by contiguous cell ranges, halo exchange before every SpMV (C1), one
-// small allreduce per scalar (C2). Local totals are published by the fused kernels; k_dist_scalar derives alpha/omega/
-// beta/rho from the reduced values with the reference's formulas, so the loop still never synchronises with the host.
-// =================================================================================================
-enum DistOp : int { DO_RHO_INIT = 0, DO_ALPHA, DO_OMEGA, DO_BETA, DO_NORMCHK };
-// With peer windows (dist.cuh) the allreduce of the staged totals happens in this same launch: one warp exchanges the `count * K`
-// doubles with every peer's mailbox, sums them in rank order, then threads 0 .. K-1 derive the scalars.
-template <int K>
-__global__ void k_dist_scalar(double* scal_all, int* flags, int op, PeerAr pa, int count) {
-    if (pa.nranks > 1) peer_allreduce_warp(pa, scal_all + (K == 1 ? (int)S_TMP0 : S_STAGE), count * K, 0, flags);
-    const int k = threadIdx.x;
-    if (k >= K) return;
-    double* scal = scal_all + k * SCAL_STRIDE;
-    const double t0 = scal_all[stage_slot<K>(0, k)], t1 = scal_all[stage_slot<K>(1, k)];
-    switch (op) {
-        case DO_RHO_INIT: scal[S_RHO] = t0; break;
-        case DO_ALPHA: scal[S_ALPHA] = scal[S_RHO] / t0; break;
-        case DO_OMEGA: scal[S_OMEGA] = t0 / t1; break;
-        case DO_BETA: {
-            const double rho_prev = scal[S_RHO];
-            scal[S_RHO_PREV] = rho_prev;
-            scal[S_RHO] = t0;
-            scal[S_BETA] = t0 / rho_prev * scal[S_ALPHA] / scal[S_OMEGA];
-            break;
-        }
-        default: {
-            const double nrm = sqrt(t0);
-            scal[S_NORM] = nrm;
-            if (nrm != nrm) atomicOr(flags, DF_MG_NAN);
-        }
-    }
-}
-// `count` quantities per system were published by a fused kernel (stage_slot): ONE allreduce for all systems
-template <int K>
-static void dist_scalar(Ctx& c, DistEnv& env, int count, int op) {
-    PeerAr pa;   // nranks == 1: the totals are already reduced (NCCL below)
-    if (env.comm->peer.on) {
-        pa = env.comm->next_allreduce();
-    } else {
-        env.comm->allreduce(c, c.d_scal + (K == 1 ? (int)S_TMP0 : S_STAGE), count * K, 0);
-    }
-    ProfScope ps(c, PC_OTHER, 0.);
-    k_dist_scalar<K><<<1, 32, 0, c.stream>>>(c.d_scal, c.d_flags, op, pa, count);
-    c.after_launch("k_dist_scalar");
-}
-template <int K>
-static void bicgstab_dist(Ctx& c, DistEnv& env, const DCsr& A, const double* b, double* x, uint64_t iterations) {
-    const int64_t n = A.nrows;  // local cells incl. halo; halo rows are empty
-    constexpr int S = Cell<K>::S;
-    Halo& H = *env.halo;
-    DBuf<double> r(&c, n * S), p(&c, n * S), nu(&c, n * S), s(&c, n * S), tv(&c, n * S);
-    for (DBuf<double>* v : {&r, &p, &nu, &s, &tv}) v->zero();
-    const int vg = grid_for(n, 256, Ctx::kVirtualBlocks), xr_cap = resident_blocks<k_bicg_xr<K>>(c, 256);
-    const double spmv_b = 12. * (double)A.nnz + 4. * (double)n + 16. * K * (double)n;
-    ProfScope whole(c, PC_BICG, (double)iterations * (2. * spmv_b + 104. * K * (double)n) + spmv_b + 16. * K * (double)n,
-                    (double)iterations * K * (24. * (double)A.nnz + 152. * (double)n), (int64_t)A.nnz * 8 + K + 4);
-    if (c.prof.enabled) c.prof.rows_of[A.nnz] = A.nrows;
-    H.exchange_cells(c, *env.comm, x, S);
-    { SpmvArgs a{}; a.x = x; a.y = r; a.y2 = p; a.b = b; a.dist = 1; launch_spmv<EP_RESID_INIT>(c, A, a, K); }
-    dist_scalar<K>(c, env, 1, DO_RHO_INIT);
-    for (uint64_t it = 0; it < iterations; ++it) {
-        H.exchange_cells(c, *env.comm, p, S);
-        { SpmvArgs a{}; a.x = p; a.y = nu; a.dist = 1; launch_spmv<EP_SUM_ALPHA>(c, A, a, K); }
-        dist_scalar<K>(c, env, 1, DO_ALPHA);
-        {
-            ProfScope ps(c, PC_VECTOR, 24. * K * (double)n);
-            k_bicg_s<K><<<vg, 256, 0, c.stream>>>(n, r, nu, s, c.d_scal);
-            c.after_launch("k_bicg_s");
-        }
-        H.exchange_cells(c, *env.comm, s, S);
-        { SpmvArgs a{}; a.x = s; a.y = tv; a.dist = 1; launch_spmv<EP_DOTS_OMEGA>(c, A, a, K); }
-        dist_scalar<K>(c, env, 2, DO_OMEGA);
-        {
-            ProfScope ps(c, PC_VECTOR, 48. * K * (double)n);
-            k_bicg_xr<K><<<virtual_grid(vg, xr_cap), 256, 0, c.stream>>>(n, x, p, s, tv, r, c.d_scal, c.d_partials, c.d_counter, vg, H.own_lo, H.own_hi, 1);
-            c.after_launch("k_bicg_xr");
-        }
-        dist_scalar<K>(c, env, 1, DO_BETA);
-        {
-            ProfScope ps(c, PC_VECTOR, 32. * K * (double)n);
-            k_bicg_p<K><<<vg, 256, 0, c.stream>>>(n, r, p, nu, c.d_scal);
-            c.after_launch("k_bicg_p");
-        }
-    }
-}
-
-// Jacobi over a row-partitioned matrix (linear_algebra.rs:172-218). The update is row-local and a partition keeps the column order
-// of every row, so the iterates are the single-GPU fast mode's bit for bit; only the residual norm that decides the break is summed
-// per rank and then across ranks. Every rank takes that decision (the latch, the magnitude check) from the same reduced bits.
-__global__ void k_jacobi_decide(double* scal, int* flags, PeerAr pa_sum, PeerAr pa_max, int iter, double threshold) {
-    if (pa_sum.nranks > 1) {   // peer path: the two allreduces in this launch (sum of r^2 and NaN rows, then max |xn|)
-        peer_allreduce_warp(pa_sum, scal + S_TMP0, 2, 0, flags);
-        peer_allreduce_warp(pa_max, scal + S_MAXABS, 1, 2, flags);
-    }
-    if (threadIdx.x != 0) return;
-    if (*(volatile int*)flags & DF_CONVERGED) return;   // latched: the residual kernel published nothing
-    jacobi_decide(scal, flags, iter, threshold, scal[S_TMP0], scal[S_MAXABS], scal[S_TMP1]);
-}
-static void jacobi_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double* x, const SolveParams& sp) {
-    const int64_t n = A.nrows;   // local cells incl. halo; halo rows are empty and store no diagonal
-    Halo& H = *env.halo;
-    Comm& cm = *env.comm;
-    const int64_t lo = H.own_lo, nown = H.own_hi - H.own_lo;
-    csr_ensure_diag(c, A);
-    CsrPtr A0 = csr_like(c, A);
-    DBuf<double> b0(&c, (size_t)std::max<int64_t>(n, 1)), xn(&c, (size_t)std::max<int64_t>(n, 1));
-    xn.zero();
-    if (nown > 0) {
-        k_jacobi_prepare<<<(int)((nown + 255) / 256), 256, 0, c.stream>>>((int)lo, (int)(lo + nown), A.rowptr, A.col, A.diag, A.val, b, A0->val, b0,
-                                                                          c.d_flags);
-        c.after_launch("k_jacobi_prepare");
-    }
-    // the owned rows as a matrix of their own: row i of the view is row lo + i (SpmvArgs::row0), columns stay local ids
-    auto owned_rows = [&](const DCsr& M) {
-        DCsr v;   // no context: the view frees nothing
-        v.nrows = nown; v.ncols = M.ncols; v.nnz = M.nnz; v.rowptr = M.rowptr + lo; v.col = M.col; v.val = M.val;
-        return v;
-    };
-    const DCsr A0v = owned_rows(*A0), Av = owned_rows(A);
-    for (uint64_t it = 0; it < sp.iterations; ++it) {
-        H.exchange(c, cm, x);
-        if (nown > 0) {
-            SpmvArgs a{};
-            a.x = x; a.y = xn; a.b = b0; a.w = sp.relaxation; a.one_minus_w = 1. - sp.relaxation; a.row0 = (int)lo;
-            launch_spmv<EP_JACOBI>(c, A0v, a);
-        }
-        H.exchange(c, cm, xn);
-        if (nown > 0) {
-            SpmvArgs r{};
-            r.x = xn; r.y2 = x; r.b = b; r.dist = 1; r.row0 = (int)lo;
-            launch_spmv<EP_JACOBI_RES>(c, Av, r);
-        } else {
-            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_TMP0, 0, 2 * sizeof(double), c.stream));   // a rank without cells adds nothing
-            ORC_CUDA(cudaMemsetAsync(c.d_scal + S_MAXABS, 0, sizeof(double), c.stream));
-        }
-        PeerAr ps, pm;   // nranks == 1: NCCL has reduced the totals already
-        if (cm.peer.on) {
-            ps = cm.next_allreduce();
-            pm = cm.next_allreduce();
-        } else {
-            cm.allreduce(c, c.d_scal + S_TMP0, 2, 0);
-            cm.allreduce(c, c.d_scal + S_MAXABS, 1, 2);
-        }
-        ProfScope pscope(c, PC_OTHER, 0.);
-        k_jacobi_decide<<<1, 32, 0, c.stream>>>(c.d_scal, c.d_flags, ps, pm, (int)it, sp.threshold);
-        c.after_launch("k_jacobi_decide");
-    }
-    k_clear_latch<<<1, 1, 0, c.stream>>>(c.d_flags);
-    c.after_launch("k_clear_latch");
-}
-
 // rows/columns [lo, hi) of A as a standalone CSR with indices shifted to 0 (the rank's diagonal block)
 __global__ void k_block_counts(int lo, int hi, const int* __restrict__ rowptr, const int* __restrict__ col, int* cnt) {
     int i = lo + blockIdx.x * blockDim.x + threadIdx.x;
@@ -2497,20 +2418,19 @@ static CsrPtr extract_block(Ctx& c, const DCsr& A, int64_t lo, int64_t hi) {
     return B;
 }
 
-void iterative_solve_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K) {
-    if (!env.on()) { iterative_solve(c, A, b, x, sp, trace, K); return; }
+void iterative_solve(Ctx& c, DCsr& A, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K, const DistEnv* env) {
+    const bool dist = env && env->on();
     ORC_REQUIRE(A.nrows == A.ncols, ORC_E_INVALID, "iterative_solve: matrix must be square");
-    ORC_REQUIRE(!sp.exact_order, ORC_E_UNSUPPORTED, "reference-order reductions are single-GPU only");
+    ORC_REQUIRE(!(dist && sp.exact_order), ORC_E_UNSUPPORTED, "reference-order reductions are single-GPU only");
     ORC_REQUIRE(K == 1 || (K == 3 && solve_batchable(sp)), ORC_E_UNSUPPORTED, "this solver cannot run three systems in lockstep");
     const int64_t n = A.nrows;
     const int S = vstride(K);
-    Halo& H = *env.halo;
-    c.exact_order = false;
+    c.exact_order = sp.exact_order;
     CsrPtr a_tmp;
     DBuf<double> b_tmp;
     DCsr* Ap = &A;
     const double* bp = b;
-    if (sp.preconditioner == ORC_PC_JACOBI) {  // row-local: no communication
+    if (sp.preconditioner == ORC_PC_JACOBI) {  // :157-168; row-local, so a partition needs no communication
         b_tmp.alloc(&c, std::max<int64_t>(n, 1) * S);
         ProfScope ps(c, PC_SCALE, 0.);
         a_tmp = jacobi_scale(c, A, b, b_tmp, K);
@@ -2518,30 +2438,34 @@ void iterative_solve_dist(Ctx& c, DistEnv& env, DCsr& A, const double* b, double
         bp = b_tmp;
     }
     switch (sp.method) {
-        case ORC_SOLVER_JACOBI: jacobi_dist(c, env, *Ap, bp, x, sp); break;
-        case ORC_SOLVER_BICGSTAB:
-            if (K == 1) bicgstab_dist<1>(c, env, *Ap, bp, x, sp.iterations);
-            else bicgstab_dist<3>(c, env, *Ap, bp, x, sp.iterations);
+        case ORC_SOLVER_JACOBI: jacobi(c, *Ap, bp, x, sp, env); break;
+        case ORC_SOLVER_GAUSS_SEIDEL:   // the sweep is one dependency chain over all rows: it has no partitioned form
+            ORC_REQUIRE(!dist, ORC_E_UNSUPPORTED, "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid");
+            gauss_seidel(c, *Ap, bp, x, sp);
             break;
-        case ORC_SOLVER_MULTIGRID: {
-            if (trace) { trace->rows.clear(); trace->nnz.clear(); trace->rows.push_back(H.own_hi - H.own_lo); trace->nnz.push_back(Ap->nnz); }
+        case ORC_SOLVER_BICGSTAB: bicgstab(c, *Ap, bp, x, sp.iterations, K, env); break;
+        case ORC_SOLVER_MULTIGRID: {  // :270-296
+            // on a partition the coarse correction is the reference's multigrid_solve on this rank's diagonal block (rows [lo, lo + nown)):
+            // aggregates never cross the partition (C4)
+            const int64_t lo = dist ? env->halo->own_lo : 0, nown = dist ? env->halo->own_hi - lo : n;
+            if (trace) { trace->rows.clear(); trace->nnz.clear(); trace->rows.push_back(nown); trace->nnz.push_back(Ap->nnz); }
             SolveParams pre = sp;
             pre.method = sp.mg_smoother;
-            ORC_REQUIRE(pre.method == ORC_SOLVER_BICGSTAB, ORC_E_UNSUPPORTED, "multi-GPU multigrid needs the BiCGSTAB smoother");
-            iterative_solve_dist(c, env, *Ap, bp, x, pre, nullptr, K);  // preconditions again (Q7), globally
-            DBuf<double> r(&c, std::max<int64_t>(n, 1) * S);
-            r.zero();
-            H.exchange_cells(c, *env.comm, x, S);
+            ORC_REQUIRE(!dist || pre.method == ORC_SOLVER_BICGSTAB, ORC_E_UNSUPPORTED, "multi-GPU multigrid needs the BiCGSTAB smoother");
+            iterative_solve(c, *Ap, bp, x, pre, nullptr, K, env);   // preconditions AGAIN (Q7), globally on a partition
+            DBuf<double> r(&c, std::max<int64_t>(n, 1) * S), corr(&c, std::max<int64_t>(nown, 1) * S);
+            CsrPtr Aloc;
+            if (dist) {
+                r.zero();
+                env->halo->exchange(c, *env->comm, x, S);
+            }
             residual(c, *Ap, bp, x, r, K);
-            // the reference's multigrid_solve on this rank's diagonal block: aggregates never cross the partition (C4)
-            const int64_t nown = H.own_hi - H.own_lo;
-            CsrPtr Aloc = extract_block(c, *Ap, H.own_lo, H.own_hi);
-            DBuf<double> corr(&c, std::max<int64_t>(nown, 1) * S);
-            multigrid_solve(c, *Aloc, r.p + H.own_lo * S, corr, 1, sp, trace, K);
-            dev_axpy_inplace(c, x + H.own_lo * S, corr, nown * S);
+            if (dist) Aloc = extract_block(c, *Ap, lo, lo + nown);
+            multigrid_solve(c, dist ? *Aloc : *Ap, r.p + lo * S, corr, 1, sp, trace, K);
+            dev_axpy_inplace(c, x + lo * S, corr, nown * S);
             break;
         }
-        default: throw Error(ORC_E_UNSUPPORTED, "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid");
+        default: throw Error(ORC_E_UNSUPPORTED, dist ? "multi-GPU solves support Jacobi, BiCGSTAB and Multigrid" : "unsupported solution method");
     }
 }
 

@@ -7,6 +7,7 @@
 namespace orc {
 
 using CsrPtr = std::unique_ptr<DCsr>;
+struct DistEnv;   // dist.cuh: the communicator and halo plan of a partition
 
 // ---- CSR plumbing ----
 CsrPtr csr_alloc(Ctx& c, int64_t nrows, int64_t ncols, int64_t nnz);            // owns pattern + values
@@ -42,7 +43,11 @@ struct MgTrace {  // keeps R_l, A_l of a Multigrid solve (parity tests) and the 
 // iterative_solve (linear_algebra.rs:144-299). b, x are device vectors. Errors surface through the device
 // flag word (checked by the caller with check_solver_flags) so that the solve never syncs with the host
 // except where sizes are data dependent (AMG setup).
-void iterative_solve(Ctx& c, DCsr& a, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K = 1);
+// On a partition (env->on()) the matrix is row-partitioned (rows = local cells, halo rows empty; columns local ids incl. halo).
+// BiCGSTAB and Jacobi run globally (halo exchange before every SpMV, allreduce for every scalar); Multigrid = global BiCGSTAB
+// pre-smoothing + the reference's multigrid_solve applied to THIS rank's diagonal block (partition-local aggregates).
+void iterative_solve(Ctx& c, DCsr& a, const double* b, double* x, const SolveParams& sp, MgTrace* trace, int K = 1,
+                     const DistEnv* env = nullptr);
 bool solve_batchable(const SolveParams& sp);   // can three systems that share the matrix run in lockstep (K = 3)?
 void pack3(Ctx& c, int64_t n, const double* a, const double* b, const double* c3, double* out);   // -> cells
 void unpack3(Ctx& c, int64_t n, const double* in, double* a, double* b, double* c3);
@@ -52,7 +57,7 @@ bool csr_values_identical(Ctx& c, const DCsr& a, const DCsr& b);
 void csr_blend(Ctx& c, const DCsr& a, double sa, const DCsr& b, double sb, DCsr& out);
 void check_solver_flags(Ctx& c);  // throws the mapped ORC_E_* if a device flag is set, and clears the word
 void throw_for_flags(int flags);  // the mapping itself (a status word received from a peer rank)
-void bicgstab(Ctx& c, const DCsr& a, const double* b, double* x, uint64_t iterations, int K = 1);
+void bicgstab(Ctx& c, const DCsr& a, const double* b, double* x, uint64_t iterations, int K = 1, const DistEnv* env = nullptr);
 
 // single-launch solvers for small systems (small.cu): the whole BiCGSTAB loop / all Gauss-Seidel sweeps in one block
 bool small_enabled();                                                            // ORC_B200_SMALL=0 switches the one-block kernels off
