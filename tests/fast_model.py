@@ -11,6 +11,8 @@ shuffle tree. Vectors of K systems are arrays of shape (K, n); system k is the K
 
 An intentional change of a kernel's summation order must update this model in the same change (DESIGN.md §5).
 """
+import os
+
 import numpy as np
 
 # ---- constants of the kernels (tests/test_fast_model.py reads them back from the sources) ----------------------------------
@@ -187,19 +189,21 @@ class Mat:
         return self._diag
 
     def plan(self):
-        """Entry slots in ascending position: slot s holds entry rowptr[i] + s of every row i longer than s."""
+        """(order, slots): `order` lists the rows by descending length (stable), and slot s holds entry rowptr[i] + s of every row
+        longer than s, i.e. of the first k_s rows of `order`: (k_s, values, columns) in that order. Working in `order` turns every
+        slot's rows into a prefix (contiguous slices instead of a scatter); each row still adds its entries in ascending position."""
         if self._plan is None:
             lens = self.lengths
             order = np.argsort(-lens, kind="stable").astype(np.int64)
             counts = np.bincount(lens, minlength=1) if self.nrows else np.zeros(1, np.int64)
             longer = self.nrows - np.cumsum(counts)   # rows with more than s entries, s = 0, 1, ...
+            start = self.rowptr[:-1][order]
             slots = []
             for s in range(self.max_row):
                 k = int(longer[s])
-                rows = None if k == self.nrows else order[:k].copy()
-                idx = (self.rowptr[:-1] if rows is None else self.rowptr[rows]) + s
-                slots.append((rows, self.val[idx], self.col[idx]))
-            self._plan = slots
+                idx = start[:k] + s
+                slots.append((k, self.val[idx], self.col[idx]))
+            self._plan = (order, slots)
         return self._plan
 
 
@@ -224,25 +228,55 @@ def spmv(A, X, exact_order=False):
     G = 1 (k_spmv, linalg.cu:437-448): acc = 0; acc += a_ik x_k in ascending k.
     G = 4 / 8 (k_spmv_vec, :485-511): lane gl adds entries lo+gl, lo+gl+G, ... in ascending order (UN only batches the loads),
     then the width-G shuffle tree."""
-    XT = np.ascontiguousarray(np.atleast_2d(X).T)           # (ncols, K): one gather fetches the K values of a column
-    K = XT.shape[1]
+    X = np.atleast_2d(np.asarray(X, dtype=np.float64))
+    K = X.shape[0]
     G = lanes_per_row(A, exact_order)
-    if G == 1:
-        acc = np.zeros((A.nrows, K))
-        for rows, v, c in A.plan():
-            if rows is None:
-                acc = acc + v[:, None] * XT[c]
-            else:
-                acc[rows] = acc[rows] + v[:, None] * XT[c]
-        return np.ascontiguousarray(acc.T)
-    lanes = np.zeros((G, A.nrows, K))
-    for s, (rows, v, c) in enumerate(A.plan()):
-        gl = s % G
-        if rows is None:
-            lanes[gl] = lanes[gl] + v[:, None] * XT[c]
-        else:
-            lanes[gl, rows] = lanes[gl, rows] + v[:, None] * XT[c]
-    return np.ascontiguousarray(segment_tree(np.moveaxis(lanes, 0, -1), G).T)
+    order, slots = A.plan()
+    # K = 1: plain vectors; K > 1: (ncols, K), one gather fetches the K values of a column
+    XT = X[0] if K == 1 else np.ascontiguousarray(X.T)
+    shape = (A.nrows,) if K == 1 else (A.nrows, K)
+    lanes = np.zeros((G,) + shape)                          # rows in `order`
+
+    def rows(lo, hi):   # every slot over the rows [lo, hi) of `order`: no row is shared, so the chunks are independent
+        tmp = np.empty((hi - lo,) + shape[1:])
+        for s, (k, v, c) in enumerate(slots):
+            e = min(hi, k)
+            if e <= lo:
+                break
+            prod = tmp[:e - lo]
+            np.take(XT, c[lo:e], axis=0, out=prod, mode="clip")   # the columns are in range: "clip" only skips a buffer
+            np.multiply(v[lo:e] if K == 1 else v[lo:e, None], prod, out=prod)
+            acc = lanes[s % G, lo:e]
+            np.add(acc, prod, out=acc)
+
+    chunks = _row_chunks(A.nrows, len(A.col))
+    if len(chunks) == 1:
+        rows(*chunks[0])
+    else:   # NumPy releases the GIL inside take / multiply / add
+        list(_pool().map(lambda c: rows(*c), chunks))
+    out = np.empty(shape)
+    out[order] = lanes[0] if G == 1 else segment_tree(np.moveaxis(lanes, 0, -1), G)
+    return out[None] if K == 1 else np.ascontiguousarray(out.T)
+
+
+_POOL = {}
+
+
+def _pool():
+    """The SpMV threads of this process (a forked worker starts its own)."""
+    pid = os.getpid()
+    if pid not in _POOL:
+        from concurrent.futures import ThreadPoolExecutor
+        _POOL.clear()
+        _POOL[pid] = ThreadPoolExecutor(max_workers=os.cpu_count() or 1)
+    return _POOL[pid]
+
+
+def _row_chunks(n, entries):
+    """Row ranges of `order` for the threads of one SpMV: one range for small matrices, else one per core."""
+    parts = 1 if entries < 1 << 20 else (os.cpu_count() or 1)
+    edges = np.linspace(0, n, parts + 1).astype(np.int64)
+    return [(int(a), int(b)) for a, b in zip(edges[:-1], edges[1:]) if b > a] or [(0, 0)]
 
 
 def fused_sum(A, c):
@@ -417,6 +451,27 @@ def reordered_system(A, perm):
 # iterative_solve and Multigrid (linalg.cu:2200-2289)
 # =============================================================================================================================
 BICGSTAB, JACOBI, MULTIGRID = "bicgstab", "jacobi", "multigrid"
+MG_DIVERGED, DIVERGED = "Multigrid diverged", "solution diverged"   # ORC_E_MG_DIVERGED, ORC_E_DIVERGED
+
+
+class ModelDiverged(RuntimeError):
+    """A divergence exit of the GPU path, taken by the model. str() is the GPU's message; `code` names its status
+    (orc_b200._lib.E_MG_DIVERGED or E_DIVERGED)."""
+
+    @property
+    def code(self):
+        from orc_b200 import _lib
+        return _lib.E_MG_DIVERGED if str(self) == MG_DIVERGED else _lib.E_DIVERGED
+
+
+def check_field_sums(*fields):
+    """The `u_avg != u_avg` exit of steady_iterate (capi.cu, solver.rs:217-221). A sum is NaN in every order exactly when a term is
+    NaN or the terms hold both infinities (finite terms that overflow are the one order-dependent case; the kernels' fields never
+    come near DBL_MAX before they turn NaN)."""
+    for f in fields:
+        f = np.asarray(f)
+        if np.isnan(f).any() or (np.isposinf(f).any() and np.isneginf(f).any()):
+            raise ModelDiverged(DIVERGED)
 
 
 def transpose(R):
@@ -481,6 +536,10 @@ def _multigrid_level(A, r, level, levels, iterations, threshold, kw, pos, min_le
         return out
 
     ep = smooth(ep, threshold)
+    # residual_norm_check (EP_RESID_NORM on the unscaled level matrix, :97-105): sqrt(sum r_i^2) is NaN exactly when some r_i is
+    # NaN (squares are >= 0 or +inf), whatever the order of the sum; r_i itself comes from the kernel's row order
+    if np.isnan(rp - spmv(Ac, ep)).any():
+        raise ModelDiverged(MG_DIVERGED)
     if level < mg_levels and Ac.nrows > 16:
         corr = _multigrid_level(Ac, rp, level + 1, levels, iterations, threshold, kw, pos, min_level, smoother, mg_levels)
         ep = ep + corr

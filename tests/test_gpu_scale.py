@@ -161,18 +161,18 @@ def test_one_simple_iteration_at_size(oracle):
       (measured on B200: 4e-8 ... 1.2e-7; 13 nested, doubly preconditioned BiCGSTAB calls per Multigrid solve multiply the 1e-12
       per-call differences of the test above). Every kernel of the bench path runs (lockstep K = 3 momentum solves, four AMG
       levels, fused reductions over many virtual blocks).
-    * Fast reductions at the reference's 50 inner iterations: NOT comparable at this size, printed only. The reference's BiCGSTAB
-      has no convergence test (src/linear_algebra.rs:247-269): it keeps iterating on a converged system, dividing rounding noise by
-      rounding noise, so ANY change of summation order moves the result in the leading digits (measured here: 1e-2 of the
-      velocity norm after one iteration; DESIGN.md §5). That is the conditioning of the reference algorithm, not a kernel error:
-      the same kernels agree to 1e-12 per level while the iteration is still converging (test above)."""
+    * Fast reductions at the reference's 50 inner iterations: no tolerance against the oracle means anything here (the reference's
+      unguarded BiCGSTAB turns any change of summation order into differences in the leading digits, DESIGN.md §5). The
+      benchmark's version of this case (its pressure relaxation of 1e-4 instead of the default 0.01) is pinned bit for bit against
+      the composed fast-mode model instead:
+      test_gpu_fast_simple.test_hex48_bench_settings_from_rest_and_reset."""
     from orc_b200 import settings as S
     pm, om = make_pair(oracle, syn.hex_box(48, 48, 48))
     for m in (pm, om):
         syn.channel_bcs(m)
     n = pm.n_cells
     z = np.zeros(n)
-    for mode, inner in ((S.ReductionMode.ReferenceOrder, 50), (S.ReductionMode.Fast, 5), (S.ReductionMode.Fast, 50)):
+    for mode, inner in ((S.ReductionMode.ReferenceOrder, 50), (S.ReductionMode.Fast, 5)):
         uo, vo, wo, po_, orep, _ = om.solve_steady(z, z, z, z, oracle.Settings(iterations=inner), RHO, MU, 1, 1)
         vel = np.sqrt(sum(np.linalg.norm(b) ** 2 for b in (uo, vo, wo)))
         ps = orc_b200.NumericalSettings(reduction_mode=mode)
@@ -186,8 +186,7 @@ def test_one_simple_iteration_at_size(oracle):
         errs = [np.linalg.norm(a - b) / vel for a, b in zip((u, v, w), (uo, vo, wo))] + [rel_l2(p, po_)]
         print(f"fast reductions vs oracle after one iteration at 48^3, {inner} inner iterations (u, v, w / |vel|, p):", [f"{e:.2e}" for e in errs])
         assert all(np.isfinite(a).all() for a in (u, v, w, p))
-        if inner == 5:
-            assert max(errs) <= 1e-6, errs
+        assert max(errs) <= 1e-6, errs
 
 
 def test_bench_mesh_amg_setup_matches_oracle(oracle, ctx):
