@@ -61,7 +61,8 @@ enum { ORC_BC_INTERIOR = 2, ORC_BC_WALL = 3, ORC_BC_PRESSURE_INLET = 4, ORC_BC_P
 /* Gauss-Seidel behaviour. The reference arm always panics (src/linear_algebra.rs:219-246). */
 enum { ORC_GS_REFERENCE_PANIC = 0, /* run nothing, return ORC_E_GS_MAINTENANCE                                   */
        ORC_GS_LEXICOGRAPHIC = 1,   /* intended forward SOR sweep in row order, exact (dataflow kernel)           */
-       ORC_GS_MULTICOLOUR = 2 };   /* greedy multicolour ordering: documented ordering difference (DESIGN.md)    */
+       ORC_GS_MULTICOLOUR = 2 };   /* greedy colouring in row order, colours swept in ascending order (DESIGN.md);
+                                      structurally symmetric patterns only (else ORC_E_UNSUPPORTED)          */
 /* Momentum assembly recurrence (SURVEY.md Q2, src/discretization.rs:182-197 + :340-351). */
 enum { ORC_ASSEMBLY_EXACT = 0,  /* cell i sees NEW diagonals of neighbours j<i, OLD of j>i, like the reference     */
        ORC_ASSEMBLY_FROZEN = 1 }; /* every face sees previous-iteration diagonals (documented deviation)            */

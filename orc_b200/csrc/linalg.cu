@@ -1153,17 +1153,34 @@ __global__ void k_gs_serial(int n, const int* rowptr, const int* col, const doub
         x[i] = xi;
     }
 }
-// ---- multicolour variant (documented ordering difference): greedy colouring by independent-set peeling
-__global__ void k_colour_round(int n, const int* __restrict__ rowptr, const int* __restrict__ col, int* colour, int round, int* remaining) {
-    // a row joins colour `round` if it is uncoloured and has the smallest index among its uncoloured neighbours
+// ---- multicolour variant (a different ordering): the greedy colouring in row order, colour(i) = the smallest colour that no stored
+// lower neighbour j < i has. It is built in rounds: row i is coloured in the first round in which every lower neighbour was coloured
+// in an EARLIER round (`coloured_in`, -1 while uncoloured). A neighbour coloured in the same round, or a racing read of its write,
+// reads as `round` or -1 and defers i, so each row sees the final colours of all its lower neighbours: the result is the sequential
+// greedy colouring whatever the thread timing. On a structurally symmetric pattern it is a proper colouring (an upper neighbour j of
+// i has i as a lower neighbour), so the rows of one colour are independent. st[0] counts the rows left, st[1] = 1 + the largest colour.
+__global__ void k_colour_round(int n, const int* __restrict__ rowptr, const int* __restrict__ col, int* colour, int* coloured_in, int round,
+                               int* st) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || colour[i] >= 0) return;
-    bool ok = true;
-    for (int k = rowptr[i]; k < rowptr[i + 1] && ok; ++k) {
+    if (i >= n || coloured_in[i] >= 0) return;
+    const int lo = rowptr[i], hi = rowptr[i + 1];
+    for (int k = lo; k < hi; ++k) {
         int j = col[k];
-        if (j < i) { int cj = ((volatile int*)colour)[j]; if (cj < 0 || cj == round) ok = false; }
+        if (j < i) { int rj = ((volatile int*)coloured_in)[j]; if (rj < 0 || rj >= round) { atomicAdd(st, 1); return; } }
     }
-    if (ok) colour[i] = round; else atomicAdd(remaining, 1);
+    // smallest colour unused by the lower neighbours, 64 candidates per pass (it is at most their number, so the loop ends)
+    int c = 0;
+    for (int base = 0;; base += 64) {
+        unsigned long long used = 0;
+        for (int k = lo; k < hi; ++k) {
+            int j = col[k];
+            if (j < i) { int d = colour[j] - base; if (d >= 0 && d < 64) used |= 1ull << d; }
+        }
+        if (~used) { c = base + __ffsll((long long)~used) - 1; break; }
+    }
+    colour[i] = c;
+    coloured_in[i] = round;
+    atomicMax(st + 1, c + 1);
 }
 __global__ void k_gs_colour(int n, const int* __restrict__ rowptr, const int* __restrict__ col, const double* __restrict__ val,
                             const int* __restrict__ diag, const double* __restrict__ b, double* x, double w, double one_minus_w,
@@ -1193,18 +1210,25 @@ static void gauss_seidel(Ctx& c, DCsr& A, const double* b, double* x, const Solv
     csr_ensure_diag(c, A);
     const double w = sp.relaxation, omw = 1. - sp.relaxation;
     if (sp.gs_mode == ORC_GS_MULTICOLOUR) {
-        DBuf<int> colour(&c, n), rem(&c, 1);
-        ORC_CUDA(cudaMemsetAsync(colour.p, 0xff, sizeof(int) * (size_t)n, c.stream));
+        // a one-sided entry (i stores j, j does not store i) could give i and j one colour, and one sweep would then write x_j
+        // while another row of the colour reads it
+        csr_check_symmetry(c, A);
+        ORC_REQUIRE(A.sym == 1, ORC_E_UNSUPPORTED,
+                    "multicolour Gauss-Seidel needs a structurally symmetric pattern ((i, j) stored exactly when (j, i) is stored)");
+        DBuf<int> colour(&c, n), coloured_in(&c, n), st(&c, 2);
+        ORC_CUDA(cudaMemsetAsync(coloured_in.p, 0xff, sizeof(int) * (size_t)n, c.stream));
         int ncol = 0;
-        for (;; ++ncol) {
-            rem.zero();
-            k_colour_round<<<(n + 255) / 256, 256, 0, c.stream>>>(n, A.rowptr, A.col, colour, ncol, rem);
+        for (int round = 0;; ++round) {
+            // every round colours at least the lowest uncoloured row
+            ORC_REQUIRE(round < n, ORC_E_INTERNAL, "multicolour GS: colouring did not terminate");
+            st.zero();
+            k_colour_round<<<(n + 255) / 256, 256, 0, c.stream>>>(n, A.rowptr, A.col, colour, coloured_in, round, st);
             c.after_launch("k_colour_round");
-            int h = 0;
-            rem.download(&h);
+            int h[2] = {0, 0};
+            st.download(h);
             c.sync();
-            if (h == 0) { ++ncol; break; }
-            ORC_REQUIRE(ncol < 4096, ORC_E_INTERNAL, "multicolour GS: colouring did not terminate");
+            ncol = std::max(ncol, h[1]);
+            if (h[0] == 0) break;
         }
         for (uint64_t it = 0; it < sp.iterations; ++it)
             for (int q = 0; q < ncol; ++q) {

@@ -64,7 +64,7 @@ class RestrictionMethods(enum.IntEnum):  # src/lib.rs:197-201
 class GaussSeidelMode(enum.IntEnum):
     ReferencePanic = 0   # what the reference does: "Gauss-Seidel out for maintenance :)" (src/linear_algebra.rs:245)
     Lexicographic = 1    # intended forward SOR sweep, exact
-    Multicolour = 2      # documented ordering difference
+    Multicolour = 2      # greedy colouring in row order, colours swept in ascending order (DESIGN.md §5)
 
 
 class AssemblyMode(enum.IntEnum):

@@ -191,17 +191,6 @@ def test_gauss_seidel_reference_mode_reports_the_panic(ctx):
     assert e.value.code == orc_b200._lib.E_GS_MAINTENANCE
 
 
-def test_gauss_seidel_multicolour_converges(ctx):
-    from orc_b200.settings import GaussSeidelMode
-    a = random_spd_like(800, 0.01, seed=15)
-    g = la.CsrMatrix.from_scipy(a, ctx)
-    xs = np.random.default_rng(7).standard_normal(800)
-    b = a @ xs
-    x = np.zeros(800)
-    la.iterative_solve(g, b, x, 60, SolutionMethod.GaussSeidel, 1.0, 1e-3, PreconditionMethod.NONE, gs_mode=GaussSeidelMode.Multicolour)
-    assert rel_l2(x, xs) < 1e-6
-
-
 @pytest.mark.parametrize("n,density,sym", [(2, 1.0, True), (33, 0.3, True), (1001, 0.006, True), (4000, 0.002, True), (500, 0.02, False)])
 def test_restriction_strongest_bit_exact(oracle, ctx, n, density, sym):
     a = random_spd_like(n, density, seed=20 + n, sym=sym)
