@@ -47,8 +47,6 @@ static MV view(const DMesh& d) {
     return m;
 }
 
-constexpr int kAsmChunk = 16;   // cells per block ticket of k_momentum_dataflow: 128 threads, eight lanes per cell
-
 template <class T>
 static void up(Ctx& c, DBuf<T>& b, const std::vector<T>& h) {
     b.alloc(&c, std::max<size_t>(h.size(), 1));
@@ -86,17 +84,6 @@ std::unique_ptr<DMesh> mesh_upload(Ctx& c, const HostMesh& m) {
     for (size_t r = 0; r + 1 < m.rowptr.size(); ++r) d->max_row = std::max(d->max_row, (int)(m.rowptr[r + 1] - m.rowptr[r]));
     up(c, d->level_ptr, m.level_ptr); up(c, d->level_order, m.level_order);
     for (int l = 0; l < d->nlevels; ++l) d->max_level_width = std::max(d->max_level_width, m.level_ptr[l + 1] - m.level_ptr[l]);
-    {   // block chunks of the dataflow assembly: up to kAsmChunk consecutive positions of level_order, all of one level
-        std::vector<int> cp;
-        cp.push_back(0);
-        for (int l = 0; l < d->nlevels; ++l)
-            for (int b = m.level_ptr[l]; b < m.level_ptr[l + 1]; b += kAsmChunk) cp.push_back(std::min(b + kAsmChunk, m.level_ptr[l + 1]));
-        d->asm_nchunks = (int)cp.size() - 1;
-        up(c, d->asm_chunk_ptr, cp);
-        d->asm_ready.alloc(&c, (size_t)std::max<int64_t>(m.n_cells, 1));
-        d->asm_ready.zero();
-        d->asm_ticket.alloc(&c, 1);
-    }
     c.sync();
     mesh_refresh_zones(c, *d, m);
     return d;
@@ -413,25 +400,9 @@ struct FluxIn {
 template <bool COHERENT>
 __device__ __forceinline__ double ld_diag(const double* d, int i) { return COHERENT ? __ldcg(d + i) : d[i]; }
 
-// The per-cell ready flags of the dataflow assembly. Writer: diagonals with st.cg, then st.release.gpu on the flag (MEMBAR.GPU + store).
-// Reader: polls the flag with a RELAXED gpu-scope load and then reads the diagonals with ld.cg, i.e. from L2, the point of
-// coherence — the loads are issued only after the loop has left (no speculation), and nothing is served from L1, so no acquire
-// fence is needed. (ld.acquire.gpu compiles to LDG.STRONG.GPU + CCTL.IVALL: every poll would invalidate the SM's whole L1 — measured:
-// the assembly took 22 ms instead of 5.)
-__device__ __forceinline__ int ld_relaxed_gpu(const int* p) {
-    int v;
-    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_gpu(int* p, int v) { asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-constexpr long long kAsmSpinLimit = 1ll << 24;
-
-// `ready` != nullptr (dataflow assembly): an owned neighbour with a lower id must have published its new diagonals (flag == epoch)
-// before they are read — the reference's in-place loop has already been there (Q2). Everything that does not depend on them is
-// loaded first, so that those loads are in flight while the lane waits.
 template <bool COHERENT>
 __device__ __forceinline__ double face_flux(const MV& m, const FluxIn& in, int f, int cell, V3 n, V3 diag_i, const double* du,
-                                            const double* dv, const double* dw, int* flags, const int* ready = nullptr, int epoch = 0) {
+                                            const double* dv, const double* dw, int* flags) {
     const int z = m.fz[f], zt = m.zt[z];
     switch (zt) {
         case ORC_BC_WALL: case ORC_BC_SYMMETRY: return 0.;
@@ -447,12 +418,6 @@ __device__ __forceinline__ double face_flux(const MV& m, const FluxIn& in, int f
             V3 g_i = v3(in.gx[cell], in.gy[cell], in.gz[cell]), g_j = v3(in.gx[nb], in.gy[nb], in.gz[nb]);
             double vol_i = m.vol[cell], vol_j = m.vol[nb];
             const double p_i = in.p[cell], p_j = in.p[nb];
-            if (COHERENT && ready != nullptr && nb < cell && nb >= m.lo) {
-                long long spins = 0;
-                while (ld_relaxed_gpu(ready + nb) != epoch) {
-                    if (++spins > kAsmSpinLimit) { atomicOr(flags, DF_SPIN); break; }
-                }
-            }
             double a_j = vnorm(v3(ld_diag<COHERENT>(du, nb) * n.x, ld_diag<COHERENT>(dv, nb) * n.y, ld_diag<COHERENT>(dw, nb) * n.z));
             double term_1 = vdot(vadd(vel_i, vel_j), n);
             double term_2 = (vol_i / a_i + vol_j / a_j) * (p_i - p_j) / vnorm(d);
@@ -725,8 +690,6 @@ struct MomArgs {
     int momentum, limiter;
     double rho;
     int* flags;
-    int* ready = nullptr;       // dataflow assembly: per-cell flags, this call's epoch
-    int epoch = 0;
 };
 
 // The advective neighbour coefficient a_nb of one face (discretization.rs:217-286), shared by the one-thread and the eight-lane
@@ -836,7 +799,7 @@ __device__ __forceinline__ void momentum_cell8(const MomArgs& a, int i, unsigned
             const int nb = m.cf_nb[q];
             const V3 n_out = outward(m, f, i);
             const double area = m.area[f];
-            const double face_flux_v = face_flux<COHERENT>(m, a.in, f, i, n_out, diag_i, a.du_in, a.dv_in, a.dw_in, a.flags, a.ready, a.epoch);
+            const double face_flux_v = face_flux<COHERENT>(m, a.in, f, i, n_out, diag_i, a.du_in, a.dv_in, a.dw_in, a.flags);
             f_i = face_flux_v * area * a.rho;
             const double face_pressure = a.pface[f];
             a_nb = neighbour_coefficient(a, i, nb, f_i, cvel);
@@ -882,7 +845,6 @@ __device__ __forceinline__ void momentum_cell8(const MomArgs& a, int i, unsigned
     a.au[di] = nu_; a.av[di] = nv_; a.aw[di] = nw_;
     if (COHERENT) { __stcg(a.du_out + i, nu_); __stcg(a.dv_out + i, nv_); __stcg(a.dw_out + i, nw_); }
     else { a.du_out[i] = nu_; a.dv_out[i] = nv_; a.dw_out[i] = nw_; }
-    if (COHERENT && a.ready != nullptr) st_release_gpu(a.ready + i, a.epoch);   // the new diagonals are out: higher neighbours may read them
 }
 
 // Exact mode: cells grouped by dependency level (level(i) = 1 + max level of neighbours j < i); one
@@ -898,26 +860,6 @@ __global__ void __launch_bounds__(128) k_momentum_levels(MomArgs a, const int* _
         const int b = level_ptr[L], e = level_ptr[L + 1];
         for (int idx = b + (gtid >> 3); idx < e; idx += (gsz >> 3)) momentum_cell8<true>(a, level_order[idx], gmask, gl);
         grid.sync();
-    }
-}
-// The same recurrence without grid barriers: blocks take chunks of level_order by atomic ticket (a chunk never crosses a level, so
-// the cells of a block are independent of each other); a face whose neighbour has a lower id waits for THAT cell's ready flag
-// only. A cell of level L can only wait for cells of lower levels, i.e. of earlier tickets, whose blocks are already running:
-// no cooperative launch needed, no deadlock. What a level costs is one flag round trip plus the flux arithmetic behind it instead
-// of a grid barrier plus the whole load chain of a cell (the loads are issued before the wait).
-__global__ void __launch_bounds__(128) k_momentum_dataflow(MomArgs a, const int* __restrict__ chunk_ptr, int nchunks, const int* __restrict__ level_order,
-                                                           unsigned int* ticket) {
-    __shared__ unsigned int s_ticket;
-    const int grp = threadIdx.x >> 3, gl = threadIdx.x & 7;
-    const unsigned gmask = 0xffu << (threadIdx.x & 24);
-    for (;;) {
-        __syncthreads();
-        if (threadIdx.x == 0) s_ticket = atomicAdd(ticket, 1u);
-        __syncthreads();
-        const unsigned int t = s_ticket;
-        if (t >= (unsigned int)nchunks) return;
-        const int pos = chunk_ptr[t] + grp;
-        if (pos < chunk_ptr[t + 1]) momentum_cell8<true>(a, level_order[pos], gmask, gl);
     }
 }
 // No recurrence (Linear / LinearWeighted face velocity, or frozen mode): plain cell-parallel launch.
@@ -1000,27 +942,6 @@ void build_momentum_advection(Ctx& c, const DMesh& d, AsmWork& w, const AsmSetti
     const bool recurrence = (s.v_interp == ORC_V_RHIE_CHOW);
     if (recurrence && s.assembly_mode == ORC_ASSEMBLY_EXACT) {
         a.du_in = du; a.dv_in = dv; a.dw_in = dw;
-        // Lab variant, off by default (ORC_B200_ASM_DATAFLOW=1): bit-identical, but measured SLOWER than the grid-barrier kernel at 128^3
-        // (21.8 vs 5.1 ms per assembly; 2.4 ms with the waits compiled out, so the flag waits themselves cost ~50 us per dependency
-        // level; neither dropping the release fence nor a poll back-off nor static chunk assignment changes that:
-        // profiles/r2_assembly_dataflow_lab.txt).
-        static const bool dataflow = [] { const char* e = getenv("ORC_B200_ASM_DATAFLOW"); return e && atoi(e) != 0; }();
-        if (dataflow && d.asm_nchunks > 0) {
-            int per_sm_df = 0;
-            ORC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_df, k_momentum_dataflow, 128, 0));
-            ORC_REQUIRE(per_sm_df > 0, ORC_E_CUDA, "k_momentum_dataflow cannot be made resident");
-            a.ready = d.asm_ready.p;
-            a.epoch = ++d.asm_epoch;
-            ORC_CUDA(cudaMemsetAsync(d.asm_ticket.p, 0, sizeof(unsigned int), c.stream));
-            k_momentum_dataflow<<<std::min(per_sm_df * c.sm_count, d.asm_nchunks), 128, 0, c.stream>>>(a, d.asm_chunk_ptr.p, d.asm_nchunks, d.level_order.p,
-                                                                                                   d.asm_ticket.p);
-            c.after_launch("k_momentum_dataflow");
-            if (peclet3_dev) {
-                k_peclet<<<grid_for(d.N, 256, c.sm_count * 4), 256, 0, c.stream>>>((int)d.N, (int)d.own_lo, (int)d.own_hi, w.pe, c.d_partials, c.d_counter, peclet3_dev);
-                c.after_launch("k_peclet");
-            }
-            return;
-        }
         int per_sm = 0;
         ORC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_momentum_levels, 128, 0));
         ORC_REQUIRE(per_sm > 0, ORC_E_CUDA, "k_momentum_levels cannot be made resident");

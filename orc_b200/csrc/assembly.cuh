@@ -27,12 +27,6 @@ struct DMesh {
     // level schedule of the momentum recurrence
     DBuf<int> level_ptr, level_order;
     int max_level_width = 0;
-    // dataflow schedule of the same recurrence (k_momentum_dataflow): level_order cut into block chunks that never cross a level,
-    // a ready flag per cell (= the epoch of the assembly call that last wrote its diagonals), the ticket counter
-    DBuf<int> asm_chunk_ptr, asm_ready;
-    DBuf<unsigned int> asm_ticket;
-    int asm_nchunks = 0;
-    mutable int asm_epoch = 0;
     // zone table (refreshed when the host table changes)
     DBuf<int> zone_type;
     DBuf<double> zone_scalar, zone_vec;

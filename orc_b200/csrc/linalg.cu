@@ -1280,21 +1280,8 @@ static void gauss_seidel(Ctx& c, DCsr& A, const double* b, double* x, const Solv
 // `state[k]`: 0 = row k undecided, 1 = decided without a pick, 2 + j = decided and picked column j. Flag and payload
 // share one word, so a single store publishes the decision and a single load observes it: no fences on the critical
 // path (one L2 round trip per dependency hop). `combined[]` is only a monotone hint for the candidate scan.
-__device__ int g_dfr_sleep_ns = 0;   // back-off between polls of the restriction kernel (set from ORC_B200_DFR_SLEEP at the first launch)
-__device__ __forceinline__ int spin_until_decided(const int* state, int* flags) {
-    long long spins = 0;
-    int v;
-    const int nap = g_dfr_sleep_ns;
-    while ((v = *(volatile const int*)state) == 0) {
-        if (nap) __nanosleep(nap);
-        if ((++spins & 1023) == 0) {
-            if (spins > SPIN_LIMIT) { atomicOr(flags, DF_SPIN); return -1; }
-            if (*(volatile int*)flags & DF_SPIN) return -1;
-        }
-    }
-    return v;
-}
 constexpr int DFR_WARPS = 8;     // warps per block of the restriction kernel
+constexpr int DFR_SM_BLOCKS = 8;   // resident blocks per SM: 8 warps x 8 blocks = 2048 threads, a full SM
 // Ticket shape: rows a warp handles ONE AFTER THE OTHER per block ticket (a ticket covers WARPS * rows consecutive rows). A row that
 // waits for its warp has not even issued its loads when the row it depends on decides; with more than one row per warp the front of
 // a dependency chain therefore pays a whole row latency every WARPS rows instead of one flag round trip per hop
@@ -1303,16 +1290,10 @@ constexpr int DFR_WARPS = 8;     // warps per block of the restriction kernel
 // per hierarchy); the hex boxes are throughput bound — four rows per warp are 1.6 x faster (5.2 vs 8.3 ms), because a block whose
 // warps hold one row each idles until its slowest row is done. The aggregates do not depend on the shape. The rule: hierarchies of
 // simplex meshes (fine-matrix rows of <= 5 entries; DCsr::simplex is inherited by every matrix derived from the fine one) take one
-// row per warp, everything else four. ORC_B200_DFR_ROWS overrides. (A tuner that timed both shapes on the first builds was tried
-// and dropped: the momentum and the pressure matrix of a size prefer different shapes and the first iterations are not
-// representative, so it cost the hex bench 6-27 ms per iteration.)
-static int dfr_rows_small() {   // the one-block kernel (state in shared memory, 32 warps): four rows per warp unless overridden
-    static const int env = [] { const char* e = getenv("ORC_B200_DFR_ROWS"); return e ? std::max(1, std::min(16, atoi(e))) : 0; }();
-    return env ? env : 4;
-}
+// row per warp, everything else four; the one-block kernel for small systems always takes four. (A tuner that timed both shapes on
+// the first builds was tried and dropped: the momentum and the pressure matrix of a size prefer different shapes and the first
+// iterations are not representative, so it cost the hex bench 6-27 ms per iteration.)
 static int dfr_rows_for(Ctx& c, DCsr& A) {
-    static const int env = [] { const char* e = getenv("ORC_B200_DFR_ROWS"); return e ? std::max(1, std::min(16, atoi(e))) : 0; }();
-    if (env) return env;
     if (A.simplex < 0) { csr_ensure_max_row(c, A); A.simplex = (A.max_row <= 5) ? 1 : 0; }
     return A.simplex == 1 ? 1 : 4;
 }
@@ -1437,117 +1418,6 @@ __global__ void __launch_bounds__(DFR_WARPS * 32) k_strongest_dataflow(int n, co
     __shared__ unsigned int s_chunk;
     strongest_dataflow_body<DFR_WARPS>(n, rowptr, col, val, state, combined, pick, picked_by, ticket, flags, &s_chunk, rows_per_warp);
 }
-// ---- The same dataflow with G lanes per row (G = 8, 16, 32), E entries per lane, and WARP tickets. ----
-// Every row a warp owns is ACTIVE: its entries, the row bounds of its columns and its candidate's lower touchers are loaded and the
-// group polls — so when the row it depends on decides, the hop costs one flag round trip. (With several rows per warp handled one
-// after the other, the front of a dependency chain keeps arriving at rows that have not issued a single load: 240 ns per row on the
-// Kuhn-split tet slabs against 1.5 with one active row per warp, profiles/r2_restriction_rows.txt.) Short rows (fine level: 7 entries
-// hex, 5 tet) take 8 lanes, so a warp keeps four rows active and an SM 256 instead of 64.
-// Tickets are per warp (no block barrier: a warp whose rows are done moves on at once). Ticket t owns the rows
-// (t / 32) * 32 GPW + t % 32 + 32 g, g < GPW = 32 / G: consecutive rows — which usually depend on each other — go to different
-// warps, the rows of one warp are 32 apart. A row only waits for LOWER rows; those belong to tickets of the same or of earlier
-// 32-ticket groups, tickets are handed out in order and far more than 32 warps are resident, so the lowest undecided row is always
-// owned by (or about to be taken by) a running warp: no deadlock. Waits between groups of one warp rely on independent thread
-// scheduling (sm_70+).
-template <int G, int E>
-__global__ void __launch_bounds__(DFR_WARPS * 32) k_strongest_groups(int n, const int* __restrict__ rowptr, const int* __restrict__ col,
-                                                                     const double* __restrict__ val, int* state, int* combined, int* pick,
-                                                                     int* picked_by, unsigned int* ticket, int* flags) {
-    constexpr int GPW = 32 / G;
-    const int lane = threadIdx.x & 31;
-    const int gl = lane & (G - 1), grp = lane / G;
-    const unsigned int gmask = (G == 32) ? 0xffffffffu : (((1u << G) - 1u) << (grp * G));
-    const unsigned int ntickets = (unsigned int)(((n + 32 * GPW - 1) / (32 * GPW)) * 32);
-    for (;;) {
-        unsigned int t = 0;
-        if (lane == 0) t = atomicAdd(ticket, 1u);
-        t = __shfl_sync(0xffffffffu, t, 0);
-        if (t >= ntickets) return;
-        const long long il = (long long)(t >> 5) * (32 * GPW) + (t & 31u) + 32 * grp;
-        if (il < n) {
-            const int i = (int)il;
-            const int lo = rowptr[i], hi = rowptr[i + 1];
-            int e_j[E], e_lo[E], e_hi[E];
-            double e_v[E];
-            bool e_free[E];
-#pragma unroll
-            for (int e = 0; e < E; ++e) {
-                const int k = lo + e * G + gl;
-                e_j[e] = -1; e_lo[e] = 0; e_hi[e] = 0; e_v[e] = 0.; e_free[e] = false;
-                if (k < hi) { e_j[e] = col[k]; e_v[e] = val[k]; e_free[e] = (e_j[e] != i); }
-            }
-#pragma unroll
-            for (int e = 0; e < E; ++e)
-                if (e_free[e]) { e_lo[e] = rowptr[e_j[e]]; e_hi[e] = rowptr[e_j[e] + 1]; }
-            int chosen = -1;
-            bool give_up = false;
-            for (;;) {
-                int cb[E];
-#pragma unroll
-                for (int e = 0; e < E; ++e) cb[e] = e_free[e] ? *(volatile int*)(combined + e_j[e]) : 1;
-                double best = DBL_MAX;   // strongest_coeff starts at Float::MAX
-                int best_k = INT_MAX;    // position in the row: the FIRST minimum wins
-#pragma unroll
-                for (int e = 0; e < E; ++e) {
-                    if (cb[e] != 0) e_free[e] = false;
-                    if (e_free[e] && e_v[e] < best) { best = e_v[e]; best_k = lo + e * G + gl; }   // e ascending = k ascending within the lane
-                }
-#pragma unroll
-                for (int o = G / 2; o > 0; o >>= 1) {   // group argmin on (value, position): symmetric, every lane ends with the result
-                    const double ov = __shfl_xor_sync(gmask, best, o);
-                    const int ok = __shfl_xor_sync(gmask, best_k, o);
-                    if (ok != INT_MAX && (best_k == INT_MAX || ov < best || (ov == best && ok < best_k))) { best = ov; best_k = ok; }
-                }
-                if (best_k == INT_MAX) break;  // nothing available: row i pushes nothing
-                const int we = (best_k - lo) / G, src = grp * G + ((best_k - lo) & (G - 1));
-                int sj = e_j[0], sl = e_lo[0], sh_ = e_hi[0];
-#pragma unroll
-                for (int e = 1; e < E; ++e) if (we == e) { sj = e_j[e]; sl = e_lo[e]; sh_ = e_hi[e]; }
-                const int j = __shfl_sync(gmask, sj, src), jlo = __shfl_sync(gmask, sl, src), jhi = __shfl_sync(gmask, sh_, src);
-                // every row that can take j before row i is a LOWER TOUCHER of j (see strongest_dataflow_body)
-                int taken = 0, bad = 0;
-                for (int base = jlo; base < jhi && !taken; base += G) {
-                    const int kk = base + gl;
-                    int k = INT_MAX;
-                    if (kk < jhi) k = col[kk];
-                    const bool mine = (k < i && k != j);
-                    long long spins = 0;
-                    for (;;) {
-                        int st = 1;
-                        if (mine) st = *(volatile const int*)(state + k);
-                        const unsigned int took = __ballot_sync(gmask, mine && st == 2 + j);
-                        const unsigned int pending = __ballot_sync(gmask, mine && st == 0);
-                        if (took) { taken = 1; break; }
-                        if (!pending) break;
-                        if ((++spins & 1023) == 0) {
-                            int stop = 0;
-                            if (spins > SPIN_LIMIT) { atomicOr(flags, DF_SPIN); stop = 1; }
-                            else if (*(volatile int*)flags & DF_SPIN) stop = 1;
-                            if (__any_sync(gmask, stop)) { bad = 1; break; }
-                        }
-                    }
-                    if (bad) break;
-                    if (__any_sync(gmask, k >= i)) break;   // columns ascend: no lower toucher follows
-                }
-                if (bad) { give_up = true; break; }
-                if (!taken) { chosen = j; break; }
-                if (gl == 0) *(volatile int*)(combined + j) = 1;  // hint for later scans
-#pragma unroll
-                for (int e = 0; e < E; ++e) if (e_j[e] == j) e_free[e] = false;
-                __syncwarp(gmask);
-            }
-            if (gl == 0) {
-                if (chosen >= 0) {
-                    *(volatile int*)(combined + chosen) = 1;
-                    picked_by[chosen] = i;
-                }
-                pick[i] = chosen;
-                *(volatile int*)(state + i) = (chosen >= 0 && !give_up) ? 2 + chosen : 1;
-            }
-        }
-        __syncwarp();
-    }
-}
 // one block, `state` and `combined` in shared memory (2 n ints): systems of up to kStrongestSmallRows rows
 constexpr int kStrongestSmallRows = 24576;
 __global__ void __launch_bounds__(1024, 1) k_strongest_small(int n, const int* __restrict__ rowptr, const int* __restrict__ col,
@@ -1668,43 +1538,18 @@ CsrPtr build_restriction(Ctx& c, DCsr& A, int method, CsrPtr* rt_out) {
                 ORC_CUDA(cudaFuncSetAttribute(k_strongest_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * kStrongestSmallRows * sizeof(int))));
                 attr_set = true;
             }
-            k_strongest_small<<<1, 1024, 2 * (size_t)n * sizeof(int), c.stream>>>(n, A.rowptr, A.col, A.val, pick, picked_by, c.d_flags, dfr_rows_small());
+            k_strongest_small<<<1, 1024, 2 * (size_t)n * sizeof(int), c.stream>>>(n, A.rowptr, A.col, A.val, pick, picked_by, c.d_flags, 4);
             c.after_launch("k_strongest_small");
         } else if (A.sym == 1) {
             DBuf<int> decided(&c, n);
             DBuf<unsigned int> ticket(&c, 1);
             decided.zero();
             ticket.zero();
-            // lab variant, off by default (bit-exact, measured slower than the block-ticket kernel: profiles/r2_restriction_rows.txt)
-            static const bool groups_on = [] { const char* e = getenv("ORC_B200_DFR_GROUPS"); return e && atoi(e) != 0; }();
-            if (groups_on && A.max_row > 0 && A.max_row <= 128) {
-                const int per_sm = 2048 / (DFR_WARPS * 32);
-                auto go = [&](auto kern, int gpw) {
-                    const long long ntickets = ((n + 32LL * gpw - 1) / (32LL * gpw)) * 32;
-                    const int grid = (int)std::max<long long>(1, std::min<long long>((ntickets + DFR_WARPS - 1) / DFR_WARPS, (long long)c.sm_count * per_sm));
-                    kern<<<grid, DFR_WARPS * 32, 0, c.stream>>>(n, A.rowptr, A.col, A.val, decided, combined, pick, picked_by, ticket, c.d_flags);
-                    c.after_launch("k_strongest_groups");
-                };
-                const int m = A.max_row;
-                if (m <= 8) go(k_strongest_groups<8, 1>, 4);
-                else if (m <= 16) go(k_strongest_groups<8, 2>, 4);
-                else if (m <= 32) go(k_strongest_groups<16, 2>, 2);
-                else if (m <= 64) go(k_strongest_groups<32, 2>, 1);
-                else go(k_strongest_groups<32, 4>, 1);
-            } else {
             const int rows = dfr_rows_for(c, A);
             const int nchunks = (n + DFR_WARPS * rows - 1) / (DFR_WARPS * rows);
-            static const int blocks_per_sm = [] {   // lab knobs (profiles/r2_restriction_knobs.txt): resident blocks per SM, poll back-off
-                const char* e = getenv("ORC_B200_DFR_BLOCKS");
-                const char* z = getenv("ORC_B200_DFR_SLEEP");
-                const int nap = z ? atoi(z) : 0;
-                cudaMemcpyToSymbol(g_dfr_sleep_ns, &nap, sizeof(int));
-                return e ? std::max(1, std::min(8, atoi(e))) : 8;
-            }();
-            k_strongest_dataflow<<<std::max(1, std::min(nchunks, c.sm_count * blocks_per_sm)), DFR_WARPS * 32, 0, c.stream>>>(
+            k_strongest_dataflow<<<std::max(1, std::min(nchunks, c.sm_count * DFR_SM_BLOCKS)), DFR_WARPS * 32, 0, c.stream>>>(
                 n, A.rowptr, A.col, A.val, decided, combined, pick, picked_by, ticket, c.d_flags, rows);
             c.after_launch("k_strongest_dataflow");
-            }
         } else {
             k_strongest_serial<<<1, 32, 0, c.stream>>>(n, A.rowptr, A.col, A.val, combined, pick, picked_by);
             c.after_launch("k_strongest_serial");
