@@ -58,6 +58,8 @@ enum { ORC_RESTRICT_INJECTION = 0, ORC_RESTRICT_STRONGEST = 1 };                
 /* TGRID boundary ids, src/mesh.rs:50-66 */
 enum { ORC_BC_INTERIOR = 2, ORC_BC_WALL = 3, ORC_BC_PRESSURE_INLET = 4, ORC_BC_PRESSURE_OUTLET = 5, ORC_BC_SYMMETRY = 7,
        ORC_BC_VELOCITY_INLET = 10 };
+/* passive scalar condition of a boundary zone (orc_mesh_set_zone_scalar); every zone starts as ZERO_GRADIENT */
+enum { ORC_SBC_ZERO_GRADIENT = 0, ORC_SBC_FIXED = 1 };
 /* Gauss-Seidel behaviour. The reference arm always panics (src/linear_algebra.rs:219-246). */
 enum { ORC_GS_REFERENCE_PANIC = 0, /* run nothing, return ORC_E_GS_MAINTENANCE                                   */
        ORC_GS_LEXICOGRAPHIC = 1,   /* intended forward SOR sweep in row order, exact (dataflow kernel)           */
@@ -152,6 +154,9 @@ int32_t orc_mesh_geometry_device(orc_ctx* ctx, const orc_mesh* m, double* face_a
 int32_t orc_mesh_zones(const orc_mesh* m, int64_t* ids, int64_t* types, double* scalar, double* vector3, char* names64);
 /* mesh.get_face_zone(name) + assignment of zone_type/scalar_value/vector_value (src/tests.rs:60-76) */
 int32_t orc_mesh_set_zone(orc_mesh* m, const char* name, int64_t zone_type, double scalar, double vx, double vy, double vz);
+/* the passive scalar condition of zone `name`: kind ORC_SBC_ZERO_GRADIENT or ORC_SBC_FIXED (value = phi on the zone's faces). An
+ * unknown name, another kind or a non-finite value return ORC_E_INVALID. Partitions taken afterwards inherit it. */
+int32_t orc_mesh_set_zone_scalar(orc_mesh* m, const char* name, int32_t kind, double value);
 /* the shared sparsity pattern (diag + face neighbours, sorted columns): rowptr[N+1], col[nnz] */
 int32_t orc_mesh_pattern(const orc_mesh* m, int64_t* rowptr, int64_t* col);
 /* assembly level schedule (host logic, testable without a GPU): level_of_cell[N] */
@@ -238,6 +243,21 @@ int32_t orc_steady_level_sizes(orc_steady* st, int64_t* out, int32_t cap, int32_
 /* orc_gradients of the handle's resident u, v, w, p, without their round trip through the host: the OWNED rows (n_own of a
  * partition, after a halo exchange of the four fields), same layout, NULL outputs and errors as orc_gradients. */
 int32_t orc_steady_gradients(orc_steady* st, int32_t gradient, double* grad_p3n, double* grad_u9n);
+
+/* ---- passive scalar transport on the converged flow (an extension beyond the reference; DESIGN.md §1 is its specification) ------
+ * steady div(rho u phi) - div(Gamma grad phi) = 0 with the face mass fluxes of the flow (face flux of the settings' velocity
+ * interpolation and gradient scheme, Rhie-Chow with the momentum diagonals as they are). Convection: s->momentum (UD, CD1 or TVD with
+ * s->limiter); CD2 and ORC_V_NONE return ORC_E_UNSUPPORTED. A mesh without a FIXED zone, gamma < 0 or NaN return ORC_E_INVALID. */
+/* The system of one sweep with the given phi, for parity tests (shaped after orc_build_pressure_correction): host vectors of the
+ * mesh's n_cells; a_out has the mesh pattern, b_out n_cells doubles. On a partition mesh every rank calls it together (its halo
+ * entries are refreshed from their owners) and the owned rows are the whole mesh's rows. */
+int32_t orc_build_scalar_transport(orc_ctx* ctx, orc_mesh* m, const orc_csr* a_u, const orc_csr* a_v, const orc_csr* a_w,
+                                   const double* u, const double* v, const double* w, const double* p, const double* phi,
+                                   double gamma, double rho, const orc_settings* s, orc_csr** a_out, double* b_out);
+/* `sweeps` assemble + iterative_solve sweeps (the handle's matrix solver settings) on the handle's resident flow, which is left
+ * untouched. phi: in/out, the exposed cells (owned cells of a partition; every rank calls it together). One sweep is exact for UD
+ * and CD1; TVD is a Picard iteration. */
+int32_t orc_steady_solve_scalar(orc_steady* st, double gamma, uint64_t sweeps, double* phi);
 void orc_steady_destroy(orc_steady* st);
 
 /* ---- flow initialisation: the step before the loop (src/solver.rs:246-352) ------------------------- */

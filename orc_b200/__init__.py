@@ -21,7 +21,7 @@ from .context import Context, default_context  # noqa: F401
 from .settings import (NumericalSettings, MatrixSolverSettings, MomentumDiscretization, PressureInterpolation,  # noqa: F401
                        VelocityInterpolation, GradientReconstructionMethods, SolutionMethod, PreconditionMethod,
                        RestrictionMethods, TVD_LUD, TVD_QUICK, TVD_UMIST)
-from .mesh import Mesh, FaceConditionTypes  # noqa: F401
+from .mesh import Mesh, FaceConditionTypes, ScalarCondition  # noqa: F401
 from .io import read_mesh, read_data, write_data, write_gradients  # noqa: F401
 from .linear_algebra import CsrMatrix, iterative_solve  # noqa: F401
 from .solver import (solve_steady, SteadySolver, initialize_flow, initialize_flow_new, check_boundary_conditions,  # noqa: F401

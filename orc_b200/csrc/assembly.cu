@@ -92,13 +92,15 @@ std::unique_ptr<DMesh> mesh_upload(Ctx& c, const HostMesh& m) {
 void mesh_refresh_zones(Ctx& c, DMesh& d, const HostMesh& m) {
     if (d.zone_epoch == m.zone_epoch) return;
     const size_t Z = m.zones.size();
-    std::vector<int> zt(Z);
-    std::vector<double> zs(Z), zv(3 * Z);
+    std::vector<int> zt(Z), sk(Z);
+    std::vector<double> zs(Z), zv(3 * Z), sv(Z);
     for (size_t k = 0; k < Z; ++k) {
         zt[k] = m.zones[k].type; zs[k] = m.zones[k].scalar;
         zv[3 * k] = m.zones[k].vec[0]; zv[3 * k + 1] = m.zones[k].vec[1]; zv[3 * k + 2] = m.zones[k].vec[2];
+        sk[k] = m.zones[k].scalar_bc_kind; sv[k] = m.zones[k].scalar_bc_value;
     }
     up(c, d.zone_type, zt); up(c, d.zone_scalar, zs); up(c, d.zone_vec, zv);
+    up(c, d.zone_sbc_kind, sk); up(c, d.zone_sbc_value, sv);
     c.sync();
     d.nzones = (int)Z;
     d.zone_epoch = m.zone_epoch;
@@ -1092,6 +1094,167 @@ void extract_diagonal(Ctx& c, const DCsr& a, double* d) {
     ORC_REQUIRE(a.diag != nullptr, ORC_E_INTERNAL, "extract_diagonal: diagonal index not built");
     k_extract_diag<<<grid_for(a.nrows, 256, c.sm_count * 8), 256, 0, c.stream>>>((int)a.nrows, a.rowptr, a.diag, a.val, d, c.d_flags);
     c.after_launch("k_extract_diag");
+}
+
+// -------------------------------------------------------------------------------------------------
+// S1-S3: passive scalar transport, div(rho u phi) - div(Gamma grad phi) = 0 on the resident flow. Not in the reference: the
+// discretisation below is its own specification (DESIGN.md §1), restated operator for operator by tests/scalar_oracle.
+// -------------------------------------------------------------------------------------------------
+void validate_scalar_settings(const AsmSettings& s) {
+    if (s.momentum != ORC_MOM_UD && s.momentum != ORC_MOM_CD1 && s.momentum != ORC_MOM_TVD)
+        throw Error(ORC_E_UNSUPPORTED, "unsupported convection scheme");
+    if (s.momentum == ORC_MOM_TVD && (s.limiter < ORC_PSI_UD || s.limiter > ORC_PSI_UMIST)) throw Error(ORC_E_INVALID, "unknown TVD limiter");
+    if (s.v_interp != ORC_V_LINEAR && s.v_interp != ORC_V_LINEAR_WEIGHTED && s.v_interp != ORC_V_RHIE_CHOW)
+        throw Error(ORC_E_UNSUPPORTED, "`None` VelocityInterpolation cannot be used for interior faces");
+    if (s.gradient != ORC_G_GREEN_GAUSS_CELL && s.gradient != ORC_G_LEAST_SQUARES) throw Error(ORC_E_UNSUPPORTED, "unsupported gradient scheme");
+}
+
+// S1: F_f once per face, from the side of c0 (the outward normal of c0 is the face normal). Cell c1 uses -F_f, which is bit for bit
+// what face_flux evaluates from c1's side: every sum in it commutes, vunit(-d) == -vunit(d) and the norms ignore the sign.
+__global__ void __launch_bounds__(128) k_scalar_face_flux(MV m, FluxIn in, const double* __restrict__ du, const double* __restrict__ dv,
+                                                          const double* __restrict__ dw, double* F, int* flags) {
+    for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < m.F; f += gridDim.x * blockDim.x) {
+        const int c0 = m.c0[f];
+        F[f] = face_flux<false>(m, in, f, c0, fnormal(m, f), v3(du[c0], dv[c0], dw[c0]), du, dv, dw, flags);
+    }
+}
+
+// the value of phi on face f as the gradient sees it from cell i: mean of the two cells, the fixed value, or phi_i
+__device__ __forceinline__ double scalar_face_value(const MV& m, const int* zk, const double* zval, const double* phi, int f, int i) {
+    const int z = m.fz[f];
+    if (m.zt[z] == ORC_BC_INTERIOR) return (phi[m.c0[f]] + phi[m.c1[f]]) * 0.5;
+    return (zk[z] == ORC_SBC_FIXED) ? zval[z] : phi[i];
+}
+// S2 (TVD only): Green-Gauss cell-based grad phi = sum n_out * ((phi_f * A_f) / V_P), plain Vector * Float products
+__global__ void __launch_bounds__(128) k_scalar_grad(MV m, const int* __restrict__ zk, const double* __restrict__ zval, const double* __restrict__ phi,
+                                                     double* gx, double* gy, double* gz) {
+    for (int i = m.lo + blockIdx.x * blockDim.x + threadIdx.x; i < m.hi; i += gridDim.x * blockDim.x) {
+        V3 acc = vzero();
+        const double vol = m.vol[i];
+        for (int q = m.cf_ptr[i]; q < m.cf_ptr[i + 1]; ++q) {
+            const int f = m.cf_face[q];
+            const double s = scalar_face_value(m, zk, zval, phi, f, i) * m.area[f] / vol;
+            acc = vadd(acc, vmuls(outward(m, f, i), s));
+        }
+        gx[i] = acc.x; gy[i] = acc.y; gz[i] = acc.z;
+    }
+}
+
+struct ScalarArgs {
+    MV m;
+    const double *F, *phi, *gx, *gy, *gz;
+    const int* zk;
+    const double* zval;
+    double gamma, rho;
+    int scheme, limiter;
+    double *val, *b;
+};
+// min(f, 0) and max(f, 0) as comparisons: both cells of a face see the same zero whatever the sign of a zero flux
+__device__ __forceinline__ double neg_part(double f) { return f < 0. ? f : 0.; }
+__device__ __forceinline__ double pos_part(double f) { return f > 0. ? f : 0.; }
+
+// S3: one thread per owned cell, faces in ascending order, values straight into the mesh pattern through cf_slot. f is the mass
+// flux out of P: (rho * A_f) * (+-F_f). Interior face: a_P += d, a_N -= d (d = Gamma A_f / |x_N - x_P|), then the convective
+// coefficients of the face value. TVD decides the upwind cell U on the sign of the c0-side flux, so both cells of a face use the
+// same U, D and w = psi(r) / 2 (conservative). Boundary: FIXED a_P += d_b + max(f, 0), b += (d_b - min(f, 0)) phi_b with
+// d_b = Gamma A_f / |x_f - x_P|; ZERO_GRADIENT a_P += f.
+__global__ void __launch_bounds__(128) k_scalar_transport(ScalarArgs a) {
+    const MV& m = a.m;
+    for (int i = m.lo + blockIdx.x * blockDim.x + threadIdx.x; i < m.hi; i += gridDim.x * blockDim.x) {
+        double a_p = 0., b_p = 0.;
+        const V3 cc = ccentroid(m, i);
+        // duplicate (i, nb) pairs add up: clear the off-diagonals first
+        for (int q = m.cf_ptr[i]; q < m.cf_ptr[i + 1]; ++q) if (m.cf_slot[q] >= 0) a.val[m.cf_slot[q]] = 0.;
+        for (int q = m.cf_ptr[i]; q < m.cf_ptr[i + 1]; ++q) {
+            const int f = m.cf_face[q];
+            const int z = m.fz[f];
+            const int c0 = m.c0[f];
+            const double area = m.area[f];
+            const double Ff = a.F[f];
+            const double fl = (a.rho * area) * ((c0 == i) ? Ff : -Ff);
+            if (m.zt[z] == ORC_BC_INTERIOR) {
+                const int nb = (c0 == i) ? m.c1[f] : c0;
+                const int slot = m.cf_slot[q];
+                const double d = a.gamma * area / vnorm(vsub(ccentroid(m, nb), cc));
+                double c_p, c_n;
+                if (a.scheme == ORC_MOM_UD) {
+                    c_n = neg_part(fl);
+                    c_p = fl - c_n;
+                } else if (a.scheme == ORC_MOM_CD1) {
+                    c_n = fl / 2.;
+                    c_p = fl - c_n;
+                } else {
+                    const int up = (Ff >= 0.) ? c0 : m.c1[f];
+                    const int dn = (up == c0) ? m.c1[f] : c0;
+                    const double phi_u = a.phi[up], phi_d = a.phi[dn];
+                    double w = 0.5;
+                    if (phi_d != phi_u) {
+                        const V3 g_u = v3(a.gx[up], a.gy[up], a.gz[up]);
+                        const double r = 2. * vdot(g_u, vsub(ccentroid(m, dn), ccentroid(m, up))) / (phi_d - phi_u) - 1.;
+                        w = psi(a.limiter, r) / 2.;
+                    }
+                    const double c_up = (1. - w) * fl, c_dn = w * fl;
+                    if (up == i) { c_p = c_up; c_n = c_dn; } else { c_p = c_dn; c_n = c_up; }
+                }
+                a_p = a_p + d;
+                a_p = a_p + c_p;
+                a.val[slot] = a.val[slot] - d;
+                a.val[slot] = a.val[slot] + c_n;
+            } else if (a.zk[z] == ORC_SBC_FIXED) {
+                const double d_b = a.gamma * area / vnorm(vsub(fcentroid(m, f), cc));
+                a_p = a_p + (d_b + pos_part(fl));
+                b_p = b_p + (d_b - neg_part(fl)) * a.zval[z];
+            } else {
+                a_p = a_p + fl;
+            }
+        }
+        a.val[m.diag[i]] = a_p;
+        a.b[i] = b_p;
+    }
+}
+
+void scalar_face_flux(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& s, const double* du, const double* dv, const double* dw,
+                      const double* u, const double* v, const double* wv, const double* p) {
+    validate_scalar_settings(s);
+    const size_t N = (size_t)std::max<int64_t>(d.N, 1), F = (size_t)std::max<int64_t>(d.F, 1);
+    if (w.F.n != F) w.F.alloc(&c, F);
+    if (w.gpx.n != N) { w.gpx.alloc(&c, N); w.gpy.alloc(&c, N); w.gpz.alloc(&c, N); w.gpx.zero(); w.gpy.zero(); w.gpz.zero(); }
+    if (d.F == 0) return;
+    const MV m = view(d);
+    if (s.v_interp == ORC_V_RHIE_CHOW) {
+        if (d.N > 0) launch_grad_p(c, m, s.gradient, p, w.gpx, w.gpy, w.gpz);
+        if (w.halo_exchange) { double* g[3] = {w.gpx.p, w.gpy.p, w.gpz.p}; w.halo_exchange(g, 3); }
+    }
+    FluxIn in;
+    in.u = u; in.v = v; in.w = wv; in.p = p; in.gx = w.gpx; in.gy = w.gpy; in.gz = w.gpz; in.v_interp = s.v_interp;
+    ProfScope ps(c, PC_ASSEMBLY, 0.);
+    k_scalar_face_flux<<<grid_for(d.F, 128, c.sm_count * 16), 128, 0, c.stream>>>(m, in, du, dv, dw, w.F, c.d_flags);
+    c.after_launch("k_scalar_face_flux");
+}
+
+void build_scalar_transport(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& s, double gamma, double rho, const double* phi,
+                            DCsr& a, double* b) {
+    validate_scalar_settings(s);
+    ORC_REQUIRE(w.F.n == (size_t)std::max<int64_t>(d.F, 1), ORC_E_INTERNAL, "build_scalar_transport: face fluxes not computed");
+    const size_t N = (size_t)std::max<int64_t>(d.N, 1);
+    if (w.hx.n != N) { w.hx.alloc(&c, N); w.hy.alloc(&c, N); w.hz.alloc(&c, N); w.hx.zero(); w.hy.zero(); w.hz.zero(); }
+    if (d.N == 0) return;
+    const MV m = view(d);
+    const int g = grid_for(d.N, 128, c.sm_count * 16);
+    if (s.momentum == ORC_MOM_TVD) {
+        {
+            ProfScope ps(c, PC_ASSEMBLY, 0.);
+            k_scalar_grad<<<g, 128, 0, c.stream>>>(m, d.zone_sbc_kind, d.zone_sbc_value, phi, w.hx, w.hy, w.hz);
+            c.after_launch("k_scalar_grad");
+        }
+        if (w.halo_exchange) { double* h[3] = {w.hx.p, w.hy.p, w.hz.p}; w.halo_exchange(h, 3); }   // the upwind cell may be a halo cell
+    }
+    ScalarArgs sa;
+    sa.m = m; sa.F = w.F; sa.phi = phi; sa.gx = w.hx; sa.gy = w.hy; sa.gz = w.hz; sa.zk = d.zone_sbc_kind; sa.zval = d.zone_sbc_value;
+    sa.gamma = gamma; sa.rho = rho; sa.scheme = s.momentum; sa.limiter = s.limiter; sa.val = a.val; sa.b = b;
+    ProfScope ps(c, PC_ASSEMBLY, 0.);
+    k_scalar_transport<<<g, 128, 0, c.stream>>>(sa);
+    c.after_launch("k_scalar_transport");
 }
 
 }  // namespace orc

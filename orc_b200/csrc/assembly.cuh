@@ -30,6 +30,8 @@ struct DMesh {
     // zone table (refreshed when the host table changes)
     DBuf<int> zone_type;
     DBuf<double> zone_scalar, zone_vec;
+    DBuf<int> zone_sbc_kind;          // passive scalar condition per zone (ORC_SBC_*), uploaded with the zone table
+    DBuf<double> zone_sbc_value;
     uint64_t zone_epoch = 0;
 };
 
@@ -84,5 +86,23 @@ void build_pressure_correction(Ctx& c, const DMesh& d, AsmWork& w, const AsmSett
 void apply_pressure_correction(Ctx& c, const DMesh& d, const double* du, const double* dv, const double* dw, const double* p_prime,
                                double* u, double* v, double* wv, double* p, double p_relax, double u_relax, double* out8_dev);
 void extract_diagonal(Ctx& c, const DCsr& a, double* d);  // d[i] = a(i,i); missing -> DF_MISSING_ENTRY
+
+// ---- passive scalar transport on the converged flow (an extension: the reference has no such equation; DESIGN.md §1) ----
+// steady div(rho u phi) - div(Gamma grad phi) = 0 in the mesh pattern, a_P phi_P + sum a_N phi_N = b
+struct ScalarWork {
+    DBuf<double> F;                  // face flux per face, from the side of c0 (k_scalar_face_flux)
+    DBuf<double> gpx, gpy, gpz;      // grad p (Rhie-Chow)
+    DBuf<double> hx, hy, hz;         // grad phi (TVD)
+    std::function<void(double* const*, int)> halo_exchange;   // multi-GPU: as AsmWork::halo_exchange (empty on one GPU)
+};
+// momentum UD / CD1 / TVD(limiter), velocity interpolation other than None, gradient Green-Gauss cell or least squares
+void validate_scalar_settings(const AsmSettings& s);
+// F_f of every face with the resident u, v, w, p, grad p of the settings' scheme and the frozen diagonals du, dv, dw (the halo
+// cells of a partition must hold their owners' values; grad p is exchanged here)
+void scalar_face_flux(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& s, const double* du, const double* dv, const double* dw,
+                      const double* u, const double* v, const double* wv, const double* p);
+// one sweep's system with the current phi (its halo cells filled) and w.F; a shares the mesh pattern, b is a device vector
+void build_scalar_transport(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& s, double gamma, double rho, const double* phi,
+                            DCsr& a, double* b);
 
 }  // namespace orc

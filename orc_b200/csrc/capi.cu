@@ -749,6 +749,19 @@ int32_t orc_init_momentum_matrix(orc_ctx* ctx, orc_mesh* m, orc_csr** out) {
 static void require_mesh_matrix(const DMesh& d, const orc_csr* a, const char* what) {
     if (!a || a->m->nrows != d.N || a->m->nnz != d.nnz) throw Error(ORC_E_INVALID, std::string(what) + ": matrix does not have the mesh pattern");
 }
+// the diagonals of three matrices with the mesh pattern (a_u.get(i, i) in the reference), read through the mesh's diagonal index
+static void momentum_diagonals(Ctx& c, const DMesh& d, const orc_csr* a_u, const orc_csr* a_v, const orc_csr* a_w, double* du, double* dv,
+                               double* dw) {
+    const orc_csr* mats[3] = {a_u, a_v, a_w};
+    double* diags[3] = {du, dv, dw};
+    for (int q = 0; q < 3; ++q) {
+        DCsr& A = *const_cast<orc_csr*>(mats[q])->m;
+        int* keep = A.diag; bool own = A.own_diag;
+        A.diag = d.diag.p; A.own_diag = false;
+        extract_diagonal(c, A, diags[q]);
+        A.diag = keep; A.own_diag = own;
+    }
+}
 int32_t orc_build_momentum_advection(orc_ctx* ctx, orc_mesh* m, orc_csr* a_u, orc_csr* a_v, orc_csr* a_w, const orc_csr* a_di,
                                      const double* u, const double* v, const double* w, const double* p, const orc_settings* s,
                                      double rho, double* b_u, double* b_v, double* b_w, double* peclet3) {
@@ -788,15 +801,7 @@ int32_t orc_build_pressure_correction(orc_ctx* ctx, orc_mesh* m, const orc_csr* 
         DBuf<double> b(&c, N), du(&c, N), dv(&c, N), dw(&c, N);
         AsmWork work;
         c.clear_flags();
-        const orc_csr* mats[3] = {a_u, a_v, a_w};
-        double* diags[3] = {du.p, dv.p, dw.p};
-        for (int q = 0; q < 3; ++q) {
-            DCsr& A = *const_cast<orc_csr*>(mats[q])->m;
-            int* keep = A.diag; bool own = A.own_diag;
-            A.diag = d.diag.p; A.own_diag = false;
-            extract_diagonal(c, A, diags[q]);
-            A.diag = keep; A.own_diag = own;
-        }
+        momentum_diagonals(c, d, a_u, a_v, a_w, du, dv, dw);
         CsrPtr a = mesh_matrix(c, d);
         build_pressure_correction(c, d, work, asm_settings(s), rho, du, dv, dw, du_.d, dv_.d, dw_.d, dp_.d, *a, b);
         to_host(c, b_out, b, d.N);
@@ -832,15 +837,7 @@ int32_t orc_apply_pressure_correction(orc_ctx* ctx, orc_mesh* m, const orc_csr* 
         HostVecIn du_(c, u, d.N), dv_(c, v, d.N), dw_(c, w, d.N), dp_(c, p, d.N), dpp(c, p_prime, d.N);
         DBuf<double> du(&c, N), dv(&c, N), dw(&c, N), out(&c, 8);
         c.clear_flags();
-        const orc_csr* mats[3] = {a_u, a_v, a_w};
-        double* diags[3] = {du.p, dv.p, dw.p};
-        for (int q = 0; q < 3; ++q) {
-            DCsr& A = *const_cast<orc_csr*>(mats[q])->m;
-            int* keep = A.diag; bool own = A.own_diag;
-            A.diag = d.diag.p; A.own_diag = false;
-            extract_diagonal(c, A, diags[q]);
-            A.diag = keep; A.own_diag = own;
-        }
+        momentum_diagonals(c, d, a_u, a_v, a_w, du, dv, dw);
         apply_pressure_correction(c, d, du, dv, dw, dpp.d, du_.d, dv_.d, dw_.d, dp_.d, s->pressure_relaxation, s->momentum_relaxation, out);
         to_host(c, u, du_.d, d.N); to_host(c, v, dv_.d, d.N); to_host(c, w, dw_.d, d.N); to_host(c, p, dp_.d, d.N);
         double h[8];
@@ -1207,6 +1204,97 @@ int32_t orc_steady_gradients(orc_steady* st, int32_t gradient, double* grad_p3n,
         exchange(c, st->env, {st->u.p, st->v.p, st->w.p, st->p.p});   // the halo cells hold whatever the last exchange left
         gradients_to_host(c, d, st->u, st->v, st->w, st->p, gradient, d.own_lo, d.own_hi - d.own_lo, grad_p3n, grad_u9n);
         check_agreed_flags(c, st->env);
+    });
+}
+
+// ---- passive scalar transport (an extension beyond the reference, DESIGN.md §1) ---------------------------------------------------
+int32_t orc_mesh_set_zone_scalar(orc_mesh* m, const char* name, int32_t kind, double value) {
+    ORC_TRY({
+        require(m && name, "null argument");
+        int k = m->h->find_zone(name);
+        if (k < 0) throw Error(ORC_E_INVALID, std::string("face zone '") + name + "' should exist in mesh");
+        require(kind == ORC_SBC_ZERO_GRADIENT || kind == ORC_SBC_FIXED, "unknown scalar boundary condition kind");
+        require(std::isfinite(value), "scalar boundary value must be finite");
+        HostZone& z = m->h->zones[k];
+        z.scalar_bc_kind = kind; z.scalar_bc_value = value;
+        m->h->zone_epoch++;
+    });
+}
+// what every scalar entry checks first: phi is determined only with a FIXED boundary zone, and Gamma is a diffusivity
+static void require_scalar_problem(const HostMesh& h, double gamma, const AsmSettings& as) {
+    validate_scalar_settings(as);
+    require(gamma >= 0., "the diffusivity gamma must be >= 0 (and not NaN)");
+    bool fixed = false;
+    for (const HostZone& z : h.zones) fixed = fixed || (z.type != ORC_BC_INTERIOR && z.scalar_bc_kind == ORC_SBC_FIXED);
+    require(fixed, "no boundary zone fixes the scalar: phi is undetermined (orc_mesh_set_zone_scalar with ORC_SBC_FIXED)");
+}
+int32_t orc_build_scalar_transport(orc_ctx* ctx, orc_mesh* m, const orc_csr* a_u, const orc_csr* a_v, const orc_csr* a_w,
+                                   const double* u, const double* v, const double* w, const double* p, const double* phi,
+                                   double gamma, double rho, const orc_settings* s, orc_csr** a_out, double* b_out) {
+    ORC_TRY({
+        require(ctx && m && m->h && u && v && w && p && phi && s && a_out && b_out, "null argument");
+        const AsmSettings as = asm_settings(s);
+        require_scalar_problem(*m->h, gamma, as);
+        Ctx& c = ctx->c;
+        DMesh& d = device_mesh(c, m);
+        require_mesh_matrix(d, a_u, "a_u"); require_mesh_matrix(d, a_v, "a_v"); require_mesh_matrix(d, a_w, "a_w");
+        ScalarWork work;
+        const DistEnv env = m->plan ? partition_env(ctx, m, nullptr) : DistEnv();
+        if (env.on()) { Comm* cm = env.comm; Halo* hl = env.halo; Ctx* cp = &c; work.halo_exchange = [cm, hl, cp](double* const* f, int n) { hl->exchange(*cp, *cm, f, n); }; }
+        const size_t N = (size_t)std::max<int64_t>(d.N, 1);
+        HostVecIn du_(c, u, d.N), dv_(c, v, d.N), dw_(c, w, d.N), dp_(c, p, d.N), dphi(c, phi, d.N);
+        DBuf<double> b(&c, N), du(&c, N), dv(&c, N), dw(&c, N);
+        c.clear_flags();
+        momentum_diagonals(c, d, a_u, a_v, a_w, du, dv, dw);
+        exchange(c, env, {du_.d.p, dv_.d.p, dw_.d.p, dp_.d.p});
+        exchange(c, env, {du.p, dv.p, dw.p, dphi.d.p});
+        CsrPtr a = mesh_matrix(c, d);
+        scalar_face_flux(c, d, work, as, du, dv, dw, du_.d, dv_.d, dw_.d, dp_.d);
+        build_scalar_transport(c, d, work, as, gamma, rho, dphi.d, *a, b);
+        to_host(c, b_out, b, d.N);
+        check_agreed_flags(c, env);
+        *a_out = wrap(detach(c, std::move(a)));
+    });
+}
+// The flow state of the handle is read, never written: on a partition its fields and diagonals are copied before their halo
+// exchange (the copies' halo cells get the owners' values), so the next iterate() sees exactly what it would have seen.
+int32_t orc_steady_solve_scalar(orc_steady* st, double gamma, uint64_t sweeps, double* phi) {
+    ORC_TRY({
+        require(st && phi, "null argument");
+        const AsmSettings as = asm_settings(&st->s);
+        require_scalar_problem(*st->mesh->h, gamma, as);
+        Ctx& c = *st->c;
+        DMesh& d = device_mesh(c, st->mesh);
+        const DistEnv& env = st->env;
+        const SolveParams sp = solve_params(&st->s, env.on() ? INT64_MAX : st->N_global);
+        const int64_t N = d.N, lo = d.own_lo, cnt = d.own_hi - d.own_lo;
+        const size_t Nz = (size_t)std::max<int64_t>(N, 1);
+        c.clear_flags();
+        ScalarWork work;
+        work.halo_exchange = st->work.halo_exchange;
+        const double *u = st->u, *v = st->v, *w = st->w, *p = st->p, *du = st->du, *dv = st->dv, *dw = st->dw;
+        DBuf<double> flow;
+        if (env.on()) {
+            flow.alloc(&c, 7 * Nz);
+            const double* src[7] = {u, v, w, p, du, dv, dw};
+            for (int k = 0; k < 7; ++k) ORC_CUDA(cudaMemcpyAsync(flow.p + k * Nz, src[k], sizeof(double) * N, cudaMemcpyDeviceToDevice, c.stream));
+            exchange(c, env, {flow.p, flow.p + Nz, flow.p + 2 * Nz, flow.p + 3 * Nz});
+            exchange(c, env, {flow.p + 4 * Nz, flow.p + 5 * Nz, flow.p + 6 * Nz});
+            u = flow.p; v = flow.p + Nz; w = flow.p + 2 * Nz; p = flow.p + 3 * Nz; du = flow.p + 4 * Nz; dv = flow.p + 5 * Nz; dw = flow.p + 6 * Nz;
+        }
+        DBuf<double> x(&c, Nz), b(&c, Nz);
+        x.zero();
+        if (cnt > 0) ORC_CUDA(cudaMemcpyAsync(x.p + lo, phi, sizeof(double) * cnt, cudaMemcpyHostToDevice, c.stream));
+        CsrPtr a = mesh_matrix(c, d);
+        scalar_face_flux(c, d, work, as, du, dv, dw, u, v, w, p);
+        for (uint64_t k = 0; k < sweeps; ++k) {
+            exchange(c, env, {x.p});                                       // the neighbours' phi for the gradient and the face values
+            build_scalar_transport(c, d, work, as, gamma, st->rho, x, *a, b);
+            iterative_solve(c, *a, b, x, sp, nullptr, 1, &env);
+        }
+        to_host(c, phi, x.p + lo, cnt);
+        check_agreed_flags(c, env);
+        c.prof_resolve();
     });
 }
 

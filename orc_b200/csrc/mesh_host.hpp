@@ -22,6 +22,9 @@ struct HostZone {  // src/mesh.rs:12-17
     double scalar = 0.;
     double vec[3] = {0., 0., 0.};
     std::string name;
+    // passive scalar condition of the zone (orc_mesh_set_zone_scalar; not part of the reference's FaceZone)
+    int32_t scalar_bc_kind = 0;     // ORC_SBC_ZERO_GRADIENT / ORC_SBC_FIXED
+    double scalar_bc_value = 0.;
 };
 
 struct HostMesh {

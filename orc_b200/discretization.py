@@ -112,3 +112,19 @@ def potential_gradient(mesh, psi, ctx=None):
     u, v, w = np.zeros(n), np.zeros(n), np.zeros(n)
     _lib.check(_lib.lib().orc_potential_gradient(ctx.handle, mesh.handle, _p(psi), _p(u), _p(v), _p(w)))
     return u, v, w
+
+
+def build_scalar_transport(mesh, a_u, a_v, a_w, u, v, w, p, phi, gamma, rho, settings):
+    """The system of one passive scalar sweep (DESIGN.md §1: steady div(rho u phi) - div(Gamma grad phi) = 0; not in the reference)
+    with the face fluxes of the flow u, v, w, p and the diagonals of a_u, a_v, a_w, for the given phi -> (a, b). Convection scheme:
+    settings.momentum (UD, CD1 or TVD with settings.limiter). On a partition mesh every rank calls it together with its local
+    vectors (halo cells included) and gets its local rows."""
+    mesh._bind(a_u.ctx)
+    n = mesh.n_cells
+    s = settings.to_c()
+    u, v, w, p, phi = _f64(u), _f64(v), _f64(w), _f64(p), _f64(phi)
+    out = C.c_void_p()
+    b = np.zeros(n)
+    _lib.check(_lib.lib().orc_build_scalar_transport(a_u.ctx.handle, mesh.handle, a_u.handle, a_v.handle, a_w.handle, _p(u), _p(v), _p(w),
+                                                     _p(p), _p(phi), C.c_double(gamma), C.c_double(rho), C.byref(s), C.byref(out), _p(b)))
+    return CsrMatrix(out, a_u.ctx), b

@@ -37,6 +37,12 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
+class ScalarCondition(enum.IntEnum):
+    """Condition of a boundary zone for the passive scalar (include/orc_b200.h ORC_SBC_*; not part of the reference)."""
+    ZeroGradient = 0
+    Fixed = 1
+
+
 class FaceZoneView:
     """`mesh.get_face_zone(name)` of the reference (src/mesh.rs:189-195) returns a &mut FaceZone; assignments to
     zone_type / scalar_value / vector_value go through orc_mesh_set_zone."""
@@ -176,6 +182,11 @@ class Mesh:
     def set_zone(self, name, zone_type, scalar=0.0, vector=(0.0, 0.0, 0.0)):
         _lib.check(_lib.lib().orc_mesh_set_zone(self._h, name.encode(), C.c_int64(int(zone_type)), C.c_double(scalar),
                                                 C.c_double(vector[0]), C.c_double(vector[1]), C.c_double(vector[2])))
+
+    def set_zone_scalar(self, name, kind, value=0.0):
+        """The passive scalar condition of zone `name` (every zone starts as ZeroGradient): ScalarCondition.Fixed holds phi = value
+        on the zone's faces. Partitions taken afterwards inherit it."""
+        _lib.check(_lib.lib().orc_mesh_set_zone_scalar(self._h, name.encode(), C.c_int32(int(kind)), C.c_double(value)))
 
     def get_face_zone(self, name):  # src/mesh.rs:189-195
         if name not in self.zones()["names"]:

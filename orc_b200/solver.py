@@ -131,6 +131,18 @@ class SteadySolver:
         gp, gu = self.gradients(gradient_scheme)
         _write_gradient_lines(output_file_name, _owned_centroids(self.mesh), gp, gu, decimal_precision)
 
+    def solve_scalar(self, gamma, phi=None, sweeps=1):
+        """A passive scalar carried by the resident flow (DESIGN.md §1; not in the reference): `sweeps` assemble + solve sweeps of
+        steady div(rho u phi) - div(gamma grad phi) = 0 with the handle's settings (convection scheme settings.momentum, the
+        matrix solver of settings.matrix_solver) and the zones' scalar conditions (Mesh.set_zone_scalar). Starts from `phi` (zero by
+        default) and returns phi of the exposed cells. The flow state is left as it was. On a partition mesh every rank calls it
+        together."""
+        x = np.zeros(self.n) if phi is None else _f64(phi).copy()
+        if x.size != self.n:
+            raise ValueError("phi must have one value per exposed cell")
+        _lib.check(_lib.lib().orc_steady_solve_scalar(self._h, C.c_double(gamma), C.c_uint64(sweeps), _p(x)))
+        return x
+
     def reset(self):
         """Back to the state solve_steady starts from: zero fields, momentum matrices re-initialised (diag 1)."""
         _lib.check(_lib.lib().orc_steady_reset(self._h))

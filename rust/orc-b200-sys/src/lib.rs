@@ -50,6 +50,10 @@ extern "C" {
     pub fn orc_steady_gradients(st: *mut orc_steady, gradient: i32, grad_p3n: *mut f64, grad_u9n: *mut f64) -> i32;
     // check_boundary_conditions (src/solver.rs:710-770): 0 PressureOnly, 1 VelocityOnly, 2 Hybrid
     pub fn orc_check_boundary_conditions(m: *const orc_mesh, constraint_type: *mut i32) -> i32;
+    // passive scalar transport (not in the reference): zone condition (0 zero gradient, 1 fixed), and `sweeps` assemble + solve
+    // sweeps on the steady handle's resident flow; phi in/out
+    pub fn orc_mesh_set_zone_scalar(m: *mut orc_mesh, name: *const c_char, kind: i32, value: f64) -> i32;
+    pub fn orc_steady_solve_scalar(st: *mut orc_steady, gamma: f64, sweeps: u64, phi: *mut f64) -> i32;
 }
 
 fn settings_to_c(ns: &NumericalSettings) -> orc_settings {
