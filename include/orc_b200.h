@@ -232,7 +232,7 @@ int32_t orc_steady_get_fields(orc_steady* st, double* u, double* v, double* w, d
 int32_t orc_steady_iterate(orc_steady* st, uint64_t iterations, orc_report* last /* nullable */);
 /* back to the state solve_steady starts from (src/solver.rs:43-49): zero fields, momentum matrices re-initialised */
 int32_t orc_steady_reset(orc_steady* st);
-/* per-phase device time (ms, CUDA events) accumulated since creation:
+/* per-phase device time (ms, CUDA events) accumulated since creation (a coupled handle counts its scalar sweeps to the correction):
  * momentum assembly, 3 momentum solves, pressure assembly, pressure solve, correction */
 int32_t orc_steady_phase_ms(orc_steady* st, double* out5);
 /* 1 if the last orc_steady_iterate solved u, v, w in lockstep (a_u == a_v == a_w bit for bit, checked on the device; env
@@ -258,6 +258,20 @@ int32_t orc_build_scalar_transport(orc_ctx* ctx, orc_mesh* m, const orc_csr* a_u
  * untouched. phi: in/out, the exposed cells (owned cells of a partition; every rank calls it together). One sweep is exact for UD
  * and CD1; TVD is a Picard iteration. */
 int32_t orc_steady_solve_scalar(orc_steady* st, double gamma, uint64_t sweeps, double* phi);
+/* Boussinesq coupling of the scalar into the loop (DESIGN.md §1): every orc_steady_iterate adds the body force
+ * -rho beta (phi - phi_ref) g of the resident phi to the momentum sources, and after the correction runs `sweeps` sweeps of the scalar
+ * system (as orc_steady_solve_scalar with gamma) from the resident phi. p is then the reduced pressure. sweeps = 0 uncouples and
+ * ignores the other arguments. gamma as for orc_steady_solve_scalar; beta, phi_ref and g finite. Validation as
+ * orc_steady_solve_scalar (no FIXED zone, gamma < 0 / NaN: ORC_E_INVALID; CD2, V_NONE: ORC_E_UNSUPPORTED); a refused call leaves
+ * the handle as it was. orc_steady_reset zeroes the resident phi and keeps the coupling. */
+int32_t orc_steady_couple_scalar(orc_steady* st, double gamma, double beta, double phi_ref, double gx, double gy, double gz, uint64_t sweeps);
+/* the resident phi of the exposed (owned) cells; zero until set or computed */
+int32_t orc_steady_set_scalar(orc_steady* st, const double* phi);
+int32_t orc_steady_get_scalar(orc_steady* st, double* phi);
+/* outward flux of the resident phi through zone `name` with the resident flow's face mass fluxes and the coupling's gamma:
+ * out2 = (diffusive, convective), each summed over the zone's faces in ascending face order (a partition: each rank's total, added in
+ * rank order). An uncoupled handle or an unknown zone: ORC_E_INVALID. */
+int32_t orc_steady_scalar_zone_flux(orc_steady* st, const char* name, double* out2);
 void orc_steady_destroy(orc_steady* st);
 
 /* ---- flow initialisation: the step before the loop (src/solver.rs:246-352) ------------------------- */

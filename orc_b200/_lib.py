@@ -53,6 +53,7 @@ EXPORTS = [
     "orc_solve_steady", "orc_check_boundary_conditions", "orc_build_pressure_laplace", "orc_initialize_flow", "orc_initialize_flow_new", "orc_build_velocity_potential", "orc_potential_gradient", "orc_gradients", "orc_steady_create", "orc_steady_set_fields", "orc_steady_get_fields", "orc_steady_iterate", "orc_steady_reset",
     "orc_steady_phase_ms", "orc_steady_batched", "orc_steady_level_sizes", "orc_steady_gradients", "orc_steady_destroy", "orc_bench_amg_setup", "orc_bench_spmv", "orc_bench_bicgstab", "orc_bench_spmv_batch", "orc_bench_bicgstab_batch", "orc_prof_enable", "orc_prof_config", "orc_prof_get", "orc_prof_get_ref_bytes", "orc_prof_get_spmv_detail", "orc_comm_unique_id", "orc_ctx_comm_init", "orc_ctx_peer_window", "orc_ctx_peer_open", "orc_ctx_peer_disable", "orc_ctx_peer_enabled", "orc_mesh_partition", "orc_mesh_partition_window",
     "orc_mesh_partition_info", "orc_mesh_partition_maps", "orc_mesh_set_zone_scalar", "orc_build_scalar_transport", "orc_steady_solve_scalar",
+    "orc_steady_couple_scalar", "orc_steady_set_scalar", "orc_steady_get_scalar", "orc_steady_scalar_zone_flux",
 ]
 
 

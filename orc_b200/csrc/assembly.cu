@@ -1257,4 +1257,58 @@ void build_scalar_transport(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSett
     c.after_launch("k_scalar_transport");
 }
 
+// S4: Boussinesq body force -rho beta (phi - phi_ref) g, fused with the b += b_di of the momentum right-hand sides: one pass of
+// 88 B per owned cell (reads b x3, b_di x3, phi, V; writes b x3). Halo rows get (b + b_di) only, as the three k_add_inplace give.
+__global__ void k_momentum_source_buoyancy(int64_t n, int64_t lo, int64_t hi, double* bu, double* bv, double* bw, const double* __restrict__ bdu,
+                                           const double* __restrict__ bdv, const double* __restrict__ bdw, const double* __restrict__ phi,
+                                           const double* __restrict__ vol, double rho_beta, double phi_ref, double gx, double gy, double gz) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        double x = bu[i] + bdu[i], y = bv[i] + bdv[i], z = bw[i] + bdw[i];
+        if (i >= lo && i < hi) {
+            const double s = (rho_beta * (phi[i] - phi_ref)) * vol[i];
+            x = x - s * gx; y = y - s * gy; z = z - s * gz;
+        }
+        bu[i] = x; bv[i] = y; bw[i] = z;
+    }
+}
+void momentum_source_buoyancy(Ctx& c, const DMesh& d, double* b_u, double* b_v, double* b_w, const double* b_u_di, const double* b_v_di,
+                              const double* b_w_di, const double* phi, double rho_beta, double phi_ref, const double g[3]) {
+    if (d.N <= 0) return;
+    ProfScope ps(c, PC_ASSEMBLY, 0.);
+    k_momentum_source_buoyancy<<<grid_for(d.N, 256, 1184), 256, 0, c.stream>>>(d.N, d.own_lo, d.own_hi, b_u, b_v, b_w, b_u_di, b_v_di, b_w_di, phi,
+                                                                               d.cvol, rho_beta, phi_ref, g[0], g[1], g[2]);
+    c.after_launch("k_momentum_source_buoyancy");
+}
+
+// S5: the outward flux of phi through every face of zone `zone` (zero elsewhere), from its cell c0 with mass flux
+// f = (rho A_f) F_f: FIXED(phi_b) diffusive d_b (phi_P - phi_b), convective max(f, 0) phi_P + min(f, 0) phi_b; ZERO_GRADIENT 0 and
+// f phi_P. out2: two planes of F doubles (diffusive, convective).
+__global__ void __launch_bounds__(128) k_scalar_zone_flux(MV m, const int* __restrict__ zk, const double* __restrict__ zval, const double* __restrict__ F,
+                                                          const double* __restrict__ phi, double gamma, double rho, int zone, double* diff, double* conv) {
+    for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < m.F; f += gridDim.x * blockDim.x) {
+        double dd = 0., cc = 0.;
+        if (m.fz[f] == zone) {
+            const int p = m.c0[f];
+            const double area = m.area[f];
+            const double fl = (rho * area) * F[f];
+            if (zk[zone] == ORC_SBC_FIXED) {
+                const double d_b = gamma * area / vnorm(vsub(fcentroid(m, f), ccentroid(m, p)));
+                dd = d_b * (phi[p] - zval[zone]);
+                cc = pos_part(fl) * phi[p] + neg_part(fl) * zval[zone];
+            } else {
+                cc = fl * phi[p];
+            }
+        }
+        diff[f] = dd; conv[f] = cc;
+    }
+}
+void scalar_zone_flux(Ctx& c, const DMesh& d, const ScalarWork& w, double gamma, double rho, const double* phi, int zone, double* out2F) {
+    ORC_REQUIRE(w.F.n == (size_t)std::max<int64_t>(d.F, 1), ORC_E_INTERNAL, "scalar_zone_flux: face fluxes not computed");
+    if (d.F == 0) return;
+    ProfScope ps(c, PC_ASSEMBLY, 0.);
+    k_scalar_zone_flux<<<grid_for(d.F, 128, c.sm_count * 16), 128, 0, c.stream>>>(view(d), d.zone_sbc_kind, d.zone_sbc_value, w.F, phi, gamma, rho,
+                                                                                 zone, out2F, out2F + d.F);
+    c.after_launch("k_scalar_zone_flux");
+}
+
 }  // namespace orc

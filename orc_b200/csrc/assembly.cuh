@@ -104,5 +104,12 @@ void scalar_face_flux(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& 
 // one sweep's system with the current phi (its halo cells filled) and w.F; a shares the mesh pattern, b is a device vector
 void build_scalar_transport(Ctx& c, const DMesh& d, ScalarWork& w, const AsmSettings& s, double gamma, double rho, const double* phi,
                             DCsr& a, double* b);
+// Boussinesq coupling (DESIGN.md §1): b_k <- (b_k + b_di,k) - (s_P * g_k) with s_P = ((rho * beta) * (phi_P - phi_ref)) * V_P on the
+// owned rows, b_k + b_di,k on the halo rows, k = u, v, w (one launch)
+void momentum_source_buoyancy(Ctx& c, const DMesh& d, double* b_u, double* b_v, double* b_w, const double* b_u_di, const double* b_v_di,
+                              const double* b_w_di, const double* phi, double rho_beta, double phi_ref, const double g[3]);
+// outward diffusive / convective flux of phi through each face of zone index `zone` with w.F (zero on other faces): out2F = two
+// planes of d.F doubles
+void scalar_zone_flux(Ctx& c, const DMesh& d, const ScalarWork& w, double gamma, double rho, const double* phi, int zone, double* out2F);
 
 }  // namespace orc

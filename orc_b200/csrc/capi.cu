@@ -118,6 +118,12 @@ struct orc_steady {
     bool last_batched = false;
     double phase_ms[5] = {0, 0, 0, 0, 0};
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // Boussinesq coupling of the scalar (orc_steady_couple_scalar; sweeps == 0: not coupled) and the resident phi with the buffers
+    // of its sweeps, all allocated on first use so that a handle that never uses them carries none
+    struct Coupling { double gamma = 0., beta = 0., phi_ref = 0., g[3] = {0., 0., 0.}; uint64_t sweeps = 0; } cpl;
+    DBuf<double> phi, phi_b;
+    CsrPtr phi_a;
+    ScalarWork swork;
     ~orc_steady() {
         for (auto& e : ev) if (e) cudaEventDestroy(e);
     }
@@ -226,6 +232,37 @@ static int flags_from_double(double v) {
     return f;
 }
 
+// what every scalar entry checks first: phi is determined only with a FIXED boundary zone, and Gamma is a diffusivity
+static void require_scalar_problem(const HostMesh& h, double gamma, const AsmSettings& as) {
+    validate_scalar_settings(as);
+    require(gamma >= 0., "the diffusivity gamma must be >= 0 (and not NaN)");
+    bool fixed = false;
+    for (const HostZone& z : h.zones) fixed = fixed || (z.type != ORC_BC_INTERIOR && z.scalar_bc_kind == ORC_SBC_FIXED);
+    require(fixed, "no boundary zone fixes the scalar: phi is undetermined (orc_mesh_set_zone_scalar with ORC_SBC_FIXED)");
+}
+// `sweeps` assemble + iterative_solve sweeps of the scalar system from phi = x on the flow u, v, w, p with the diagonals du, dv, dw
+// (their halo cells filled); x's halo cells are refreshed before every sweep. a shares the mesh pattern, b has N entries.
+static void scalar_sweeps(Ctx& c, const DMesh& d, const DistEnv& env, ScalarWork& work, const AsmSettings& as, const SolveParams& sp,
+                          double gamma, double rho, uint64_t sweeps, const double* du, const double* dv, const double* dw, const double* u,
+                          const double* v, const double* w, const double* p, DCsr& a, double* b, double* x) {
+    scalar_face_flux(c, d, work, as, du, dv, dw, u, v, w, p);
+    for (uint64_t k = 0; k < sweeps; ++k) {
+        exchange(c, env, {x});                                       // the neighbours' phi for the gradient and the face values
+        build_scalar_transport(c, d, work, as, gamma, rho, x, a, b);
+        iterative_solve(c, a, b, x, sp, nullptr, 1, &env);
+    }
+}
+// the resident phi (zero) and the buffers of the coupled sweeps, on first use
+static void ensure_scalar(orc_steady& st) {
+    if (st.phi.p) return;
+    Ctx& c = *st.c;
+    const size_t N = (size_t)std::max<int64_t>(st.N, 1);
+    st.phi.alloc(&c, N); st.phi.zero();
+    st.phi_b.alloc(&c, N); st.phi_b.zero();
+    st.phi_a = mesh_matrix(c, *st.dm);
+    st.swork.halo_exchange = st.work.halo_exchange;
+}
+
 static void steady_iterate(orc_steady& st, uint64_t iterations, uint64_t report_every, orc_report_cb cb, void* user, orc_report* last) {
     Ctx& c = *st.c;
     DMesh& d = device_mesh(c, st.mesh);
@@ -233,6 +270,8 @@ static void steady_iterate(orc_steady& st, uint64_t iterations, uint64_t report_
     // multi-GPU solves always use the fused reductions (ORC_REDUCE_AUTO never picks the single-GPU reference-order kernels there)
     const SolveParams sp = solve_params(&st.s, st.env.on() ? INT64_MAX : st.N_global);
     const int64_t N = st.N;
+    const bool coupled = st.cpl.sweeps > 0;
+    if (coupled) require_scalar_problem(*st.mesh->h, st.cpl.gamma, as);   // the zones' scalar conditions may have changed since
     cudaEvent_t t_report;
     ORC_CUDA(cudaEventCreate(&t_report));
     struct EvGuard { cudaEvent_t e; ~EvGuard() { cudaEventDestroy(e); } } guard{t_report};
@@ -245,7 +284,12 @@ static void steady_iterate(orc_steady& st, uint64_t iterations, uint64_t report_
         int pid = c.prof_begin(PC_ASSEMBLY, 0.);
         build_momentum_advection(c, d, st.work, as, st.rho, *st.a_u, *st.a_v, *st.a_w, *st.a_di, st.du, st.dv, st.dw, st.u, st.v, st.w, st.p,
                                  st.b_u, st.b_v, st.b_w, st.scal.p + 8);                                   // solver.rs:61-79
-        dev_axpy_inplace(c, st.b_u, st.b_u_di, N); dev_axpy_inplace(c, st.b_v, st.b_v_di, N); dev_axpy_inplace(c, st.b_w, st.b_w_di, N);  // :80-82
+        if (coupled) {  // b + b_di + the body force of phi as it stood when the iteration started (DESIGN.md §1)
+            momentum_source_buoyancy(c, d, st.b_u, st.b_v, st.b_w, st.b_u_di, st.b_v_di, st.b_w_di, st.phi, st.rho * st.cpl.beta, st.cpl.phi_ref,
+                                     st.cpl.g);
+        } else {
+            dev_axpy_inplace(c, st.b_u, st.b_u_di, N); dev_axpy_inplace(c, st.b_v, st.b_v_di, N); dev_axpy_inplace(c, st.b_w, st.b_w_di, N);  // :80-82
+        }
         c.prof_end(pid);
         exchange(c, st.env, {st.du.p, st.dv.p, st.dw.p});  // new diagonals for the pressure system; the "old" state of the next assembly (C4)
         ORC_CUDA(cudaEventRecord(st.ev[1], c.stream));
@@ -269,6 +313,11 @@ static void steady_iterate(orc_steady& st, uint64_t iterations, uint64_t report_
         ORC_CUDA(cudaEventRecord(st.ev[4], c.stream));
         apply_pressure_correction(c, d, st.du, st.dv, st.dw, st.p_prime, st.u, st.v, st.w, st.p, st.s.pressure_relaxation,
                                   st.s.momentum_relaxation, st.scal.p);                                    // :193-204
+        if (coupled) {  // the scalar sweeps on the corrected flow and this iteration's diagonals (counted in the correction phase)
+            exchange(c, st.env, {st.u.p, st.v.p, st.w.p, st.p.p});
+            scalar_sweeps(c, d, st.env, st.swork, as, sp, st.cpl.gamma, st.rho, st.cpl.sweeps, st.du, st.dv, st.dw, st.u, st.v, st.w, st.p,
+                          *st.phi_a, st.phi_b, st.phi);
+        }
         ORC_CUDA(cudaEventRecord(st.ev[5], c.stream));
         if (dist) {  // C2: iteration scalars; the status word travels along so that every rank takes the same exit
             Comm& cm = *st.env.comm;
@@ -887,6 +936,7 @@ int32_t orc_steady_reset(orc_steady* st) {
         init_momentum_matrix(c, d, *st->a_u); init_momentum_matrix(c, d, *st->a_v); init_momentum_matrix(c, d, *st->a_w);
         dev_fill(c, st->du, 1., d.N); dev_fill(c, st->dv, 1., d.N); dev_fill(c, st->dw, 1., d.N);
         for (DBuf<double>* b : {&st->b_u, &st->b_v, &st->b_w, &st->p_prime, &st->u, &st->v, &st->w, &st->p}) b->zero();
+        st->phi.zero();   // the resident phi, if any; the coupling stays
         st->iteration = 0;
     });
 }
@@ -1220,14 +1270,6 @@ int32_t orc_mesh_set_zone_scalar(orc_mesh* m, const char* name, int32_t kind, do
         m->h->zone_epoch++;
     });
 }
-// what every scalar entry checks first: phi is determined only with a FIXED boundary zone, and Gamma is a diffusivity
-static void require_scalar_problem(const HostMesh& h, double gamma, const AsmSettings& as) {
-    validate_scalar_settings(as);
-    require(gamma >= 0., "the diffusivity gamma must be >= 0 (and not NaN)");
-    bool fixed = false;
-    for (const HostZone& z : h.zones) fixed = fixed || (z.type != ORC_BC_INTERIOR && z.scalar_bc_kind == ORC_SBC_FIXED);
-    require(fixed, "no boundary zone fixes the scalar: phi is undetermined (orc_mesh_set_zone_scalar with ORC_SBC_FIXED)");
-}
 int32_t orc_build_scalar_transport(orc_ctx* ctx, orc_mesh* m, const orc_csr* a_u, const orc_csr* a_v, const orc_csr* a_w,
                                    const double* u, const double* v, const double* w, const double* p, const double* phi,
                                    double gamma, double rho, const orc_settings* s, orc_csr** a_out, double* b_out) {
@@ -1256,8 +1298,24 @@ int32_t orc_build_scalar_transport(orc_ctx* ctx, orc_mesh* m, const orc_csr* a_u
         *a_out = wrap(detach(c, std::move(a)));
     });
 }
-// The flow state of the handle is read, never written: on a partition its fields and diagonals are copied before their halo
-// exchange (the copies' halo cells get the owners' values), so the next iterate() sees exactly what it would have seen.
+// The handle's u, v, w, p, du, dv, dw with their halo cells filled, read, never written: on a partition they are copied to `flow`
+// before their halo exchange (the copies' halo cells get the owners' values), so the next iterate() sees exactly what it would have
+// seen.
+static void resident_flow(orc_steady& st, DBuf<double>& flow, const double* out[7]) {
+    const double* src[7] = {st.u, st.v, st.w, st.p, st.du, st.dv, st.dw};
+    for (int k = 0; k < 7; ++k) out[k] = src[k];
+    if (!st.env.on()) return;
+    Ctx& c = *st.c;
+    const size_t Nz = (size_t)std::max<int64_t>(st.N, 1);
+    flow.alloc(&c, 7 * Nz);
+    for (int k = 0; k < 7; ++k) {
+        ORC_CUDA(cudaMemcpyAsync(flow.p + k * Nz, src[k], sizeof(double) * st.N, cudaMemcpyDeviceToDevice, c.stream));
+        out[k] = flow.p + k * Nz;
+    }
+    exchange(c, st.env, {flow.p, flow.p + Nz, flow.p + 2 * Nz, flow.p + 3 * Nz});
+    exchange(c, st.env, {flow.p + 4 * Nz, flow.p + 5 * Nz, flow.p + 6 * Nz});
+}
+// The flow state of the handle is left as it was (resident_flow).
 int32_t orc_steady_solve_scalar(orc_steady* st, double gamma, uint64_t sweeps, double* phi) {
     ORC_TRY({
         require(st && phi, "null argument");
@@ -1267,34 +1325,100 @@ int32_t orc_steady_solve_scalar(orc_steady* st, double gamma, uint64_t sweeps, d
         DMesh& d = device_mesh(c, st->mesh);
         const DistEnv& env = st->env;
         const SolveParams sp = solve_params(&st->s, env.on() ? INT64_MAX : st->N_global);
-        const int64_t N = d.N, lo = d.own_lo, cnt = d.own_hi - d.own_lo;
-        const size_t Nz = (size_t)std::max<int64_t>(N, 1);
+        const int64_t lo = d.own_lo, cnt = d.own_hi - d.own_lo;
+        const size_t Nz = (size_t)std::max<int64_t>(d.N, 1);
         c.clear_flags();
         ScalarWork work;
         work.halo_exchange = st->work.halo_exchange;
-        const double *u = st->u, *v = st->v, *w = st->w, *p = st->p, *du = st->du, *dv = st->dv, *dw = st->dw;
         DBuf<double> flow;
-        if (env.on()) {
-            flow.alloc(&c, 7 * Nz);
-            const double* src[7] = {u, v, w, p, du, dv, dw};
-            for (int k = 0; k < 7; ++k) ORC_CUDA(cudaMemcpyAsync(flow.p + k * Nz, src[k], sizeof(double) * N, cudaMemcpyDeviceToDevice, c.stream));
-            exchange(c, env, {flow.p, flow.p + Nz, flow.p + 2 * Nz, flow.p + 3 * Nz});
-            exchange(c, env, {flow.p + 4 * Nz, flow.p + 5 * Nz, flow.p + 6 * Nz});
-            u = flow.p; v = flow.p + Nz; w = flow.p + 2 * Nz; p = flow.p + 3 * Nz; du = flow.p + 4 * Nz; dv = flow.p + 5 * Nz; dw = flow.p + 6 * Nz;
-        }
+        const double* f[7];
+        resident_flow(*st, flow, f);
         DBuf<double> x(&c, Nz), b(&c, Nz);
         x.zero();
         if (cnt > 0) ORC_CUDA(cudaMemcpyAsync(x.p + lo, phi, sizeof(double) * cnt, cudaMemcpyHostToDevice, c.stream));
         CsrPtr a = mesh_matrix(c, d);
-        scalar_face_flux(c, d, work, as, du, dv, dw, u, v, w, p);
-        for (uint64_t k = 0; k < sweeps; ++k) {
-            exchange(c, env, {x.p});                                       // the neighbours' phi for the gradient and the face values
-            build_scalar_transport(c, d, work, as, gamma, st->rho, x, *a, b);
-            iterative_solve(c, *a, b, x, sp, nullptr, 1, &env);
-        }
+        scalar_sweeps(c, d, env, work, as, sp, gamma, st->rho, sweeps, f[4], f[5], f[6], f[0], f[1], f[2], f[3], *a, b, x);
         to_host(c, phi, x.p + lo, cnt);
         check_agreed_flags(c, env);
         c.prof_resolve();
+    });
+}
+
+// ---- Boussinesq coupling of the scalar into the loop (an extension beyond the reference, DESIGN.md §1) -----------------------------
+int32_t orc_steady_couple_scalar(orc_steady* st, double gamma, double beta, double phi_ref, double gx, double gy, double gz, uint64_t sweeps) {
+    ORC_TRY({
+        require(st != nullptr, "null argument");
+        if (sweeps == 0) {
+            st->cpl = orc_steady::Coupling();
+        } else {
+            require_scalar_problem(*st->mesh->h, gamma, asm_settings(&st->s));
+            require(std::isfinite(beta) && std::isfinite(phi_ref) && std::isfinite(gx) && std::isfinite(gy) && std::isfinite(gz),
+                    "beta, phi_ref and g must be finite");
+            ensure_scalar(*st);
+            orc_steady::Coupling k;
+            k.gamma = gamma; k.beta = beta; k.phi_ref = phi_ref; k.g[0] = gx; k.g[1] = gy; k.g[2] = gz; k.sweeps = sweeps;
+            st->cpl = k;
+        }
+    });
+}
+int32_t orc_steady_set_scalar(orc_steady* st, const double* phi) {
+    ORC_TRY({
+        require(st && phi, "null argument");
+        ensure_scalar(*st);
+        Ctx& c = *st->c;
+        const int64_t lo = st->dm->own_lo, cnt = st->dm->own_hi - lo;
+        if (cnt > 0) ORC_CUDA(cudaMemcpyAsync(st->phi.p + lo, phi, sizeof(double) * cnt, cudaMemcpyHostToDevice, c.stream));
+        c.sync();
+    });
+}
+int32_t orc_steady_get_scalar(orc_steady* st, double* phi) {
+    ORC_TRY({
+        require(st && phi, "null argument");
+        ensure_scalar(*st);
+        to_host(*st->c, phi, st->phi.p + st->dm->own_lo, st->dm->own_hi - st->dm->own_lo);
+        st->c->sync();
+    });
+}
+int32_t orc_steady_scalar_zone_flux(orc_steady* st, const char* name, double* out2) {
+    ORC_TRY({
+        require(st && name && out2, "null argument");
+        const HostMesh& h = *st->mesh->h;
+        const int zone = h.find_zone(name);
+        if (zone < 0) throw Error(ORC_E_INVALID, std::string("face zone '") + name + "' should exist in mesh");
+        require(st->cpl.sweeps > 0, "the handle is not coupled (orc_steady_couple_scalar): the zone flux uses the coupling's gamma");
+        const AsmSettings as = asm_settings(&st->s);
+        require_scalar_problem(h, st->cpl.gamma, as);
+        Ctx& c = *st->c;
+        DMesh& d = device_mesh(c, st->mesh);
+        c.clear_flags();
+        DBuf<double> flow;
+        const double* f[7];
+        resident_flow(*st, flow, f);
+        scalar_face_flux(c, d, st->swork, as, f[4], f[5], f[6], f[0], f[1], f[2], f[3]);
+        const size_t F = (size_t)std::max<int64_t>(d.F, 1);
+        DBuf<double> terms(&c, 2 * F);
+        terms.zero();
+        scalar_zone_flux(c, d, st->swork, st->cpl.gamma, st->rho, st->phi, zone, terms);
+        std::vector<double> t(2 * F);
+        to_host(c, t.data(), terms, 2 * (int64_t)F);
+        c.sync();
+        double mine[2] = {0., 0.};   // ascending face order; faces of other zones hold +0
+        for (int64_t q = 0; q < d.F; ++q) { mine[0] += t[q]; mine[1] += t[F + q]; }
+        out2[0] = mine[0]; out2[1] = mine[1];
+        if (st->env.on()) {   // every boundary face belongs to one rank: the ranks' totals, added in rank order
+            Comm& cm = *st->env.comm;
+            DBuf<double> one(&c, 2);
+            out2[0] = out2[1] = 0.;
+            for (int r = 0; r < cm.nranks; ++r) {
+                double v[2] = {r == cm.rank ? mine[0] : 0., r == cm.rank ? mine[1] : 0.};
+                ORC_CUDA(cudaMemcpyAsync(one.p, v, sizeof(v), cudaMemcpyHostToDevice, c.stream));
+                cm.allreduce(c, one.p, 2, 0);
+                ORC_CUDA(cudaMemcpyAsync(v, one.p, sizeof(v), cudaMemcpyDeviceToHost, c.stream));
+                c.sync();
+                out2[0] += v[0]; out2[1] += v[1];
+            }
+        }
+        check_agreed_flags(c, st->env);
     });
 }
 

@@ -143,6 +143,41 @@ class SteadySolver:
         _lib.check(_lib.lib().orc_steady_solve_scalar(self._h, C.c_double(gamma), C.c_uint64(sweeps), _p(x)))
         return x
 
+    def couple_scalar(self, gamma, beta, phi_ref, gravity, sweeps=1):
+        """Buoyancy-driven flow (Boussinesq, DESIGN.md §1; not in the reference): from now on every iterate() adds the body force
+        -rho * beta * (phi - phi_ref) * gravity of the resident scalar to the momentum equations and, after the pressure correction,
+        runs `sweeps` sweeps of the scalar transport of solve_scalar(gamma) from the resident phi. p becomes the reduced pressure.
+        `gravity` is (g_x, g_y, g_z). reset() zeroes phi and keeps the coupling."""
+        gx, gy, gz = (float(g) for g in gravity)
+        if sweeps < 1:
+            raise ValueError("sweeps must be >= 1 (uncouple_scalar() uncouples)")
+        _lib.check(_lib.lib().orc_steady_couple_scalar(self._h, C.c_double(gamma), C.c_double(beta), C.c_double(phi_ref), C.c_double(gx),
+                                                       C.c_double(gy), C.c_double(gz), C.c_uint64(sweeps)))
+
+    def uncouple_scalar(self):
+        """Back to the plain loop: iterate() neither adds a body force nor solves for phi (the resident phi is kept)."""
+        _lib.check(_lib.lib().orc_steady_couple_scalar(self._h, C.c_double(0.0), C.c_double(0.0), C.c_double(0.0), C.c_double(0.0),
+                                                       C.c_double(0.0), C.c_double(0.0), C.c_uint64(0)))
+
+    def set_scalar(self, phi):
+        """The resident phi of the exposed cells."""
+        x = _f64(phi)
+        if x.size != self.n:
+            raise ValueError("phi must have one value per exposed cell")
+        _lib.check(_lib.lib().orc_steady_set_scalar(self._h, _p(x)))
+
+    def get_scalar(self):
+        x = np.zeros(self.n)
+        _lib.check(_lib.lib().orc_steady_get_scalar(self._h, _p(x)))
+        return x
+
+    def scalar_zone_flux(self, name):
+        """(diffusive, convective) outward flux of the resident phi through zone `name` on the resident flow (coupled handles only:
+        the diffusivity is the coupling's gamma). On a partition mesh every rank calls it together and gets the whole zone's flux."""
+        out = np.zeros(2)
+        _lib.check(_lib.lib().orc_steady_scalar_zone_flux(self._h, name.encode(), _p(out)))
+        return float(out[0]), float(out[1])
+
     def reset(self):
         """Back to the state solve_steady starts from: zero fields, momentum matrices re-initialised (diag 1)."""
         _lib.check(_lib.lib().orc_steady_reset(self._h))

@@ -54,6 +54,12 @@ extern "C" {
     // sweeps on the steady handle's resident flow; phi in/out
     pub fn orc_mesh_set_zone_scalar(m: *mut orc_mesh, name: *const c_char, kind: i32, value: f64) -> i32;
     pub fn orc_steady_solve_scalar(st: *mut orc_steady, gamma: f64, sweeps: u64, phi: *mut f64) -> i32;
+    // Boussinesq coupling of the scalar into the loop (sweeps = 0 uncouples), the resident phi of the owned cells, and the
+    // (diffusive, convective) outward flux of phi through a zone
+    pub fn orc_steady_couple_scalar(st: *mut orc_steady, gamma: f64, beta: f64, phi_ref: f64, gx: f64, gy: f64, gz: f64, sweeps: u64) -> i32;
+    pub fn orc_steady_set_scalar(st: *mut orc_steady, phi: *const f64) -> i32;
+    pub fn orc_steady_get_scalar(st: *mut orc_steady, phi: *mut f64) -> i32;
+    pub fn orc_steady_scalar_zone_flux(st: *mut orc_steady, name: *const c_char, out2: *mut f64) -> i32;
 }
 
 fn settings_to_c(ns: &NumericalSettings) -> orc_settings {
